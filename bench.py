@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the compress-step benchmark (BASELINE.json metric) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2] [--impl ours|reference] [--dump-outputs DIR]
 
 One *step* = one pass of the compress hot path over one batch of synthetic KV cache: every call the
 config names (for the default c2: ``streaming_llm_compress(4, 508)`` then
@@ -109,7 +109,15 @@ def parse_args():
     ap.add_argument("--e2e-slab", type=int, default=8, help="streams per host<->device slab in the e2e leg")
     ap.add_argument("--cpu-sample-batch", type=int, default=0,
                     help="streams in the CPU sample (0: enough (b,h) rows to occupy every host thread, at most 8)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned (rank 0) to DIR/*.npy as float32, so that two builds "
+                         "can be compared output for output; see dump_outputs()")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "functions"):
+        ap.error("--dump-outputs writes the outputs of the compress functions (--impl ours --mode functions)")
+    return args
 
 
 def measured_peak():
@@ -472,11 +480,13 @@ def vote_inputs(cfg, B, kv, device):
 
     extra = {}
     flops = 0
+    g = torch.Generator(device=device).manual_seed(5678)   # the same queries on every run
     for m, kw in cfg["calls"]:
         if "_vote_group" not in kw:
             continue
         G, Wn = kw["_vote_group"], kw["observation_window"]
-        qs = [(1.5 * torch.randn(B, cfg["H"] * G, Wn, cfg["D"], device=device)).to(kv[0][0].dtype) for _ in range(cfg["L"])]
+        qs = [(1.5 * torch.randn(B, cfg["H"] * G, Wn, cfg["D"], generator=g, device=device)).to(kv[0][0].dtype)
+              for _ in range(cfg["L"])]
         extra["obs_queries"] = qs
         passes = 1 if kw.get("_vote_lse") else 2
         flops += passes * 2 * 128 * cfg["S"] * cfg["D"] * B * cfg["H"] * cfg["L"]  # 128 = padded query rows of the MMA
@@ -496,9 +506,11 @@ def vote_inputs(cfg, B, kv, device):
     return extra, flops
 
 
-def time_calls(cfg, B, kv, steps, warmup, device, barrier=None, sampler=None, back_to_back=0, sustain_s=0.0):
+def time_calls(cfg, B, kv, steps, warmup, device, barrier=None, sampler=None, back_to_back=0, sustain_s=0.0,
+               outputs=None):
     """`steps` timed passes of the config's calls on `kv` (CUDA events on torch's current stream = the launch stream).
-    Returns (total_ms, per_call list of dicts, launches, vote_flops)."""
+    Returns (total_ms, per_call list of dicts, launches, vote_flops).  `outputs` (a list) receives what each call of
+    the last timed pass returned."""
     import torch
 
     import kvcompress
@@ -514,13 +526,15 @@ def time_calls(cfg, B, kv, steps, warmup, device, barrier=None, sampler=None, ba
         fns.append((kvcompress.get_compress_fn(m), run_kw))
     torch.cuda.synchronize()
 
-    def one_step(events=None):
+    def one_step(events=None, keep=None):
         for i, (fn, kw) in enumerate(fns):
             if events is not None:
                 events[i][0].record()
             out = fn(kv, **kw)
             if events is not None:
                 events[i][1].record()
+            if keep is not None:
+                keep.append(out)
             del out
 
     for _ in range(warmup):
@@ -539,7 +553,7 @@ def time_calls(cfg, B, kv, steps, warmup, device, barrier=None, sampler=None, ba
     t_wall = time.perf_counter()
     t_begin.record()
     for s in range(steps):
-        one_step(ev[s])
+        one_step(ev[s], outputs if s == steps - 1 else None)
     t_end.record()
     if barrier:
         barrier()
@@ -855,6 +869,40 @@ def strong_section(args, device, world, rank, barrier):
     return out
 
 
+# --------------------------------------------------------------------------- output dump
+DUMP_BYTES = 60_000_000  # row data of all files together; the .npy headers and lengths add well under 1 MB
+
+
+def dump_outputs(out_dir, cfg, outputs):
+    """Write what the config's calls returned, one list of (K, V) per call, so that two builds can be compared output
+    for output.  Per call `i` and method `m`:
+
+    * `{i}_{m}_out_len.npy`  float64 [L]: rows each layer came back with;
+    * `{i}_{m}_k.npy`, `{i}_{m}_v.npy`  float32 [rows, D]: for every layer in turn, a sample of its output rows (the
+      (batch, head, position) rows drawn without replacement by numpy's PCG64 seeded with (i, layer), ascending; all
+      rows when a layer has fewer), so that the files together stay under 64 MB.  The sample depends only on the
+      output shapes: equal lengths mean the same rows are compared."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    n_tensors = sum(2 * len(out) for out in outputs)
+    cap = max(1, DUMP_BYTES // (4 * cfg["D"] * n_tensors))   # sampled rows per output tensor
+    for i, ((method, _), out) in enumerate(zip(cfg["calls"], outputs)):
+        lens, ks, vs = [], [], []
+        for li, (k, v) in enumerate(out):
+            B, H, S, _ = k.shape
+            lens.append(S)
+            pick = np.sort(np.random.default_rng([i, li]).choice(B * H * S, size=min(B * H * S, cap), replace=False))
+            b, h, s = (torch.from_numpy(x).to(k.device) for x in np.unravel_index(pick, (B, H, S)))
+            ks.append(k[b, h, s].float().cpu().numpy())
+            vs.append(v[b, h, s].float().cpu().numpy())
+        prefix = os.path.join(out_dir, f"{i}_{method}")
+        np.save(prefix + "_out_len.npy", np.asarray(lens, dtype=np.float64))
+        np.save(prefix + "_k.npy", np.concatenate(ks))
+        np.save(prefix + "_v.npy", np.concatenate(vs))
+
+
 # --------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -889,8 +937,14 @@ def run_ours(args):
     W = max(args.warmup, 3)
     K = args.steps
     sampler = ClockSampler(local)
-    total_ms, per_call_list, launches, vote_flops, _ = time_calls(cfg, B, kv, K, W, device, barrier, sampler)
+    outputs = [] if args.dump_outputs else None
+    total_ms, per_call_list, launches, vote_flops, _ = time_calls(cfg, B, kv, K, W, device, barrier, sampler,
+                                                                  outputs=outputs)
     clocks = sampler.stop()
+    if outputs is not None:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, cfg, outputs)
+        del outputs
     if world > 1:
         t = torch.tensor([total_ms], device=device, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

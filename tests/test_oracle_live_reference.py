@@ -1,11 +1,11 @@
 """Oracle and host planner against the REAL reference, live, on randomly drawn calls.
 
-The committed fixtures (tests/golden/) pin the oracle on 125 hand-picked cases.  Where the reference checkout is
-present (the build container: ``/root/reference``; it never travels to the GPU box, and nothing marked ``gpu`` reads
-it) this module additionally imports the unmodified reference under a private module name and compares, for seeded
-random methods / arguments / shapes / dtypes: output lengths, which layers come back untouched or as views, and the
-kept rows (identical on continuous fp32 data, valid under the tie rule on bf16 and on tie-heavy data).  Skipped
-without the checkout.
+The committed fixtures (tests/golden/) pin the oracle on 125 hand-picked cases.  Where a checkout of the original
+project is named by the ``KVCOMPRESS_REFERENCE`` environment variable (the directory that holds its ``kvcompress``
+package; it is not part of this repository, and nothing marked ``gpu`` reads it) this module additionally imports the
+unmodified reference under a private module name and compares, for seeded random methods / arguments / shapes /
+dtypes: output lengths, which layers come back untouched or as views, and the kept rows (identical on continuous fp32
+data, valid under the tie rule on bf16 and on tie-heavy data).  Skipped without the checkout.
 """
 
 import importlib.util
@@ -20,9 +20,10 @@ import cases
 from oracle import kvc_oracle as O
 from test_planner import plan_for
 
-REF_DIR = "/root/reference/kvcompress"
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF_DIR, "__init__.py")),
-                                reason="reference checkout not present (build container only)")
+REF_ROOT = os.environ.get("KVCOMPRESS_REFERENCE", "")
+REF_DIR = os.path.join(os.path.abspath(REF_ROOT), "kvcompress") if REF_ROOT else ""
+pytestmark = pytest.mark.skipif(not REF_DIR or not os.path.isfile(os.path.join(REF_DIR, "__init__.py")),
+                                reason="KVCOMPRESS_REFERENCE does not name a checkout of the original project")
 
 
 @pytest.fixture(scope="module")
@@ -44,7 +45,7 @@ def ref():
         raise
     finally:
         sys.dont_write_bytecode = dont
-    assert mod.__file__.startswith("/root/reference")
+    assert mod.__file__.startswith(REF_DIR)
     return mod
 
 
