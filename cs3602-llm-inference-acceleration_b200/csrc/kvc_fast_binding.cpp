@@ -70,7 +70,9 @@ public:
                 gather_.push_back((int)i);
                 plans_.push_back(p);
                 // caller-supplied rows / scores need tensors this path does not take
-                if (p.k_sel > 0 && (p.score == KVC_SCORE_GIVEN_INDEX || p.score == KVC_SCORE_GIVEN_SCORE)) simple_ = false;
+                if (p.k_sel > 0 && (p.score == KVC_SCORE_GIVEN_INDEX || p.score == KVC_SCORE_GIVEN_SCORE ||
+                                    p.score == KVC_SCORE_GIVEN_SCORE_SHARED))
+                    simple_ = false;
             } else if (r[0] == VIEW) {
                 simple_ = false;  // views are pure Python slicing: nothing to speed up
             }

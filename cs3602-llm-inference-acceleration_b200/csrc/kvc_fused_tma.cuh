@@ -181,7 +181,8 @@ __global__ void __launch_bounds__(NT, MINB) kvc_fused_tma_kernel(const __grid_co
     const int ksel = L.ksel;
     const int score = L.score;
     const bool kdense = L.kss == RB;
-    const bool by_value = score == KVC_SCORE_GIVEN_SCORE || L.n_in != nullptr;  // per-row values come from memory
+    const bool given_score = score == KVC_SCORE_GIVEN_SCORE || score == KVC_SCORE_GIVEN_SCORE_SHARED;
+    const bool by_value = given_score || L.n_in != nullptr;  // per-row values come from memory
     const bool scan = ksel > 0 && score != KVC_SCORE_GIVEN_INDEX && !by_value;
 
     if (stager) {
@@ -218,8 +219,9 @@ __global__ void __launch_bounds__(NT, MINB) kvc_fused_tma_kernel(const __grid_co
         for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;
         if (tid == 0) misc[kMiscMaxRaw] = 0;
         __syncthreads();
-        if (score == KVC_SCORE_GIVEN_SCORE) {
-            const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)bh * R;
+        if (given_score) {
+            // [B,H,R] per-head rows, or [B,R] rows shared by the heads of a batch entry
+            const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)(score == KVC_SCORE_GIVEN_SCORE ? bh : b) * R;
             load_keys_vectorised<DT, NT>(src, R, keys, [&](int i, uint32_t raw) { keys[i] = (Key)raw; });
             __syncthreads();
             snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc, /*invert=*/false);

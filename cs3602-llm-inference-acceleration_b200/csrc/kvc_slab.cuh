@@ -250,12 +250,13 @@ __global__ void __launch_bounds__(NT, MINB) kvc_slab_compress_kernel(const __gri
         // that a bad index can never become a wild bulk copy
         const int32_t* src = L.idx_in + (int64_t)bh * ksel;
         for (int i = tid; i < ksel; i += NT) sidx[i] = min(max(src[i], 0), L.S - 1);
-    } else if (ksel > 0 && score == KVC_SCORE_GIVEN_SCORE) {
-        // caller-supplied scores of the region's rows ([B,H,R], cache dtype, handed over in the idx_in slot): pooled,
-        // the highest kept (the vote mode of snapkv_lite; same steps as the fused kernel's GIVEN_SCORE branch)
+    } else if (ksel > 0 && (score == KVC_SCORE_GIVEN_SCORE || score == KVC_SCORE_GIVEN_SCORE_SHARED)) {
+        // caller-supplied scores of the region's rows ([B,H,R], or [B,R] shared by the heads of a batch entry; cache
+        // dtype, handed over in the idx_in slot): pooled, the highest kept (the vote mode of snapkv_lite, H2O's
+        // head-summed attention mass; same steps as the fused kernel's GIVEN_SCORE branch)
         for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;
         __syncthreads();
-        const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)bh * R;
+        const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)(score == KVC_SCORE_GIVEN_SCORE ? bh : b) * R;
         load_keys_vectorised<DT, NT>(src, R, keys, [&](int i, uint32_t raw) { keys[i] = (Key)raw; });
         __syncthreads();
         snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc, /*invert=*/false);

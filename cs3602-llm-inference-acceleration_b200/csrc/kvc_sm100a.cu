@@ -23,6 +23,7 @@
 
 #include "kvc_device.cuh"
 #include "kvc_fused_tma.cuh"
+#include "kvc_h2o.cuh"
 #include "kvc_slab.cuh"
 #include "kvc_vote.cuh"
 
@@ -30,9 +31,9 @@
 // times in parallel, each pass keeping one group of entry points (and only the kernels they launch), and links the
 // objects.  KVC_PART is a bit mask: 1 = compress / select / norms entry points (+ the library-wide state) and the
 // bf16 fused kernels, 2 = slab entry points and the bf16 in-place kernels, 4 = vote, 8 = slab append kernels,
-// 16 = f16/f32 fused kernels, 32 = f16/f32 in-place kernels.
+// 16 = f16/f32 fused kernels, 32 = f16/f32 in-place kernels, 64 = H2O score accumulation.
 #ifndef KVC_PART
-#define KVC_PART 63
+#define KVC_PART 127
 #endif
 #define KVC_HAS_CORE (KVC_PART & 1)
 #define KVC_HAS_SLAB (KVC_PART & 2)
@@ -40,6 +41,7 @@
 #define KVC_HAS_APPEND (KVC_PART & 8)
 #define KVC_HAS_FUSED_OTHER (KVC_PART & 16)
 #define KVC_HAS_SLAB_OTHER (KVC_PART & 32)
+#define KVC_HAS_H2O (KVC_PART & 64)
 
 #define KVC_STR2(x) #x
 #define KVC_STR(x) KVC_STR2(x)
@@ -613,10 +615,11 @@ int kvc_compress_layers_ws(const kvc_shape* shape, int32_t n_layers, const kvc_l
         if (p.k_sel > 0) {
             if (p.sel_lo < 0 || p.sel_hi > p.seq_len || p.sel_lo > p.sel_hi) return KVC_ERR_INVALID_ARG;
             if (p.k_sel > p.sel_hi - p.sel_lo) return KVC_ERR_INVALID_ARG;
-            if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE) return KVC_ERR_INVALID_ARG;
+            if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE_SHARED) return KVC_ERR_INVALID_ARG;
+            const bool given_score = p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_GIVEN_SCORE_SHARED;
             if (p.score == KVC_SCORE_GIVEN_INDEX && !x.idx_in) return KVC_ERR_INVALID_ARG;
-            if (p.score == KVC_SCORE_GIVEN_SCORE && !x.score_in) return KVC_ERR_INVALID_ARG;
-            if ((p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_SNAPKV_POOL) && p.pool_kernel > 2 * kMaxPoolHalo)
+            if (given_score && !x.score_in) return KVC_ERR_INVALID_ARG;
+            if ((given_score || p.score == KVC_SCORE_SNAPKV_POOL) && p.pool_kernel > 2 * kMaxPoolHalo)
                 return KVC_ERR_UNSUPPORTED;
         }
         if (C == 0) continue;
@@ -652,7 +655,8 @@ int kvc_compress_layers_ws(const kvc_shape* shape, int32_t n_layers, const kvc_l
             d.k_out = (char*)x.k_out;
             d.v_out = (char*)x.v_out;
             d.idx_out = x.idx_out;
-            d.idx_in = p.score == KVC_SCORE_GIVEN_SCORE ? (const int32_t*)x.score_in : x.idx_in;
+            d.idx_in = (p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_GIVEN_SCORE_SHARED) ? (const int32_t*)x.score_in
+                                                                                              : x.idx_in;
             d.ksb = x.k_stride_b * e;
             d.ksh = x.k_stride_h * e;
             d.kss = x.k_stride_s * e;
@@ -931,10 +935,11 @@ int kvc_slab_compress(const kvc_shape* shape, int32_t n_layers, const kvc_layer_
         if (p.k_sel > 0) {
             if (p.sel_lo < p.sink || p.sel_hi > p.seq_len - p.tail || p.sel_lo > p.sel_hi) return KVC_ERR_INVALID_ARG;
             if (p.k_sel > p.sel_hi - p.sel_lo) return KVC_ERR_INVALID_ARG;
-            if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE) return KVC_ERR_INVALID_ARG;
-            if ((p.score == KVC_SCORE_GIVEN_INDEX || p.score == KVC_SCORE_GIVEN_SCORE) && (!idx_in || !idx_in[l]))
+            if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE_SHARED) return KVC_ERR_INVALID_ARG;
+            const bool given_score = p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_GIVEN_SCORE_SHARED;
+            if ((p.score == KVC_SCORE_GIVEN_INDEX || given_score) && (!idx_in || !idx_in[l]))
                 return KVC_ERR_INVALID_ARG;
-            if ((p.score == KVC_SCORE_SNAPKV_POOL || p.score == KVC_SCORE_GIVEN_SCORE) && p.pool_kernel > 2 * kMaxPoolHalo)
+            if ((p.score == KVC_SCORE_SNAPKV_POOL || given_score) && p.pool_kernel > 2 * kMaxPoolHalo)
                 return KVC_ERR_UNSUPPORTED;
         }
         if (p.sink + p.k_sel + p.tail == 0) continue;
@@ -1197,5 +1202,70 @@ int kvc_snapkv_vote_compress(const kvc_shape* shape, int32_t n_layers, const kvc
 }
 
 #endif  // KVC_HAS_VOTE
+
+#if KVC_HAS_H2O
+int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_layer* layers, float decay,
+                       void* stream) {
+    if (!shape || n_layers < 0 || (n_layers > 0 && !layers)) return KVC_ERR_INVALID_ARG;
+    const int B = shape->batch, H = shape->heads, dt = shape->dtype;
+    if (B <= 0 || H <= 0 || B > 65535) return KVC_ERR_INVALID_ARG;
+    if (dt != KVC_DTYPE_F32 && dt != KVC_DTYPE_F16 && dt != KVC_DTYPE_BF16) return KVC_ERR_UNSUPPORTED;
+    if (n_layers == 0) return KVC_OK;
+    const int e = elem_bytes(dt);
+    for (int l = 0; l < n_layers; ++l) {
+        const kvc_h2o_layer& x = layers[l];
+        if (x.key_len < 0 || !x.acc) return KVC_ERR_INVALID_ARG;
+        if (x.attn && x.n_query <= 0) return KVC_ERR_INVALID_ARG;
+        if (x.score_lo < 0 || x.score_hi < x.score_lo || x.score_hi > x.key_len) return KVC_ERR_INVALID_ARG;
+        if (x.score_hi > x.score_lo && !x.score_out) return KVC_ERR_INVALID_ARG;
+        if (((uintptr_t)x.attn | (uintptr_t)x.acc | (uintptr_t)x.score_out) % e) return KVC_ERR_UNSUPPORTED;
+    }
+    DeviceGuard guard(shape->device);
+    NvtxRange nvtx_range("kvc_h2o_accumulate");
+    if (guard.status != KVC_OK) return guard.status;
+    const int tc = 32 * (16 / e);  // key columns per CTA
+    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
+        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+        H2oBatchDev bd;
+        memset(&bd, 0, sizeof(bd));
+        bd.B = B;
+        bd.H = H;
+        bd.decay = decay;
+        int n_active = 0, max_tiles = 0;
+        for (int l = 0; l < nl; ++l) {
+            const kvc_h2o_layer& x = layers[l0 + l];
+            if (x.key_len == 0) continue;
+            H2oLayerDev& d = bd.layers[n_active++];
+            d.attn = (const char*)x.attn;
+            d.asb = x.a_stride_b * e;
+            d.ash = x.a_stride_h * e;
+            d.asq = x.a_stride_q * e;
+            d.acc = (char*)x.acc;
+            d.csb = x.acc_stride_b * e;
+            d.csh = x.acc_stride_h * e;
+            d.score = x.score_hi > x.score_lo ? (char*)x.score_out : nullptr;
+            d.Q = x.n_query;
+            d.K = x.key_len;
+            d.prev = x.prev_len;
+            d.lo = x.score_lo;
+            d.hi = x.score_hi;
+            d.vec = x.attn && ((uintptr_t)x.attn % 16 == 0) && ((d.asb | d.ash | d.asq) % 16 == 0);
+            const int tiles = (x.key_len + tc - 1) / tc;
+            if (tiles > max_tiles) max_tiles = tiles;
+        }
+        if (n_active == 0) continue;
+        dim3 grid((unsigned)max_tiles, (unsigned)B, (unsigned)n_active);
+        switch (dt) {
+            case KVC_DTYPE_F32: kvc_h2o_accumulate_kernel<KVC_DTYPE_F32><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); break;
+            case KVC_DTYPE_F16: kvc_h2o_accumulate_kernel<KVC_DTYPE_F16><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); break;
+            default: kvc_h2o_accumulate_kernel<KVC_DTYPE_BF16><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); break;
+        }
+        cudaError_t err = cudaGetLastError();
+        if (err != cudaSuccess) return cuda_fail(err, "kvc_h2o_accumulate_kernel launch");
+        g_launches.fetch_add(1);
+    }
+    return KVC_OK;
+}
+#endif  // KVC_HAS_H2O
 
 }  // extern "C"

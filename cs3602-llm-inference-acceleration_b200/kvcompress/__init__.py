@@ -18,6 +18,7 @@ from .methods import (
     h2o_l2_compress,
     h2o_attention_compress,
     H2OAttentionManager,
+    H2OScoreSlab,
     create_h2o_manager_from_model,
     snapkv_lite_compress,
     pyramid_kv_compress,
@@ -40,7 +41,8 @@ from .utils import (
 
 __all__ = [
     "l2_compress", "fix_size_l2_compress", "streaming_llm_compress", "evict_for_space", "recent_only_compress",
-    "h2o_l2_compress", "h2o_attention_compress", "H2OAttentionManager", "create_h2o_manager_from_model",
+    "h2o_l2_compress", "h2o_attention_compress", "H2OAttentionManager", "H2OScoreSlab",
+    "create_h2o_manager_from_model",
     "snapkv_lite_compress", "pyramid_kv_compress", "adaptive_l2_compress",
     "get_compress_fn", "list_methods", "register_method", "COMPRESS_METHODS",
     "to_dynamic_cache", "normalize_kv_cache", "get_cache_size_mb", "get_cache_info", "get_seq_len",

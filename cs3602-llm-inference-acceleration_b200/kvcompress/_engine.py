@@ -37,6 +37,13 @@ KVC_OK = 0
 _STATUS_EXC = {1: ValueError, 2: ValueError, 3: ValueError, 4: RuntimeError}
 
 _RANKED = (P.SCORE_L2_LOW, P.SCORE_L2_HIGH, P.SCORE_SNAPKV_POOL)  # scores derived from key norms
+_GIVEN_SCORES = (P.SCORE_GIVEN_SCORE, P.SCORE_GIVEN_SCORE_SHARED)  # scores supplied by the caller
+
+
+def _score_shape(plan, B: int, H: int) -> tuple:
+    """Shape of the caller-supplied scores of a SCORE_GIVEN_SCORE(_SHARED) plan."""
+    region = plan.sel_hi - plan.sel_lo
+    return (B, region) if plan.score == P.SCORE_GIVEN_SCORE_SHARED else (B, H, region)
 _lib = None
 _WS_NEED = {}  # (plan set, group) -> workspace bytes the launch needs (0: everything fits on chip)
 
@@ -90,6 +97,8 @@ def load_library():
     lib.kvc_snapkv_vote_compress.restype = ctypes.c_int
     lib.kvc_snapkv_vote_compress.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
                                              ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]
+    lib.kvc_h2o_accumulate.restype = ctypes.c_int
+    lib.kvc_h2o_accumulate.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_float, ctypes.c_void_p]
     if lib.kvc_abi_version() != KVC_ABI_VERSION:
         raise RuntimeError(f"{_LIB_NAME}: ABI version {lib.kvc_abi_version()} != {KVC_ABI_VERSION} — rebuild the library")
     _lib = lib
@@ -215,7 +224,8 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
     The outputs of a group with one common length are carved out of ONE allocation.
 
     given_indices: {layer_idx: int32 tensor [B, H, k_sel]} for SCORE_GIVEN_INDEX plans.
-    given_scores: {layer_idx: cache-dtype tensor [B, H, sel_hi - sel_lo]} for SCORE_GIVEN_SCORE plans.
+    given_scores: {layer_idx: cache-dtype tensor [B, H, sel_hi - sel_lo]} for SCORE_GIVEN_SCORE plans,
+        [B, sel_hi - sel_lo] (one row per batch entry, shared by its heads) for SCORE_GIVEN_SCORE_SHARED plans.
     return_indices: also return {layer_idx: int32 tensor [B, H, C]} of kept absolute rows.
     norms: per-layer stored key norms (``[B, H, >= S]``, cache dtype, last dim dense; ``None`` entries allowed) — what
         ``torch.norm(K, p=2, dim=-1)`` returns for the rows.  Layers that have them are ranked from 2-4 bytes per row
@@ -330,13 +340,13 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
                 idx_in_ptr = gi.data_ptr()
                 keepalive.append(gi)
             score_in_ptr = 0
-            if plan.score == P.SCORE_GIVEN_SCORE and plan.k_sel > 0:
+            if plan.score in _GIVEN_SCORES and plan.k_sel > 0:
                 gs = None if given_scores is None else given_scores.get(li)
                 if gs is None:
                     raise ValueError(f"layer {li}: plan needs caller-supplied scores")
-                if gs.dtype != dtype or not gs.is_contiguous() or tuple(gs.shape) != (B, H, plan.sel_hi - plan.sel_lo) \
-                        or gs.device != device:
-                    raise ValueError(f"layer {li}: scores must be a contiguous {dtype} [B, H, region] tensor on {device}")
+                want = _score_shape(plan, B, H)
+                if gs.dtype != dtype or not gs.is_contiguous() or tuple(gs.shape) != want or gs.device != device:
+                    raise ValueError(f"layer {li}: scores must be a contiguous {dtype} {list(want)} tensor on {device}")
                 if on_host and not gs.is_pinned():
                     gs = gs.pin_memory()
                     host_temps = True
@@ -556,3 +566,51 @@ def snapkv_vote_compress(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans,
     if return_votes:
         ret.append(votes_by_layer)
     return ret[0] if len(ret) == 1 else tuple(ret)
+
+
+_H2O = struct.Struct("P3qP2qP6i")  # kvc_h2o_layer: attn | 3 strides | acc | 2 strides | score_out | n_query key_len prev_len
+assert _H2O.size == 88             #                score_lo score_hi reserved
+
+
+def h2o_accumulate(layers: Sequence[tuple], decay: float) -> None:
+    """H2O attention-score bookkeeping for several layers in ONE ``kvc_h2o_accumulate`` launch.
+
+    layers: ``(attn, acc, score_out, prev_len, key_len, score_lo, score_hi)`` per layer —
+      attn ``[B, Hq, n_query, key_len]`` attention probabilities with a dense last dimension, or ``None`` to only
+      re-score; acc ``[B, Hq, >= key_len]`` accumulators (same dtype, dense last dimension), updated in place:
+      ``acc = round(round(acc * decay) + attn.sum(dim=2))`` for ``j < prev_len``, ``attn.sum(dim=2)`` beyond it (from
+      zero when ``prev_len < 0`` or ``> key_len``); score_out ``[>= B * (score_hi - score_lo)]`` dense, or ``None``:
+      ``acc[:, :, score_lo:score_hi].sum(dim=1)`` of the updated accumulators.
+    Every tensor must be a CUDA tensor of one dtype and device, with one (B, Hq); nothing is synchronised."""
+    if not layers:
+        return
+    acc0 = layers[0][1]
+    _require_cuda(acc0, "acc")
+    B, Hq = acc0.size(0), acc0.size(1)
+    buf = bytearray(_H2O.size * len(layers))
+    for m, (attn, acc, score, prev_len, key_len, lo, hi) in enumerate(layers):
+        if acc.dtype != acc0.dtype or acc.device != acc0.device or acc.dim() != 3 or acc.size(0) != B \
+                or acc.size(1) != Hq or acc.size(2) < key_len or acc.stride(2) != 1:
+            raise ValueError(f"layer {m}: acc must be a [B={B}, Hq={Hq}, >= {key_len}] {acc0.dtype} tensor on "
+                             f"{acc0.device} with a dense last dimension")
+        a_ptr, a_st, n_query = 0, (0, 0, 0), 0
+        if attn is not None:
+            _require_cuda(attn, f"layer {m} attention")
+            if attn.dtype != acc0.dtype or attn.device != acc0.device or attn.dim() != 4 or attn.size(0) != B \
+                    or attn.size(1) != Hq or attn.size(3) != key_len or (attn.stride(3) != 1 and key_len > 1):
+                raise ValueError(f"layer {m}: attention must be a [B={B}, Hq={Hq}, n_query, {key_len}] {acc0.dtype} "
+                                 f"tensor on {acc0.device} with a dense last dimension")
+            a_ptr, a_st, n_query = attn.data_ptr(), attn.stride()[:3], attn.size(2)
+        s_ptr = 0
+        if score is not None:
+            if score.dtype != acc0.dtype or score.device != acc0.device or not score.is_contiguous() \
+                    or score.numel() < B * (hi - lo):
+                raise ValueError(f"layer {m}: score_out must be a contiguous {acc0.dtype} tensor of >= B * region "
+                                 f"elements on {acc0.device}")
+            s_ptr = score.data_ptr()
+        _H2O.pack_into(buf, m * _H2O.size, a_ptr, a_st[0], a_st[1], a_st[2], acc.data_ptr(), acc.stride(0),
+                       acc.stride(1), s_ptr, n_query, key_len, prev_len, lo, hi, 0)
+    shape = _SHAPE.pack(B, Hq, 0, KVC_DTYPE[acc0.dtype], acc0.device.index)
+    status = load_library().kvc_h2o_accumulate(shape, len(layers), bytes(buf), float(decay),
+                                               ctypes.c_void_p(_stream_ptr(acc0.device)))
+    _check(status, "kvc_h2o_accumulate")

@@ -27,6 +27,7 @@ SCORE_L2_HIGH = 2
 SCORE_SNAPKV_POOL = 3
 SCORE_GIVEN_INDEX = 4
 SCORE_GIVEN_SCORE = 5
+SCORE_GIVEN_SCORE_SHARED = 6  # GIVEN_SCORE with one [B, region] row per batch entry, shared by its heads
 
 KEEP = "keep"      # layer is returned untouched (the same tensor objects)
 VIEW = "view"      # layer is replaced by the view  x[:, :, -view_n:, :]  (no bytes move)
@@ -190,6 +191,16 @@ def plan_h2o(seq_lens: Sequence[int], start_size: int, heavy_hitter_size: int, r
         num_to_keep = min(heavy_hitter_size, middle_end - middle_start)  # :125
         plans.append(_sandwich(seq_len, start_size, middle_start, middle_end, num_to_keep, recent_size, score))
     return plans
+
+
+def h2o_score_region(seq_len: int, acc_len: int, start_size: int, heavy_hitter_size: int, recent_size: int):
+    """reference h2o_attention.py:153-213 (get_heavy_hitter_indices): the heavy-hitter region ``[lo, hi)`` ranked by
+    accumulators that cover ``acc_len`` keys when the cache holds ``seq_len`` rows, and the number of rows it yields.
+    ``(0, 0, 0)`` when the region is empty."""
+    lo, hi = start_size, min(seq_len, acc_len) - recent_size
+    if hi <= lo:
+        return 0, 0, 0
+    return lo, hi, min(heavy_hitter_size, hi - lo)
 
 
 # --------------------------------------------------------------------------- snapkv_lite

@@ -6,6 +6,10 @@ each cached position receives, and once the cache exceeds ``start_size + heavy_h
 compacted to sinks + heavy hitters + recent rows (the gather runs on the sm_100a kernels with the manager's rows as
 ``KVC_SCORE_GIVEN_INDEX``), after which the manager starts over — positions have moved (reference :164-177).
 
+``cache="slab"`` runs the same loop on a :class:`KVSlabCache` (the model appends in place, ``compress_`` compacts in
+place), as ``evaluate_with_compression`` does.  With an :class:`H2OScoreSlab` as ``h2o_manager`` the score bookkeeping
+runs on the device as well: one accumulate launch per update, one compaction launch per compression.
+
 The model must be able to return attention weights (``attn_implementation="eager"``); ``tokenizer`` only needs
 ``encode(text, return_tensors="pt")`` — pass ``input_ids=`` to skip it (offline runs).
 """
@@ -19,7 +23,7 @@ from typing import Dict, List, Optional
 import torch
 from torch.nn import CrossEntropyLoss
 
-from .evaluate import _EMPTY, _final_cache_size, evaluate_with_compression
+from .evaluate import _EMPTY, _final_cache_size, evaluate_with_compression, new_slab_for_model
 from .methods.h2o_attention import H2OAttentionManager, h2o_attention_compress
 from .utils import normalize_kv_cache, to_dynamic_cache
 
@@ -29,8 +33,11 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                                         heavy_hitter_size: int = 64, recent_size: int = 444, max_tokens: int = 3000,
                                         skip_layers: List[int] = [0, 1], device: Optional[torch.device] = None,
                                         show_progress: bool = True, *, input_ids: Optional[torch.Tensor] = None,
-                                        return_nlls: bool = False) -> Dict[str, float]:
-    """PPL / accuracy / TTFT / TPOT with attention-score H2O applied after every token."""
+                                        cache: str = "dynamic", return_nlls: bool = False) -> Dict[str, float]:
+    """PPL / accuracy / TTFT / TPOT with attention-score H2O applied after every token.  ``h2o_manager``: an
+    :class:`H2OAttentionManager` (the default) or an :class:`H2OScoreSlab`; ``cache``: ``"dynamic"`` or ``"slab"``."""
+    if cache not in ("dynamic", "slab"):
+        raise ValueError(f"cache must be 'dynamic' or 'slab', got {cache!r}")
     if device is None:
         device = next(model.parameters()).device
     if h2o_manager is None:
@@ -49,7 +56,10 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
 
     budget = start_size + heavy_hitter_size + recent_size
     loss_fn = CrossEntropyLoss(reduction="none")
-    past_key_values = None
+    past_key_values = slab = None
+    if cache == "slab":
+        slab = new_slab_for_model(model, input_ids.shape[0], capacity=seq_len, device=device)
+        past_key_values = slab.as_hf_cache()
     nlls, correct, token_times = [], [], []
     ttft = None
     steps = range(seq_len - 1)
@@ -72,17 +82,25 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
             target = input_ids[:, idx + 1:idx + 2].view(-1)
             nlls.append(float(loss_fn(logits, target).mean().item()))
             correct.append(float((torch.argmax(logits, dim=-1) == target).float().mean().item()))
-            past_key_values = outputs.past_key_values
             attentions = outputs.attentions
-            h2o_manager.update_attention_scores(attentions, skip_layers)
-            if past_key_values is not None:
-                kv_list = list(normalize_kv_cache(past_key_values))
-                if kv_list and kv_list[0][0].size(2) > budget:
-                    kept = h2o_attention_compress(kv_list, attention_scores=attentions, h2o_manager=h2o_manager,
-                                                  start_size=start_size, heavy_hitter_size=heavy_hitter_size,
-                                                  recent_size=recent_size, skip_layers=skip_layers)
-                    past_key_values = to_dynamic_cache(kept)
+            if slab is not None:
+                h2o_manager.update_attention_scores(attentions, skip_layers)
+                if slab.lengths[0] > budget:
+                    slab.compress_("h2o_attention", attention_scores=attentions, h2o_manager=h2o_manager,
+                                   start_size=start_size, heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
+                                   skip_layers=skip_layers)
                     h2o_manager.reset()
+            else:
+                past_key_values = outputs.past_key_values
+                h2o_manager.update_attention_scores(attentions, skip_layers)
+                if past_key_values is not None:
+                    kv_list = list(normalize_kv_cache(past_key_values))
+                    if kv_list and kv_list[0][0].size(2) > budget:
+                        kept = h2o_attention_compress(kv_list, attention_scores=attentions, h2o_manager=h2o_manager,
+                                                      start_size=start_size, heavy_hitter_size=heavy_hitter_size,
+                                                      recent_size=recent_size, skip_layers=skip_layers)
+                        past_key_values = to_dynamic_cache(kept)
+                        h2o_manager.reset()
             token_time = time.perf_counter() - token_start
             token_times.append(token_time)
             if ttft is None:
@@ -90,7 +108,10 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
     total_time = time.perf_counter() - total_start
 
     num_tokens = len(nlls)
-    lengths = [k.size(2) for k, _ in normalize_kv_cache(past_key_values)] if past_key_values is not None else []
+    if slab is not None:
+        lengths = list(slab.lengths)
+    else:
+        lengths = [k.size(2) for k, _ in normalize_kv_cache(past_key_values)] if past_key_values is not None else []
     result = {
         "perplexity": math.exp(sum(nlls) / num_tokens),
         "accuracy": sum(correct) / num_tokens,

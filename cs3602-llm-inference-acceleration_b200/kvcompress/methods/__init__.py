@@ -22,6 +22,7 @@ _METHOD_TABLE = (
 _EXTRA_EXPORTS = (
     ("streaming_llm", "evict_for_space"),
     ("h2o_attention", "H2OAttentionManager"),
+    ("h2o_attention", "H2OScoreSlab"),
     ("h2o_attention", "create_h2o_manager_from_model"),
 )
 

@@ -9,15 +9,21 @@ resolves and behaves as in the reference:
 * with a manager, the manager's head-summed top-k indices (shared by every batch entry and head,
   h2o_attention.py:194-213, :318-331) are handed to the gather kernel as caller-supplied indices.
 
-The score bookkeeping itself (`H2OAttentionManager`) is small torch arithmetic on the model's
-attention outputs and stays in torch.
+Two managers keep the score bookkeeping:
+
+* `H2OAttentionManager` mirrors the reference's object model in torch arithmetic (CPU or GPU tensors, batch 1);
+* `H2OScoreSlab` keeps the decayed accumulators and the head-summed score rows in preallocated device buffers:
+  one ``kvc_h2o_accumulate`` launch per update for every layer, and the compaction ranks the rows from the score
+  row itself (``KVC_SCORE_GIVEN_SCORE_SHARED``) — no ATen kernel and no host synchronisation on the decode path,
+  and every batch entry gets its own heavy hitters.
 """
 
+from collections.abc import Mapping
 from typing import Dict, List, Optional, Tuple
 
 import torch
 
-from .. import _planner
+from .. import _engine, _planner
 from ._common import as_layer_list, cached_plans, execute, seq_lens
 
 
@@ -99,6 +105,13 @@ def h2o_attention_compress(past_key_values, attention_scores=None, h2o_manager: 
     if h2o_manager is None:
         return execute(layers, plans)
 
+    if isinstance(h2o_manager, H2OScoreSlab):
+        keys = next((layers[li][0] for li in plans.gather), None)
+        if keys is None:
+            return execute(layers, plans)
+        plans, given, scores = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,
+                                                          keys.size(0), keys.size(1), keys.dtype, keys.device)
+        return _engine.run_plans(layers, plans, given_indices=given, given_scores=scores)
     plans, given = manager_plans(layers, plans, h2o_manager, heavy_hitter_size)
     return execute(layers, plans, given_indices=given)
 
@@ -130,6 +143,240 @@ def manager_plans(layers, plans, h2o_manager: H2OAttentionManager, heavy_hitter_
     return plans, given
 
 
+class _AccumulatorViews(Mapping):
+    """``accumulated_attention`` of an :class:`H2OScoreSlab`: layer -> ``[B, Hq, key_len]`` view of the device
+    accumulators (read-only: the next update overwrites them in place)."""
+
+    def __init__(self, owner: "H2OScoreSlab"):
+        self._owner = owner
+
+    def __getitem__(self, layer_idx: int) -> torch.Tensor:
+        n = self._owner._lens[layer_idx]
+        return self._owner._acc[layer_idx, :, :, :n]
+
+    def __iter__(self):
+        return iter(sorted(self._owner._lens))
+
+    def __len__(self) -> int:
+        return len(self._owner._lens)
+
+
+class H2OScoreSlab:
+    """Device-resident H2O score bookkeeping: a drop-in for :class:`H2OAttentionManager` (same constructor
+    arguments plus ``capacity``, same methods) wherever ``h2o_manager=`` is accepted.
+
+    The decayed accumulators live in one ``[num_layers, B, Hq, capacity]`` buffer next to one
+    ``[num_layers, B, capacity]`` buffer of head-summed score rows, both in the attention dtype, allocated on the
+    first update and doubled when a ``key_len`` exceeds ``capacity``.  ``update_attention_scores`` is ONE
+    ``kvc_h2o_accumulate`` launch for every layer it updates: the accumulator update with the reference's rounding
+    points (bit-identical to the torch manager for one query per step) and the score row of the heavy-hitter region
+    ``[start_size, key_len - recent_size)``.  At compression the score row is handed to the compaction as
+    ``KVC_SCORE_GIVEN_SCORE_SHARED``: each batch entry keeps its own heavy hitters, shared by its KV heads (the sum
+    runs over all ``Hq`` query heads, so GQA models need nothing else).  The host decides everything from integers it
+    holds — no ``.item()``, no synchronisation.  ``reset`` touches no device memory."""
+
+    def __init__(self, start_size: int = 4, heavy_hitter_size: int = 64, recent_size: int = 444,
+                 num_layers: int = 32, num_heads: int = 32, decay_factor: float = 0.9, device=None,
+                 capacity: Optional[int] = None):
+        self.start_size = start_size
+        self.heavy_hitter_size = heavy_hitter_size
+        self.recent_size = recent_size
+        self.total_cache_size = start_size + heavy_hitter_size + recent_size
+        self.num_layers = num_layers
+        self.num_heads = num_heads
+        self.decay_factor = decay_factor
+        self.device = device
+        self.capacity = capacity
+        self.current_seq_len = 0
+        self._acc: Optional[torch.Tensor] = None    # [L, B, Hq, capacity]
+        self._score: Optional[torch.Tensor] = None  # [L, B, capacity]; row l holds [B, hi - lo] densely
+        self._lens: Dict[int, int] = {}             # layer -> valid accumulator entries (the torch manager's size(-1))
+        self._scored: Dict[int, Tuple[int, int]] = {}  # layer -> (lo, hi) its score row currently holds
+        self._gen = 0                               # bumped whenever the buffers are reallocated
+        self._plan_cache: Dict[tuple, tuple] = {}
+
+    @property
+    def accumulated_attention(self) -> Mapping:
+        return _AccumulatorViews(self)
+
+    def reset(self) -> None:
+        self._lens = {}
+        self._scored = {}
+        self.current_seq_len = 0
+
+    # ------------------------------------------------------------------ buffers
+    def _ensure(self, batch: int, heads: int, dtype: torch.dtype, device: torch.device, need: int) -> None:
+        acc = self._acc
+        if acc is not None and (acc.shape[1:3] != (batch, heads) or acc.dtype != dtype or acc.device != device):
+            if self._lens:
+                raise ValueError(f"H2OScoreSlab: attention [B={batch}, Hq={heads}] {dtype} on {device} does not match "
+                                 f"the accumulators [B={acc.size(1)}, Hq={acc.size(2)}] {acc.dtype} on {acc.device}; "
+                                 "call reset() first")
+            acc = None
+        if acc is None:
+            cap = max(self.capacity or 0, need, 1)
+        elif need > acc.size(3):
+            cap = acc.size(3)
+            while cap < need:
+                cap *= 2
+        else:
+            return
+        new_acc = torch.empty((self.num_layers, batch, heads, cap), dtype=dtype, device=device)
+        if acc is not None:
+            new_acc[..., :acc.size(3)].copy_(acc)
+        # score rows are dense [B, region] inside a row of the buffer: they do not survive a change of pitch, and are
+        # produced again by the update that follows or, for the other layers, at the next compression
+        self._acc, self.capacity = new_acc, cap
+        self._score = torch.empty((self.num_layers, batch, cap), dtype=dtype, device=device)
+        self._scored = {}
+        self._gen += 1
+        self._plan_cache.clear()
+
+    def _score_row(self, layer_idx: int, batch: int, region: int) -> torch.Tensor:
+        return self._score[layer_idx].view(-1)[:batch * region].view(batch, region)
+
+    def _rescore(self, layers: List[Tuple[int, int, int]]) -> None:
+        """Score rows of [lo, hi) from the accumulators as they are (attn = NULL), every layer in one launch."""
+        recs = []
+        for li, lo, hi in layers:
+            n = self._lens[li]
+            recs.append((None, self._acc[li], self._score[li], n, n, lo, hi))
+            self._scored[li] = (lo, hi)
+        _engine.h2o_accumulate(recs, self.decay_factor)
+
+    # ------------------------------------------------------------------ the manager's interface
+    def update_attention_scores(self, attentions, skip_layers: List[int] = []) -> None:
+        """acc <- decay * acc (zero-extended, or reset if the cache shrank) + attn.sum(query dim), and the score row of
+        [start_size, key_len - recent_size) — one launch for every non-skipped, non-``None`` layer."""
+        if attentions is None:
+            return
+        work = []
+        for layer_idx, attn in enumerate(attentions):
+            if layer_idx in skip_layers or attn is None:
+                continue
+            if layer_idx >= self.num_layers:
+                raise ValueError(f"H2OScoreSlab: layer {layer_idx} >= num_layers={self.num_layers}")
+            if attn.dim() != 4:
+                raise ValueError(f"layer {layer_idx}: attention must be [B, Hq, n_query, key_len]")
+            work.append((layer_idx, attn if attn.stride(-1) == 1 else attn.contiguous()))
+        if not work:
+            return
+        a0 = work[0][1]
+        _engine._require_cuda(a0, "attention")
+        self._ensure(a0.size(0), a0.size(1), a0.dtype, a0.device, max(a.size(3) for _, a in work))
+        recs = []
+        for layer_idx, attn in work:
+            key_len = attn.size(3)
+            lo, hi, _ = _planner.h2o_score_region(key_len, key_len, self.start_size, self.heavy_hitter_size,
+                                                  self.recent_size)
+            recs.append((attn, self._acc[layer_idx], self._score[layer_idx], self._lens.get(layer_idx, -1), key_len,
+                         lo, hi))
+            self._lens[layer_idx] = key_len
+            self._scored[layer_idx] = (lo, hi)
+            self.current_seq_len = key_len
+        _engine.h2o_accumulate(recs, self.decay_factor)
+
+    def get_heavy_hitter_indices(self, layer_idx: int, seq_len: int) -> torch.Tensor:
+        """Indices (relative to the middle region, ascending) of its heaviest tokens — what
+        :meth:`H2OAttentionManager.get_heavy_hitter_indices` returns, selected on the device (``kvc_select``)."""
+        n = self._lens.get(layer_idx)
+        if n is None:  # no data: evenly spaced  (:167-177)
+            middle_len = (seq_len - self.recent_size) - self.start_size
+            if middle_len <= 0:
+                return torch.tensor([], dtype=torch.long)
+            step = max(1, middle_len // self.heavy_hitter_size)
+            return torch.arange(0, middle_len, step)[: self.heavy_hitter_size]
+        lo, hi, k = _planner.h2o_score_region(seq_len, n, self.start_size, self.heavy_hitter_size, self.recent_size)
+        if k == 0:
+            return torch.tensor([], dtype=torch.long, device=self._acc.device)
+        if self._scored.get(layer_idx) != (lo, hi):
+            self._rescore([(layer_idx, lo, hi)])
+        batch = self._acc.size(1)
+        top = _engine.select(self._score_row(layer_idx, batch, hi - lo), k, largest=True).long()
+        return top.squeeze(0) if batch == 1 else top
+
+    # ------------------------------------------------------------------ compaction
+    def compress_plans(self, plans, start_size: int, heavy_hitter_size: int, recent_size: int, batch: int, heads: int,
+                       dtype: torch.dtype, device):
+        """The h2o plans rewritten with this manager's heavy hitters (reference h2o_attention.py:318-331) for a cache
+        of ``[batch, heads, S, D]`` ``dtype`` layers.  Returns ``(PlanSet, given_indices, given_scores)``: layers with
+        accumulated scores rank ``[sel_lo, sel_lo + region)`` by their score row (``SCORE_GIVEN_SCORE_SHARED``), layers
+        without data since the last reset keep evenly spaced rows (``SCORE_GIVEN_INDEX``), an empty region keeps no
+        heavy hitter.  Score rows whose region differs from the last update's are re-scored in one launch."""
+        device = torch.device(device)
+        decisions, rescore = [], []
+        for li in plans.gather:
+            p = plans.plans[li]
+            if p.region == 0:
+                decisions.append(None)
+                continue
+            S, middle_len = p.seq_len, p.sel_hi - p.sel_lo
+            n = self._lens.get(li)
+            if n is None:
+                m_len = (S - self.recent_size) - self.start_size
+                picked = range(0, m_len, max(1, m_len // self.heavy_hitter_size))[: self.heavy_hitter_size] \
+                    if m_len > 0 else range(0)
+                decisions.append(("even", m_len, len(picked), min(len(picked), heavy_hitter_size, middle_len)))
+                continue
+            lo, hi, k = _planner.h2o_score_region(S, n, self.start_size, self.heavy_hitter_size, self.recent_size)
+            if k == 0:
+                decisions.append(("none",))
+                continue
+            region = hi - lo
+            count = min(k, heavy_hitter_size, middle_len)  # :321
+            if count != k or region > middle_len:
+                raise ValueError(f"layer {li}: H2OScoreSlab(start_size={self.start_size}, heavy_hitter_size="
+                                 f"{self.heavy_hitter_size}, recent_size={self.recent_size}) selects {k} of {region} rows, "
+                                 f"the compression keeps {count} of {middle_len}: use the same sizes for both")
+            if self._acc.dtype != dtype:
+                raise ValueError(f"H2OScoreSlab: the attention dtype {self._acc.dtype} differs from the cache dtype "
+                                 f"{dtype}")
+            if self._acc.size(1) != batch or self._acc.device != device:
+                raise ValueError(f"H2OScoreSlab: accumulators of batch {self._acc.size(1)} on {self._acc.device}, "
+                                 f"cache of batch {batch} on {device}")
+            if self._scored.get(li) != (lo, hi):
+                rescore.append((li, lo, hi))
+            decisions.append(("score", region, count))
+        if rescore:
+            self._rescore(rescore)
+        key = (id(plans), self._gen, batch, heads, device, tuple(decisions))
+        hit = self._plan_cache.get(key)
+        if hit is not None and hit[0] is plans:
+            return hit[1], hit[2], hit[3]
+        new_plans, given, scores = list(plans.plans), {}, {}
+        for li, d in zip(plans.gather, decisions):
+            if d is None:
+                continue
+            p = plans.plans[li]
+            middle_len = p.sel_hi - p.sel_lo
+            count = 0 if d[0] == "none" else d[-1]
+            score = _planner.SCORE_NONE
+            sel_hi = p.sel_hi
+            if count > 0 and d[0] == "even":
+                m_len, n_picked = d[1], d[2]
+                step = max(1, m_len // self.heavy_hitter_size)
+                rows = [min(max(x, 0), middle_len - 1) + p.sel_lo for x in range(0, m_len, step)[:count]]
+                if any(b <= a for a, b in zip(rows, rows[1:])):
+                    raise ValueError(f"layer {li}: evenly spaced rows {rows[:4]}... collide after clamping into the "
+                                     f"region of {middle_len} rows")
+                given[li] = (torch.arange(0, m_len, step, device=device, dtype=torch.int32)[:count]
+                             .clamp_(0, middle_len - 1).add_(p.sel_lo)
+                             .view(1, 1, count).expand(batch, heads, count).contiguous())
+                score = _planner.SCORE_GIVEN_INDEX
+            elif count > 0:
+                region = d[1]
+                sel_hi = p.sel_lo + region
+                scores[li] = self._score_row(li, batch, region)
+                score = _planner.SCORE_GIVEN_SCORE_SHARED
+            new_plans[li] = _planner.LayerPlan(_planner.GATHER, p.seq_len, sink=p.sink, sel_lo=p.sel_lo, sel_hi=sel_hi,
+                                               k_sel=count, tail=p.tail, score=score)
+        ps = _engine.PlanSet(new_plans)
+        if len(self._plan_cache) > 64:
+            self._plan_cache.clear()
+        self._plan_cache[key] = (plans, ps, given or None, scores or None)
+        return ps, given or None, scores or None
+
+
 def create_h2o_manager_from_model(model, **kwargs) -> H2OAttentionManager:
     """Manager sized from ``model.config`` (reference h2o_attention.py:366-391)."""
     config = model.config
@@ -144,4 +391,5 @@ def create_h2o_manager_from_model(model, **kwargs) -> H2OAttentionManager:
     )
 
 
-__all__ = ["H2OAttentionManager", "h2o_attention_compress", "create_h2o_manager_from_model", "manager_plans"]
+__all__ = ["H2OAttentionManager", "H2OScoreSlab", "h2o_attention_compress", "create_h2o_manager_from_model",
+           "manager_plans"]

@@ -416,7 +416,7 @@ class KVSlabCache:
         ``h2o_l2`` (:337-351); with one, its head-summed heavy hitters are the caller-supplied rows of the in-place
         compaction (they must ascend strictly — the manager sorts them, a clamp collision is refused)."""
         from .methods._common import cached_plans
-        from .methods.h2o_attention import manager_plans
+        from .methods.h2o_attention import H2OScoreSlab, manager_plans
 
         if h2o_manager is None:
             return self.compress_("h2o_l2", return_indices=return_indices, start_size=start_size,
@@ -424,6 +424,10 @@ class KVSlabCache:
         if attention_scores is not None:
             h2o_manager.update_attention_scores(attention_scores, list(skip_layers))
         plans = cached_plans(P.plan_h2o, self.lengths, start_size, heavy_hitter_size, recent_size, skip_layers=skip_layers)
+        if isinstance(h2o_manager, H2OScoreSlab):  # scores ranked on the device: no host round trip
+            plans, given, scores = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,
+                                                              self.batch, self.heads, self.dtype, self.device)
+            return self.apply_plans_(plans, given_indices=given, given_scores=scores, return_indices=return_indices)
         plans, given = manager_plans(self.to_legacy_cache(), plans, h2o_manager, heavy_hitter_size)
         for li, rows in given.items():
             if rows.size(-1) > 1 and not bool((rows[0, 0, 1:] > rows[0, 0, :-1]).all()):
@@ -481,11 +485,11 @@ class KVSlabCache:
             ptrs = (ctypes.c_void_p * len(ids))()
             for m, i in enumerate(ids):
                 gs = given_scores.get(i) if given_scores else None
-                if gs is not None:  # SCORE_GIVEN_SCORE: the region's scores travel in the idx_in slot (kvc.h)
-                    region = ps.plans[i].sel_hi - ps.plans[i].sel_lo
+                if gs is not None:  # SCORE_GIVEN_SCORE(_SHARED): the region's scores travel in the idx_in slot (kvc.h)
+                    want = _engine._score_shape(ps.plans[i], self.batch, self.heads)
                     if gs.dtype != self.dtype or not gs.is_contiguous() or gs.device != self.device \
-                            or tuple(gs.shape) != (self.batch, self.heads, region):
-                        raise ValueError(f"layer {i}: scores must be a contiguous {self.dtype} [B, H, {region}] tensor "
+                            or tuple(gs.shape) != want:
+                        raise ValueError(f"layer {i}: scores must be a contiguous {self.dtype} {list(want)} tensor "
                                          f"on {self.device}")
                     keep.append(gs)
                     ptrs[m] = gs.data_ptr()

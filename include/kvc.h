@@ -46,6 +46,9 @@
 extern "C" {
 #endif
 
+/* Additions that leave every existing struct layout, enum value and entry point as it was (a new score kind, the
+ * kvc_h2o_layer struct and kvc_h2o_accumulate) keep the version: a caller built against an older header sees the
+ * same ABI, and a caller that uses the additions fails to link or gets KVC_ERR_INVALID_ARG from an older library. */
 #define KVC_ABI_VERSION 5
 
 typedef enum kvc_status {
@@ -69,8 +72,11 @@ typedef enum kvc_score_kind {
     KVC_SCORE_L2_HIGH = 2,     /* keep the k_sel highest ||K||_2  (argsort(descending=True)[:k])    */
     KVC_SCORE_SNAPKV_POOL = 3, /* (max norm + 1e-6 - norm) -> avg_pool1d -> topk (snapkv_lite.py:96-134) */
     KVC_SCORE_GIVEN_INDEX = 4, /* caller supplies ascending absolute row indices (fix_size_l2 "random") */
-    KVC_SCORE_GIVEN_SCORE = 5  /* caller supplies per-row scores (score_in): avg_pool1d(pool_kernel) -> keep the
+    KVC_SCORE_GIVEN_SCORE = 5, /* caller supplies per-row scores (score_in): avg_pool1d(pool_kernel) -> keep the
                                   k_sel HIGHEST (snapkv vote mode: kvc_snapkv_vote output; h2o_attention.py:194-213) */
+    KVC_SCORE_GIVEN_SCORE_SHARED = 6 /* as GIVEN_SCORE, but score_in is [B, sel_hi-sel_lo] (cache dtype, dense): ONE
+                                        row per batch entry, used by every head (H2O's head-summed attention mass,
+                                        h2o_attention.py:194-213; kvc_h2o_accumulate's score_out) */
 } kvc_score_kind;
 
 /* One layer's keep-plan: integers computed by the host planner (reference arithmetic). */
@@ -233,6 +239,36 @@ int kvc_slab_append(const kvc_shape* shape, int32_t n_layers, const kvc_slab_lay
 int kvc_slab_compress(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
                       const kvc_slab_layer* slabs, int32_t* const* idx_out, const int32_t* const* idx_in,
                       void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * H2O attention-score bookkeeping (reference h2o_attention.py:78-213) on the device.
+ *
+ * Per layer, per batch entry b, query head h and key j < key_len, with fp32 arithmetic and a rounding to the
+ * attention dtype at exactly the points where the reference's torch expressions round:
+ *   mass             = round( sum_q fp32(attn[b,h,q,j]) )               (attn.sum(dim=2))
+ *   acc[b,h,j]       = round( fp32(round(fp32(acc[b,h,j]) * decay)) + fp32(mass) )   j <  prev_len
+ *   acc[b,h,j]       = mass                                                          j >= prev_len
+ *   score_out[b, j - score_lo] = round( sum_h fp32(acc[b,h,j]) ),  score_lo <= j < score_hi
+ * prev_len < 0 or prev_len > key_len: every acc entry starts from zero (the reference's reset when the cache
+ * shrank).  The query sum runs over fixed, contiguous query blocks in ascending order, the blocks then added in
+ * ascending order; with n_query = 1 mass is attn itself.  The head sum runs in ascending h.  attn == NULL: acc is
+ * neither read for an update nor written, only score_out is produced from it.  score_out may be NULL (or
+ * score_lo == score_hi) when no score row is wanted.  One launch covers every layer (KVC_MAX_LAYERS_PER_LAUNCH
+ * chunks); feed score_out to kvc_compress_layers / kvc_slab_compress as KVC_SCORE_GIVEN_SCORE_SHARED. */
+typedef struct kvc_h2o_layer {
+    const void* attn;        /* [B, Hq, n_query, key_len] attention probabilities, last dim dense; NULL: re-score only */
+    int64_t a_stride_b, a_stride_h, a_stride_q; /* elements */
+    void* acc;               /* [B, Hq, >= key_len] accumulators, attention dtype, last dim dense */
+    int64_t acc_stride_b, acc_stride_h;         /* elements */
+    void* score_out;         /* optional [B, score_hi - score_lo], dense: sum over heads of the updated acc */
+    int32_t n_query, key_len;
+    int32_t prev_len;        /* valid acc entries before the update; < 0 or > key_len: start from zero */
+    int32_t score_lo, score_hi;
+    int32_t reserved;
+} kvc_h2o_layer;
+/* shape: batch = B, heads = Hq (query heads), dtype = the attention dtype, device; head_dim is not used. */
+int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_layer* layers, float decay,
+                       void* stream);
 
 #ifdef __cplusplus
 }
