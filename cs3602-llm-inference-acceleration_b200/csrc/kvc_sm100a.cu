@@ -1266,6 +1266,153 @@ int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_l
     }
     return KVC_OK;
 }
+
+// ------------------------------------------------------------------ kvc_h2o_accumulate_qk
+// Pass-1 key splits: at most kQkMaxSplits, each a whole number of 128-row tiles (a function of key_len only).
+static void qk_splits(int key_len, int* n_split, int* split_tiles) {
+    const int tiles = (key_len + kQkRows - 1) / kQkRows;
+    const int want = tiles < kQkMaxSplits ? tiles : kQkMaxSplits;
+    *split_tiles = want > 0 ? (tiles + want - 1) / want : 1;
+    *n_split = want > 0 ? (tiles + *split_tiles - 1) / *split_tiles : 0;
+}
+
+static int64_t qk_layer_ws(const kvc_shape* shape, int group, const kvc_h2o_qk_layer& x) {
+    if (x.key_len <= 0) return 0;
+    int n_split, split_tiles;
+    qk_splits(x.key_len, &n_split, &split_tiles);
+    const int64_t bytes = (int64_t)shape->batch * shape->heads * group * x.n_query * n_split * 8;
+    return (bytes + 255) & ~(int64_t)255;
+}
+
+static int qk_validate(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers) {
+    if (!shape || n_layers < 0 || (n_layers > 0 && !layers) || group < 1) return KVC_ERR_INVALID_ARG;
+    const int B = shape->batch, H = shape->heads, D = shape->head_dim, dt = shape->dtype;
+    if (B <= 0 || H <= 0 || D <= 0 || (int64_t)B * H > 65535) return KVC_ERR_INVALID_ARG;
+    if (dt != KVC_DTYPE_F32 && dt != KVC_DTYPE_F16 && dt != KVC_DTYPE_BF16) return KVC_ERR_UNSUPPORTED;
+    const int e = elem_bytes(dt);
+    if ((D * e) % 16 || D * e > kQkMaxRowBytes) return KVC_ERR_UNSUPPORTED;
+    for (int l = 0; l < n_layers; ++l) {
+        const kvc_h2o_qk_layer& x = layers[l];
+        if (x.key_len < 0 || x.n_query <= 0 || !x.acc || !x.q || !x.k) return KVC_ERR_INVALID_ARG;
+        if (!x.mask && x.n_query > x.key_len) return KVC_ERR_INVALID_ARG;
+        if (x.score_lo < 0 || x.score_hi < x.score_lo || x.score_hi > x.key_len) return KVC_ERR_INVALID_ARG;
+        if (x.score_hi > x.score_lo && !x.score_out) return KVC_ERR_INVALID_ARG;
+        if (((uintptr_t)x.q | (uintptr_t)x.acc | (uintptr_t)x.score_out) % e) return KVC_ERR_UNSUPPORTED;
+        if ((uintptr_t)x.k % 16 || (x.k_stride_b * e) % 16 || (x.k_stride_h * e) % 16 || (x.k_stride_s * e) % 16)
+            return KVC_ERR_UNSUPPORTED;
+    }
+    return KVC_OK;
+}
+
+int64_t kvc_h2o_qk_workspace_bytes(const kvc_shape* shape, int32_t group, int32_t n_layers,
+                                   const kvc_h2o_qk_layer* layers) {
+    if (qk_validate(shape, group, n_layers, layers) != KVC_OK) return -1;
+    int64_t total = 0;
+    for (int l = 0; l < n_layers; ++l) total += qk_layer_ws(shape, group, layers[l]);
+    return total;
+}
+
+using QkFn = void (*)(const H2oQkBatchDev);
+
+extern "C++" {
+template <int DT>
+static QkFn pick_qk(bool stats, int qt) {
+    if (stats) return qt == 8 ? kvc_h2o_qk_stats_kernel<DT, 8> : qt == 4 ? kvc_h2o_qk_stats_kernel<DT, 4>
+                                                                          : kvc_h2o_qk_stats_kernel<DT, 1>;
+    return qt == 8 ? kvc_h2o_qk_accumulate_kernel<DT, 8> : qt == 4 ? kvc_h2o_qk_accumulate_kernel<DT, 4>
+                                                                   : kvc_h2o_qk_accumulate_kernel<DT, 1>;
+}
+}
+
+int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers,
+                          float decay, void* workspace, int64_t workspace_bytes, void* stream) {
+    const int v = qk_validate(shape, group, n_layers, layers);
+    if (v != KVC_OK) return v;
+    int64_t need = 0;
+    for (int l = 0; l < n_layers; ++l) need += qk_layer_ws(shape, group, layers[l]);
+    if (need > 0 && (!workspace || workspace_bytes < need || (uintptr_t)workspace % 16)) return KVC_ERR_INVALID_ARG;
+    if (need == 0) return KVC_OK;  // every layer has key_len 0
+    DeviceGuard guard(shape->device);
+    NvtxRange nvtx_range("kvc_h2o_accumulate_qk");
+    if (guard.status != KVC_OK) return guard.status;
+    const int B = shape->batch, Hkv = shape->heads, D = shape->head_dim, dt = shape->dtype;
+    const int e = elem_bytes(dt);
+    const int rb = D * e, pitch = ((rb / 16) | 1) * 16;
+    char* ws = (char*)workspace;
+    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
+        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+        H2oQkBatchDev bd;
+        memset(&bd, 0, sizeof(bd));
+        bd.B = B;
+        bd.Hkv = Hkv;
+        bd.G = group;
+        bd.D = D;
+        bd.decay = decay;
+        bd.pitch = pitch;
+        int n_active = 0, max_x1 = 0, max_tiles = 0, max_gt = 0;
+        for (int l = 0; l < nl; ++l) {
+            const kvc_h2o_qk_layer& x = layers[l0 + l];
+            if (x.key_len == 0) continue;
+            H2oQkLayerDev& d = bd.layers[n_active++];
+            d.q = (const char*)x.q;
+            d.qsb = x.q_stride_b * e;
+            d.qsh = x.q_stride_h * e;
+            d.qst = x.q_stride_t * e;
+            d.k = (const char*)x.k;
+            d.ksb = x.k_stride_b * e;
+            d.ksh = x.k_stride_h * e;
+            d.kss = x.k_stride_s * e;
+            d.mask = x.mask;
+            d.msb = x.m_stride_b;
+            d.mst = x.m_stride_t;
+            d.acc = (char*)x.acc;
+            d.csb = x.acc_stride_b * e;
+            d.csh = x.acc_stride_h * e;
+            d.score = x.score_hi > x.score_lo ? (char*)x.score_out : nullptr;
+            d.ws = (float2*)ws;
+            ws += qk_layer_ws(shape, group, x);
+            d.scaling = x.scaling;
+            d.T = x.n_query;
+            d.K = x.key_len;
+            d.prev = x.prev_len;
+            d.lo = x.score_lo;
+            d.hi = x.score_hi;
+            qk_splits(x.key_len, &d.n_split, &d.split_tiles);
+            const int gt = group * x.n_query;
+            d.n_qt = (gt + kQkQ1 - 1) / kQkQ1;
+            if (d.n_split * d.n_qt > max_x1) max_x1 = d.n_split * d.n_qt;
+            const int tiles = (x.key_len + kQkRows - 1) / kQkRows;
+            if (tiles > max_tiles) max_tiles = tiles;
+            if (gt > max_gt) max_gt = gt;
+        }
+        if (n_active == 0) continue;
+        // queries per register tile: the work of a (query, key) pair does not depend on it, only the speed does
+        const int qt = max_gt >= 8 ? 8 : max_gt >= 4 ? 4 : 1;
+        QkFn stats, accum;
+        switch (dt) {
+            case KVC_DTYPE_F32: stats = pick_qk<KVC_DTYPE_F32>(true, qt); accum = pick_qk<KVC_DTYPE_F32>(false, qt); break;
+            case KVC_DTYPE_F16: stats = pick_qk<KVC_DTYPE_F16>(true, qt); accum = pick_qk<KVC_DTYPE_F16>(false, qt); break;
+            default: stats = pick_qk<KVC_DTYPE_BF16>(true, qt); accum = pick_qk<KVC_DTYPE_BF16>(false, qt); break;
+        }
+        const size_t smem_k = 128 + 2 * (size_t)kQkRows * pitch;
+        const size_t smem1 = smem_k + (size_t)kQkQ1 * D * 4 + 2 * (size_t)kQkQ1 * kQkThreads * 4;
+        const size_t smem2 = smem_k + (size_t)kQkQ2 * D * 4 + (size_t)kQkQ2 * 4;
+        int st = ensure_tma_attrs((const void*)stats, shape->device);
+        if (st != KVC_OK) return st;
+        st = ensure_tma_attrs((const void*)accum, shape->device);
+        if (st != KVC_OK) return st;
+        stats<<<dim3((unsigned)max_x1, (unsigned)(B * Hkv), (unsigned)n_active), kQkThreads, smem1,
+                 (cudaStream_t)stream>>>(bd);
+        cudaError_t err = cudaGetLastError();
+        if (err != cudaSuccess) return cuda_fail(err, "kvc_h2o_qk_stats_kernel launch");
+        g_launches.fetch_add(1);
+        accum<<<dim3((unsigned)max_tiles, (unsigned)B, (unsigned)n_active), kQkThreads, smem2, (cudaStream_t)stream>>>(bd);
+        err = cudaGetLastError();
+        if (err != cudaSuccess) return cuda_fail(err, "kvc_h2o_qk_accumulate_kernel launch");
+        g_launches.fetch_add(1);
+    }
+    return KVC_OK;
+}
 #endif  // KVC_HAS_H2O
 
 }  // extern "C"

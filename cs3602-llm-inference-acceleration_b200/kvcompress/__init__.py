@@ -29,6 +29,7 @@ from .methods import (
     COMPRESS_METHODS,
 )
 from .slab_cache import KVSlabCache
+from .capture import capture_queries, QueryCapture
 from .evaluate import evaluate_with_compression, evaluate_baseline, compare_methods
 from .benchmark import benchmark, measure_generation_metrics, run_benchmark_suite, print_benchmark_summary
 from .utils import (
@@ -48,7 +49,7 @@ __all__ = [
     "to_dynamic_cache", "normalize_kv_cache", "get_cache_size_mb", "get_cache_info", "get_seq_len",
     "evaluate_with_compression", "evaluate_baseline", "compare_methods",
     "benchmark", "measure_generation_metrics", "run_benchmark_suite", "print_benchmark_summary",
-    "KVSlabCache",
+    "KVSlabCache", "capture_queries", "QueryCapture",
 ]
 
 __version__ = "2.0.0"

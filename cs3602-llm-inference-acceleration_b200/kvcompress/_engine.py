@@ -99,6 +99,11 @@ def load_library():
                                              ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]
     lib.kvc_h2o_accumulate.restype = ctypes.c_int
     lib.kvc_h2o_accumulate.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_float, ctypes.c_void_p]
+    lib.kvc_h2o_qk_workspace_bytes.restype = ctypes.c_int64
+    lib.kvc_h2o_qk_workspace_bytes.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_char_p]
+    lib.kvc_h2o_accumulate_qk.restype = ctypes.c_int
+    lib.kvc_h2o_accumulate_qk.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_char_p, ctypes.c_float,
+                                          ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
     if lib.kvc_abi_version() != KVC_ABI_VERSION:
         raise RuntimeError(f"{_LIB_NAME}: ABI version {lib.kvc_abi_version()} != {KVC_ABI_VERSION} — rebuild the library")
     _lib = lib
@@ -614,3 +619,90 @@ def h2o_accumulate(layers: Sequence[tuple], decay: float) -> None:
     status = load_library().kvc_h2o_accumulate(shape, len(layers), bytes(buf), float(decay),
                                                ctypes.c_void_p(_stream_ptr(acc0.device)))
     _check(status, "kvc_h2o_accumulate")
+
+
+_H2O_QK = struct.Struct("P3qP3qP2qP2qPf5i")  # kvc_h2o_qk_layer: q | 3 strides | k | 3 strides | mask | 2 strides | acc |
+assert _H2O_QK.size == 144                    # 2 strides | score_out | scaling | n_query key_len prev_len score_lo score_hi
+
+
+def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspace) -> None:
+    """H2O attention-score bookkeeping from queries and keys (``kvc_h2o_accumulate_qk``): two launches for all layers.
+
+    layers: ``(q, k, mask, acc, score_out, prev_len, score_lo, score_hi, scaling)`` per layer —
+      q ``[B, Hq, T, D]`` post-RoPE queries with a dense last dimension, Hq = group * Hkv; k ``[B, Hkv, key_len, D]`` keys
+      whose rows are 16-byte aligned (any slab view); mask ``[B, T, >= key_len]`` bool (True = visible) with a dense last
+      dimension, or ``None`` for the causal rule (query t sees keys ``j <= key_len - T + t``); acc, score_out, prev_len,
+      score_lo, score_hi as in :func:`h2o_accumulate`; scaling the logit scale (``D ** -0.5`` for most models).
+      The probabilities are ``round(exp(s - lse))`` of the fp32 logits ``s = scaling * q . k`` where visible, 0 elsewhere.
+    workspace: a uint8 CUDA tensor, or a callable that returns one of at least the bytes it is given.
+    q, k and acc share one dtype and device; nothing is synchronised."""
+    if not layers:
+        return
+    group = int(group)
+    if group < 1:
+        raise ValueError(f"group must be >= 1, got {group}")
+    q0, k0, acc0 = layers[0][0], layers[0][1], layers[0][3]
+    _require_cuda(k0, "keys")
+    if k0.dim() != 4:
+        raise ValueError(f"keys must be [B, Hkv, key_len, D], got {tuple(k0.shape)}")
+    B, Hkv, _, D = k0.shape
+    Hq = Hkv * group
+    dt, dev = k0.dtype, k0.device
+    buf = bytearray(_H2O_QK.size * len(layers))
+    keep = []
+    for m, (q, k, mask, acc, score, prev_len, lo, hi, scaling) in enumerate(layers):
+        _require_cuda(q, f"layer {m} queries")
+        _require_cuda(k, f"layer {m} keys")
+        if k.dtype != dt or k.device != dev or k.dim() != 4 or k.shape[:2] != (B, Hkv) or k.size(3) != D:
+            raise ValueError(f"layer {m}: keys must be a [B={B}, Hkv={Hkv}, key_len, D={D}] {dt} tensor on {dev}")
+        key_len = k.size(2)
+        if q.dtype != dt or q.device != dev or q.dim() != 4 or q.size(0) != B or q.size(1) != Hq or q.size(3) != D \
+                or (q.stride(3) != 1 and D > 1):
+            raise ValueError(f"layer {m}: queries must be a [B={B}, Hq={Hq}, T, D={D}] {dt} tensor on {dev} with a dense "
+                             "last dimension")
+        T = q.size(2)
+        if acc.dtype != dt or acc.device != dev or acc.dim() != 3 or acc.size(0) != B or acc.size(1) != Hq \
+                or acc.size(2) < key_len or acc.stride(2) != 1:
+            raise ValueError(f"layer {m}: acc must be a [B={B}, Hq={Hq}, >= {key_len}] {dt} tensor on {dev} with a dense "
+                             "last dimension")
+        if not _rows_ok(k):
+            k = k.contiguous()
+            keep.append(k)
+        m_ptr, m_st = 0, (0, 0)
+        if mask is not None:
+            if mask.dtype != torch.bool or mask.device != dev or mask.dim() != 3 or mask.size(0) != B \
+                    or mask.size(1) != T or mask.size(2) < key_len or (mask.stride(2) != 1 and key_len > 1):
+                raise ValueError(f"layer {m}: mask must be a bool [B={B}, T={T}, >= {key_len}] tensor on {dev} with a "
+                                 "dense last dimension")
+            m_ptr, m_st = mask.data_ptr(), mask.stride()[:2]
+        elif T > key_len:
+            raise ValueError(f"layer {m}: {T} queries over {key_len} keys need a mask")
+        s_ptr = 0
+        if score is not None:
+            if score.dtype != dt or score.device != dev or not score.is_contiguous() or score.numel() < B * (hi - lo):
+                raise ValueError(f"layer {m}: score_out must be a contiguous {dt} tensor of >= B * region elements on "
+                                 f"{dev}")
+            s_ptr = score.data_ptr()
+        qs, ks = q.stride(), k.stride()
+        _H2O_QK.pack_into(buf, m * _H2O_QK.size, q.data_ptr(), qs[0], qs[1], qs[2], k.data_ptr(), ks[0], ks[1], ks[2],
+                          m_ptr, m_st[0], m_st[1], acc.data_ptr(), acc.stride(0), acc.stride(1), s_ptr, float(scaling),
+                          T, key_len, prev_len, lo, hi)
+    recs = bytes(buf)
+    shape = _SHAPE.pack(B, Hkv, D, KVC_DTYPE[dt], dev.index)
+    lib = load_library()
+    need = int(lib.kvc_h2o_qk_workspace_bytes(shape, group, len(layers), recs))
+    if need < 0:
+        status = lib.kvc_h2o_accumulate_qk(shape, group, len(layers), recs, float(decay), None, 0, None)
+        _check(status, "kvc_h2o_accumulate_qk")
+        raise ValueError("kvc_h2o_qk_workspace_bytes: invalid arguments")
+    ws = workspace(need) if callable(workspace) else workspace
+    ws_ptr, ws_bytes = 0, 0
+    if ws is not None:
+        if ws.device != dev or not ws.is_contiguous():
+            raise ValueError(f"workspace must be a contiguous tensor on {dev}")
+        ws_ptr, ws_bytes = ws.data_ptr(), ws.numel() * ws.element_size()
+    if ws_bytes < need:
+        raise ValueError(f"workspace of {ws_bytes} bytes, kvc_h2o_accumulate_qk needs {need}")
+    status = lib.kvc_h2o_accumulate_qk(shape, group, len(layers), recs, float(decay), ctypes.c_void_p(ws_ptr), ws_bytes,
+                                       ctypes.c_void_p(_stream_ptr(dev)))
+    _check(status, "kvc_h2o_accumulate_qk")

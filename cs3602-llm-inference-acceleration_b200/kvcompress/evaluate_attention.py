@@ -10,8 +10,11 @@ compacted to sinks + heavy hitters + recent rows (the gather runs on the sm_100a
 place), as ``evaluate_with_compression`` does.  With an :class:`H2OScoreSlab` as ``h2o_manager`` the score bookkeeping
 runs on the device as well: one accumulate launch per update, one compaction launch per compression.
 
-The model must be able to return attention weights (``attn_implementation="eager"``); ``tokenizer`` only needs
-``encode(text, return_tensors="pt")`` — pass ``input_ids=`` to skip it (offline runs).
+``scores="attentions"`` (the default) needs a model that returns attention weights (``attn_implementation="eager"``).
+``scores="queries"`` runs every forward under :func:`kvcompress.capture_queries` (SDPA, no ``output_attentions``) and
+updates an :class:`H2OScoreSlab` (the default manager then) from the recorded queries and keys: the probabilities are
+rebuilt on the device from fp32 logits.  ``tokenizer`` only needs ``encode(text, return_tensors="pt")`` — pass
+``input_ids=`` to skip it (offline runs).
 """
 
 from __future__ import annotations
@@ -24,7 +27,8 @@ import torch
 from torch.nn import CrossEntropyLoss
 
 from .evaluate import _EMPTY, _final_cache_size, evaluate_with_compression, new_slab_for_model
-from .methods.h2o_attention import H2OAttentionManager, h2o_attention_compress
+from .capture import capture_queries
+from .methods.h2o_attention import H2OAttentionManager, H2OScoreSlab, h2o_attention_compress
 from .utils import normalize_kv_cache, to_dynamic_cache
 
 
@@ -33,20 +37,28 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                                         heavy_hitter_size: int = 64, recent_size: int = 444, max_tokens: int = 3000,
                                         skip_layers: List[int] = [0, 1], device: Optional[torch.device] = None,
                                         show_progress: bool = True, *, input_ids: Optional[torch.Tensor] = None,
-                                        cache: str = "dynamic", return_nlls: bool = False) -> Dict[str, float]:
+                                        cache: str = "dynamic", return_nlls: bool = False,
+                                        scores: str = "attentions") -> Dict[str, float]:
     """PPL / accuracy / TTFT / TPOT with attention-score H2O applied after every token.  ``h2o_manager``: an
-    :class:`H2OAttentionManager` (the default) or an :class:`H2OScoreSlab`; ``cache``: ``"dynamic"`` or ``"slab"``."""
+    :class:`H2OAttentionManager` (the default) or an :class:`H2OScoreSlab`; ``cache``: ``"dynamic"`` or ``"slab"``;
+    ``scores``: ``"attentions"`` (``output_attentions=True``) or ``"queries"`` (:func:`kvcompress.capture_queries`, an
+    :class:`H2OScoreSlab` manager)."""
     if cache not in ("dynamic", "slab"):
         raise ValueError(f"cache must be 'dynamic' or 'slab', got {cache!r}")
+    if scores not in ("attentions", "queries"):
+        raise ValueError(f"scores must be 'attentions' or 'queries', got {scores!r}")
     if device is None:
         device = next(model.parameters()).device
     if h2o_manager is None:
-        h2o_manager = H2OAttentionManager(start_size=start_size, heavy_hitter_size=heavy_hitter_size,
-                                          recent_size=recent_size,
-                                          num_layers=getattr(model.config, "num_hidden_layers", 32),
-                                          num_heads=getattr(model.config, "num_attention_heads", 32), device=device)
+        manager_cls = H2OScoreSlab if scores == "queries" else H2OAttentionManager
+        h2o_manager = manager_cls(start_size=start_size, heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
+                                  num_layers=getattr(model.config, "num_hidden_layers", 32),
+                                  num_heads=getattr(model.config, "num_attention_heads", 32), device=device)
     else:
+        if scores == "queries" and not isinstance(h2o_manager, H2OScoreSlab):
+            raise ValueError("scores='queries' needs an H2OScoreSlab manager")
         h2o_manager.reset()
+    use_queries = scores == "queries"
     if input_ids is None:
         input_ids = tokenizer.encode(text, return_tensors="pt")
     input_ids = input_ids[:, :max_tokens].to(device)
@@ -76,29 +88,44 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
     with torch.inference_mode():
         for idx in steps:
             token_start = time.perf_counter()
-            outputs = model(input_ids[:, idx:idx + 1], past_key_values=past_key_values, use_cache=True,
-                            output_attentions=True)
+            if use_queries:
+                with capture_queries(model) as capture:
+                    outputs = model(input_ids[:, idx:idx + 1], past_key_values=past_key_values, use_cache=True)
+                attentions = None
+                scored = dict(attention_queries=capture)
+            else:
+                outputs = model(input_ids[:, idx:idx + 1], past_key_values=past_key_values, use_cache=True,
+                                output_attentions=True)
+                attentions = outputs.attentions
+                scored = dict(attention_scores=attentions)
             logits = outputs.logits[:, -1, :].view(-1, vocab)
             target = input_ids[:, idx + 1:idx + 2].view(-1)
             nlls.append(float(loss_fn(logits, target).mean().item()))
             correct.append(float((torch.argmax(logits, dim=-1) == target).float().mean().item()))
-            attentions = outputs.attentions
+
+            def update():
+                if use_queries:
+                    h2o_manager.update_from_queries(capture.queries, capture.keys, capture.masks, capture.scaling,
+                                                    skip_layers)
+                else:
+                    h2o_manager.update_attention_scores(attentions, skip_layers)
+
             if slab is not None:
-                h2o_manager.update_attention_scores(attentions, skip_layers)
+                update()
                 if slab.lengths[0] > budget:
-                    slab.compress_("h2o_attention", attention_scores=attentions, h2o_manager=h2o_manager,
-                                   start_size=start_size, heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
-                                   skip_layers=skip_layers)
+                    slab.compress_("h2o_attention", h2o_manager=h2o_manager, start_size=start_size,
+                                   heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
+                                   skip_layers=skip_layers, **scored)
                     h2o_manager.reset()
             else:
                 past_key_values = outputs.past_key_values
-                h2o_manager.update_attention_scores(attentions, skip_layers)
+                update()
                 if past_key_values is not None:
                     kv_list = list(normalize_kv_cache(past_key_values))
                     if kv_list and kv_list[0][0].size(2) > budget:
-                        kept = h2o_attention_compress(kv_list, attention_scores=attentions, h2o_manager=h2o_manager,
-                                                      start_size=start_size, heavy_hitter_size=heavy_hitter_size,
-                                                      recent_size=recent_size, skip_layers=skip_layers)
+                        kept = h2o_attention_compress(kv_list, h2o_manager=h2o_manager, start_size=start_size,
+                                                      heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
+                                                      skip_layers=skip_layers, **scored)
                         past_key_values = to_dynamic_cache(kept)
                         h2o_manager.reset()
             token_time = time.perf_counter() - token_start

@@ -90,16 +90,34 @@ class H2OAttentionManager:
         return top
 
 
+def update_manager(h2o_manager, attention_scores=None, attention_queries=None, skip_layers=()) -> None:
+    """The manager update a compress call makes before it selects (reference :274-275): from attention probabilities,
+    or — :class:`H2OScoreSlab` only — from a :class:`kvcompress.QueryCapture` of the forward that produced them."""
+    if attention_queries is not None:
+        if not isinstance(h2o_manager, H2OScoreSlab):
+            raise ValueError("attention_queries needs an H2OScoreSlab manager: H2OAttentionManager takes attention "
+                             "probabilities (attention_scores) only")
+        if attention_scores is not None:
+            raise ValueError("pass attention_scores or attention_queries, not both")
+        cap = attention_queries
+        h2o_manager.update_from_queries(cap.queries, cap.keys, cap.masks, cap.scaling, list(skip_layers))
+    elif h2o_manager is not None and attention_scores is not None:
+        h2o_manager.update_attention_scores(attention_scores, list(skip_layers))
+
+
 def h2o_attention_compress(past_key_values, attention_scores=None, h2o_manager: Optional[H2OAttentionManager] = None,
                            start_size: int = 4, heavy_hitter_size: int = 64, recent_size: int = 444,
-                           skip_layers: List[int] = [], **kwargs) -> List[Tuple[torch.Tensor, torch.Tensor]]:
+                           skip_layers: List[int] = [], attention_queries=None,
+                           **kwargs) -> List[Tuple[torch.Tensor, torch.Tensor]]:
     """Sinks + heavy hitters + recent window; heavy hitters come from ``h2o_manager`` when given,
-    otherwise from the lowest key norms (identical to ``h2o_l2_compress``)."""
+    otherwise from the lowest key norms (identical to ``h2o_l2_compress``).  ``attention_queries``: a
+    :class:`kvcompress.QueryCapture` to update an :class:`H2OScoreSlab` from, instead of ``attention_scores``."""
     layers = as_layer_list(past_key_values)
     if not layers:
         return layers
-    if h2o_manager is not None and attention_scores is not None:
-        h2o_manager.update_attention_scores(attention_scores, skip_layers)  # :274-275
+    if attention_queries is not None and h2o_manager is None:
+        raise ValueError("attention_queries needs an H2OScoreSlab manager (h2o_manager=)")
+    update_manager(h2o_manager, attention_scores, attention_queries, skip_layers)
     plans = cached_plans(_planner.plan_h2o, seq_lens(layers), start_size, heavy_hitter_size, recent_size,
                          skip_layers=skip_layers)
     if h2o_manager is None:
@@ -194,6 +212,7 @@ class H2OScoreSlab:
         self._scored: Dict[int, Tuple[int, int]] = {}  # layer -> (lo, hi) its score row currently holds
         self._gen = 0                               # bumped whenever the buffers are reallocated
         self._plan_cache: Dict[tuple, tuple] = {}
+        self._ws: Optional[torch.Tensor] = None     # workspace of update_from_queries (uint8)
 
     @property
     def accumulated_attention(self) -> Mapping:
@@ -275,6 +294,73 @@ class H2OScoreSlab:
             self._scored[layer_idx] = (lo, hi)
             self.current_seq_len = key_len
         _engine.h2o_accumulate(recs, self.decay_factor)
+
+    def _workspace(self, nbytes: int, device: torch.device) -> torch.Tensor:
+        """The query path's workspace: kept between updates, grown by doubling, so a steady step allocates nothing."""
+        ws = self._ws
+        if ws is None or ws.device != device or ws.numel() < nbytes:
+            cap = max(ws.numel() if ws is not None and ws.device == device else 0, 4096)
+            while cap < nbytes:
+                cap *= 2
+            ws = self._ws = torch.empty((cap,), dtype=torch.uint8, device=device)
+        return ws
+
+    def update_from_queries(self, queries, keys, masks=None, scaling=None, skip_layers: List[int] = []) -> None:
+        """The update of :meth:`update_attention_scores` with the attention probabilities rebuilt on the device from the
+        post-RoPE ``queries[l]`` ``[B, Hq, T, D]`` and the cached ``keys[l]`` ``[B, Hkv, key_len, D]`` (any view whose
+        rows are dense, e.g. a slab view) — the model never has to return attention weights.  ``masks[l]``: ``None``
+        (causal: the queries are the last T positions) or a bool ``[B, 1, T, key_len]`` / ``[B, T, key_len]`` mask,
+        True = visible.  ``scaling``: the logit scale, one float or one per layer (default ``D ** -0.5``).  The
+        probabilities are ``softmax(fp32 logits).to(dtype)``: HF eager attention in a 16-bit model rounds the logits to
+        the model dtype first, SDPA and flash do not.  Two launches for every non-skipped layer with queries and keys;
+        no synchronisation (:func:`kvcompress.capture_queries` records these arguments from a model's forward)."""
+        if queries is None:
+            return
+        work = []
+        for layer_idx, q in enumerate(queries):
+            k = keys[layer_idx] if layer_idx < len(keys) else None
+            if layer_idx in skip_layers or q is None or k is None:
+                continue
+            if layer_idx >= self.num_layers:
+                raise ValueError(f"H2OScoreSlab: layer {layer_idx} >= num_layers={self.num_layers}")
+            if q.dim() != 4 or k.dim() != 4 or k.size(1) == 0 or q.size(1) % k.size(1):
+                raise ValueError(f"layer {layer_idx}: queries must be [B, Hq, T, D] and keys [B, Hkv, key_len, D] with "
+                                 f"Hkv dividing Hq, got {tuple(q.shape)} and {tuple(k.shape)}")
+            mask = None if masks is None or layer_idx >= len(masks) else masks[layer_idx]
+            if mask is not None:
+                if mask.dim() == 4:
+                    if mask.size(1) != 1:
+                        raise ValueError(f"layer {layer_idx}: a per-head mask {tuple(mask.shape)} is not supported; "
+                                         "pass [B, 1, T, key_len] or [B, T, key_len]")
+                    mask = mask[:, 0]
+                if mask.dtype != torch.bool:
+                    raise ValueError(f"layer {layer_idx}: the mask must be bool (True = visible), got {mask.dtype}")
+                if mask.dim() == 3 and mask.size(0) == 1 and q.size(0) > 1:
+                    mask = mask.expand(q.size(0), -1, -1)
+                if mask.dim() == 3 and mask.size(2) > k.size(2):
+                    mask = mask[:, :, :k.size(2)]
+                if mask.dim() == 3 and mask.size(2) > 1 and mask.stride(2) != 1:
+                    mask = mask.contiguous()
+            s = scaling[layer_idx] if isinstance(scaling, (list, tuple)) else scaling
+            work.append((layer_idx, q if q.stride(-1) == 1 else q.contiguous(), k, mask,
+                         q.size(3) ** -0.5 if s is None else float(s)))
+        if not work:
+            return
+        q0, k0 = work[0][1], work[0][2]
+        _engine._require_cuda(q0, "queries")
+        self._ensure(q0.size(0), q0.size(1), q0.dtype, q0.device, max(k.size(2) for _, _, k, _, _ in work))
+        recs = []
+        for layer_idx, q, k, mask, s in work:
+            key_len = k.size(2)
+            lo, hi, _ = _planner.h2o_score_region(key_len, key_len, self.start_size, self.heavy_hitter_size,
+                                                  self.recent_size)
+            recs.append((q, k, mask, self._acc[layer_idx], self._score[layer_idx], self._lens.get(layer_idx, -1), lo, hi,
+                         s))
+            self._lens[layer_idx] = key_len
+            self._scored[layer_idx] = (lo, hi)
+            self.current_seq_len = key_len
+        _engine.h2o_accumulate_qk(recs, self.decay_factor, q0.size(1) // k0.size(1),
+                                  lambda n: self._workspace(n, q0.device))
 
     def get_heavy_hitter_indices(self, layer_idx: int, seq_len: int) -> torch.Tensor:
         """Indices (relative to the middle region, ascending) of its heaviest tokens — what
@@ -392,4 +478,4 @@ def create_h2o_manager_from_model(model, **kwargs) -> H2OAttentionManager:
 
 
 __all__ = ["H2OAttentionManager", "H2OScoreSlab", "h2o_attention_compress", "create_h2o_manager_from_model",
-           "manager_plans"]
+           "manager_plans", "update_manager"]

@@ -411,18 +411,20 @@ class KVSlabCache:
 
     def _compress_h2o_attention(self, attention_scores=None, h2o_manager=None, start_size: int = 4,
                                 heavy_hitter_size: int = 64, recent_size: int = 444, skip_layers: Sequence[int] = (),
-                                return_indices: bool = False, **_ignored):
+                                return_indices: bool = False, attention_queries=None, **_ignored):
         """``h2o_attention_compress`` in place (reference h2o_attention.py:216-363): without a manager it is exactly
         ``h2o_l2`` (:337-351); with one, its head-summed heavy hitters are the caller-supplied rows of the in-place
-        compaction (they must ascend strictly — the manager sorts them, a clamp collision is refused)."""
+        compaction (they must ascend strictly — the manager sorts them, a clamp collision is refused).
+        ``attention_queries``: a ``QueryCapture`` that updates an ``H2OScoreSlab`` instead of ``attention_scores``."""
         from .methods._common import cached_plans
-        from .methods.h2o_attention import H2OScoreSlab, manager_plans
+        from .methods.h2o_attention import H2OScoreSlab, manager_plans, update_manager
 
         if h2o_manager is None:
+            if attention_queries is not None:
+                raise ValueError("attention_queries needs an H2OScoreSlab manager (h2o_manager=)")
             return self.compress_("h2o_l2", return_indices=return_indices, start_size=start_size,
                                   heavy_hitter_size=heavy_hitter_size, recent_size=recent_size, skip_layers=skip_layers)
-        if attention_scores is not None:
-            h2o_manager.update_attention_scores(attention_scores, list(skip_layers))
+        update_manager(h2o_manager, attention_scores, attention_queries, skip_layers)
         plans = cached_plans(P.plan_h2o, self.lengths, start_size, heavy_hitter_size, recent_size, skip_layers=skip_layers)
         if isinstance(h2o_manager, H2OScoreSlab):  # scores ranked on the device: no host round trip
             plans, given, scores = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,

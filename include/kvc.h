@@ -47,7 +47,7 @@ extern "C" {
 #endif
 
 /* Additions that leave every existing struct layout, enum value and entry point as it was (a new score kind, the
- * kvc_h2o_layer struct and kvc_h2o_accumulate) keep the version: a caller built against an older header sees the
+ * kvc_h2o_layer / kvc_h2o_qk_layer structs and their entry points) keep the version: a caller built against an older header sees the
  * same ABI, and a caller that uses the additions fails to link or gets KVC_ERR_INVALID_ARG from an older library. */
 #define KVC_ABI_VERSION 5
 
@@ -269,6 +269,44 @@ typedef struct kvc_h2o_layer {
 /* shape: batch = B, heads = Hq (query heads), dtype = the attention dtype, device; head_dim is not used. */
 int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_layer* layers, float decay,
                        void* stream);
+
+/* The same update with the attention probabilities rebuilt from the post-RoPE queries and the cached keys, so that the
+ * model can run any attention backend (SDPA, flash) and never materialise [B, Hq, n_query, key_len] probabilities.
+ * Per layer, batch entry b, query head h (KV head h / G, G = group), query t < T = n_query and key j < key_len:
+ *   s[t,j]   = scaling * sum_d fp32(q[b,h,t,d]) * fp32(k[b,h/G,j,d])    fp32, one fmaf chain in ascending d
+ *   vis(t,j) = mask[b,t,j] (nonzero = visible) if mask != NULL, else j <= key_len - T + t (causal: the queries are the
+ *              last T positions)
+ *   lse[t]   = log sum_{vis} exp(s[t,j])                                  fp32, max-shifted
+ *   attn     = round(exp(s[t,j] - lse[t])) where visible, 0 elsewhere (a query with no visible key adds 0)
+ * then exactly kvc_h2o_accumulate's update with that attn (the query sum in ascending t).  This is HF eager attention's
+ * softmax(..., dtype=float32).to(query.dtype) of fp32 logits; eager attention in a 16-bit model rounds the logits to
+ * the model dtype before its softmax, SDPA and flash do not.  Two launches per KVC_MAX_LAYERS_PER_LAUNCH layers: the
+ * per-split (max, sum exp) partials go to the workspace, the update combines them in a fixed order.  Every split and
+ * tile depends only on (key_len, n_query, group, head_dim, dtype): a layer's bits do not depend on B, the other layers
+ * of the call or the device.  KVC_ERR_INVALID_ARG: n_query > key_len without a mask, group < 1, a score region outside
+ * [0, key_len], NULL acc / q / k, a workspace smaller than kvc_h2o_qk_workspace_bytes.  KVC_ERR_UNSUPPORTED: a dtype
+ * other than f32 / f16 / bf16, head_dim * e not a multiple of 16 or above 512 bytes (D <= 256 in 16-bit, D <= 128 in
+ * fp32), K rows not 16-byte aligned. */
+typedef struct kvc_h2o_qk_layer {
+    const void* q;          /* [B, Hq, n_query, D] queries, last dim dense */
+    int64_t q_stride_b, q_stride_h, q_stride_t; /* elements */
+    const void* k;          /* [B, Hkv, key_len, D] keys, rows 16-byte aligned (a slab view qualifies) */
+    int64_t k_stride_b, k_stride_h, k_stride_s; /* elements */
+    const uint8_t* mask;    /* optional [B, n_query, key_len] bool, last dim dense; NULL: the causal rule */
+    int64_t m_stride_b, m_stride_t;             /* elements (bytes) */
+    void* acc;              /* [B, Hq, >= key_len] accumulators, as kvc_h2o_layer */
+    int64_t acc_stride_b, acc_stride_h;         /* elements */
+    void* score_out;        /* optional [B, score_hi - score_lo], dense */
+    float scaling;
+    int32_t n_query, key_len, prev_len, score_lo, score_hi;
+} kvc_h2o_qk_layer;
+/* shape: batch = B, heads = Hkv (KV heads), head_dim = D, dtype of q, K and acc, device; group = G = Hq / Hkv.
+ * Bytes of device workspace kvc_h2o_accumulate_qk needs for these layers (the sum over the layers; 0 when there is
+ * nothing to do); -1 when the arguments are invalid. */
+int64_t kvc_h2o_qk_workspace_bytes(const kvc_shape* shape, int32_t group, int32_t n_layers,
+                                   const kvc_h2o_qk_layer* layers);
+int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers,
+                          float decay, void* workspace, int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
