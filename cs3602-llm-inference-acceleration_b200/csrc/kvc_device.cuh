@@ -37,6 +37,14 @@ constexpr int kMiscWarpB = 64;  // 32 ints: per-warp counter B (eq counts)
 constexpr int kMiscHalo = 96;   // 32 ints: snapkv pooling halo (raw norms of the previous tile's tail)
 
 // ---------------------------------------------------------------- launch descriptors
+// Per-row state that moves with the kept rows (kvc_carry_layer): `group` rows of acc per (batch, KV head) unit.
+struct CarryDev {
+    char* acc;             // nullptr: nothing to carry for this layer
+    int64_t asb, ash;      // BYTE strides (batch, acc head)
+    int32_t group, prev;   // prev: valid entries before the compaction, already clamped to S
+};
+static_assert(sizeof(CarryDev) == 32, "CarryDev is part of the kernel parameters");
+
 struct LayerDev {
     const char* k_in;
     const char* v_in;
@@ -49,9 +57,9 @@ struct LayerDev {
     int32_t S, sink, lo, hi, ksel, tail, score, pool;
     const char* n_in;       // optional stored key norms [B,H,>=S] (cache dtype): scores without reading K
     int64_t nsb, nsh;       // BYTE strides of the norm array (batch, head)
-    int64_t pad;
+    CarryDev carry;         // optional per-row state compacted in place with the kept rows
 };
-static_assert(sizeof(LayerDev) == 160, "LayerDev is passed by value in kernel params");
+static_assert(sizeof(LayerDev) == 184, "LayerDev is passed by value in kernel params");
 
 struct BatchDev {
     int32_t B, H;
@@ -67,6 +75,7 @@ struct BatchDev {
     int64_t ws_keys;   // bytes of the key part of a unit
     LayerDev layers[KVC_MAX_LAYERS_PER_LAUNCH];
 };
+static_assert(sizeof(BatchDev) < 32 * 1024, "kernel parameters are limited to 32 KB");
 
 // ---------------------------------------------------------------- dtype traits
 template <int DT>

@@ -20,6 +20,8 @@
 //   gather output rows are produced 32 at a time per staging warp: every run of consecutive
 //          source rows becomes one bulk load into the slot, and the 32 rows leave with ONE bulk
 //          store into the dense output (expand + gather x2 + cat x2, e.g. fix_size_l2.py:132-147).
+//   carry  optional per-row state (kvc_carry_layer: H2O accumulators) compacted IN PLACE with the kept rows by
+//          the whole CTA, between the select and the gather (carry_unit).
 //
 // Row widths: CPR (16-byte chunks per row) is a template parameter for the widths of real models
 // (128/160/192/256/320/512-byte rows); CPR = 0 is the generic form for every other head_dim, same
@@ -98,6 +100,34 @@ struct KeepMap {
         return j < sink ? j : (j < sink + ksel ? sidx[j - sink] : j + tail0);
     }
 };
+
+// Per-row state of a unit follows its kept rows, in place (kvc_carry_layer): acc'[g][i] = acc[g][src(i)] when
+// src(i) < prev, 0 otherwise, for the `group` acc rows of KV head h and i < C.  The group x C entries go in rounds of
+// NT, g-major: every thread reads its entry, the CTA synchronises, every thread writes.  Kept rows ascend and never move
+// up (src(i) >= i), so no later round reads an entry an earlier round wrote.  Entries that neither move nor become zero
+// are not touched.  All NT threads call (CTA-uniform: c.acc != nullptr).
+template <typename Key, int NT>
+__device__ __forceinline__ void carry_unit(const CarryDev& c, const KeepMap& src_row, int C, int b, int h) {
+    char* base = c.acc + (int64_t)b * c.asb + (int64_t)h * c.group * c.ash;
+    const int n = c.group * C;
+    for (int e0 = 0; e0 < n; e0 += NT) {
+        const int e = e0 + (int)threadIdx.x;
+        Key* row = nullptr;
+        int i = 0;
+        Key val = 0;
+        bool write = false;
+        if (e < n) {
+            const int g = e / C;
+            i = e - g * C;
+            const int s = src_row(i);
+            row = reinterpret_cast<Key*>(base + (int64_t)g * c.ash);
+            write = s != i || s >= c.prev;
+            if (write && s < c.prev) val = row[s];
+        }
+        __syncthreads();
+        if (write) row[i] = val;
+    }
+}
 
 // K3: rows [0, C) of the dense outputs from the kept source rows, K then V, 32 rows per staging warp per step.
 // Called by the staging warps only (stage = this warp's index among the `nstage` of them).
@@ -285,6 +315,8 @@ __global__ void __launch_bounds__(NT, MINB) kvc_fused_tma_kernel(const __grid_co
         int32_t* io = L.idx_out + (int64_t)bh * C;
         for (int j = tid; j < C; j += NT) io[j] = src_row(j);
     }
+    // accumulators follow their rows (sidx is complete: barrier above; it stays valid until the end-of-unit barrier)
+    if (L.carry.acc != nullptr) carry_unit<Key, NT>(L.carry, src_row, C, b, h);
     if (stager)
         gather_unit(src_row, C, kbase, vbase, L.kss, L.vss, L.k_out + (int64_t)bh * C * RB,
                     L.v_out + (int64_t)bh * C * RB, RB, slot, bar, parity, warp, nsw, lane);

@@ -14,6 +14,8 @@
 //                             bulk-loads its 32 source rows, the CTA synchronises, then every warp
 //                             bulk-stores.  Kept rows are ascending and never move up (src >= dst),
 //                             so sources of later rounds lie above every destination written so far.
+//                             Optional per-row state (kvc_carry_layer: H2O accumulators, `group` rows per unit)
+//                             slides the same way, before the early return of a unit whose rows all stay put.
 #pragma once
 #include "kvc_fused_tma.cuh"
 
@@ -27,9 +29,9 @@ struct SlabLayerDev {
     const int32_t* idx_in;
     int64_t ksb, ksh, vsb, vsh, nsb, nsh;  // BYTE strides (batch, head)
     int32_t S, sink, lo, hi, ksel, tail, score, pool;
-    int64_t pad;
+    CarryDev carry;  // optional per-row state that slides with the kept rows
 };
-static_assert(sizeof(SlabLayerDev) == 128, "SlabLayerDev is passed by value in kernel params");
+static_assert(sizeof(SlabLayerDev) == 152, "SlabLayerDev is passed by value in kernel params");
 
 struct SlabBatchDev {
     int32_t B, H;
@@ -40,6 +42,7 @@ struct SlabBatchDev {
     int64_t ws_unit, ws_keys;
     SlabLayerDev layers[KVC_MAX_LAYERS_PER_LAUNCH];
 };
+static_assert(sizeof(SlabBatchDev) < 32 * 1024, "kernel parameters are limited to 32 KB");
 
 struct AppendLayerDev {
     const char* k_new;
@@ -289,6 +292,8 @@ __global__ void __launch_bounds__(NT, MINB) kvc_slab_compress_kernel(const __gri
     }
     __syncthreads();
     const int jf = misc[kMiscFirst];
+    // accumulators follow their rows, before the early return: entries past prev_len become 0 even when no row moves
+    if (L.carry.acc != nullptr) carry_unit<Key, NT>(L.carry, src_row, C, b, h);
     if (jf >= C) return;  // nothing moves (CTA-uniform)
 
     // ---------------------------------------------------------- slide rows down, K then V, in rounds

@@ -486,6 +486,28 @@ static int check_shape(const kvc_shape* shape, int* cpr_out) {
     return KVC_OK;
 }
 
+// Arguments of a layer's kvc_carry_layer (a non-NULL acc): checked before anything is enqueued.  The copy runs in place,
+// so the kept rows must be a valid in-place compaction (the slab rule: C <= S, the selection region between the sinks
+// and the tail), which makes every source row lie at or above its output row.
+static inline bool carry_ok(const kvc_carry_layer* carry, int l, const kvc_layer_plan& p, int e) {
+    if (!carry || !carry[l].acc) return true;
+    const kvc_carry_layer& c = carry[l];
+    if (c.group < 1 || c.prev_len < 0 || ((uintptr_t)c.acc % (uintptr_t)e) != 0) return false;
+    if ((int64_t)p.sink + p.k_sel + p.tail > p.seq_len) return false;
+    if (p.k_sel > 0 && (p.sel_lo < p.sink || p.sel_hi > p.seq_len - p.tail)) return false;
+    return true;
+}
+
+static inline void fill_carry(CarryDev& d, const kvc_carry_layer* carry, int l, const kvc_layer_plan& p, int e) {
+    if (!carry || !carry[l].acc) return;  // the descriptor was zeroed: acc == nullptr
+    const kvc_carry_layer& c = carry[l];
+    d.acc = (char*)c.acc;
+    d.asb = c.acc_stride_b * e;
+    d.ash = c.acc_stride_h * e;
+    d.group = c.group;
+    d.prev = c.prev_len < p.seq_len ? c.prev_len : p.seq_len;
+}
+
 }  // namespace kvc
 
 using namespace kvc;
@@ -596,6 +618,12 @@ int kvc_launch_shape(const kvc_shape* shape, int32_t n_layers, const kvc_layer_p
 
 int kvc_compress_layers_ws(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
                            const kvc_layer_io* io, void* workspace, int64_t workspace_bytes, void* stream) {
+    return kvc_compress_layers_carry(shape, n_layers, plans, io, nullptr, workspace, workspace_bytes, stream);
+}
+
+int kvc_compress_layers_carry(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
+                              const kvc_layer_io* io, const kvc_carry_layer* carry, void* workspace,
+                              int64_t workspace_bytes, void* stream) {
     if (!shape || n_layers < 0 || (n_layers > 0 && (!plans || !io))) return KVC_ERR_INVALID_ARG;
     if (n_layers == 0) return KVC_OK;
     int cpr = 0;
@@ -622,6 +650,7 @@ int kvc_compress_layers_ws(const kvc_shape* shape, int32_t n_layers, const kvc_l
             if ((given_score || p.score == KVC_SCORE_SNAPKV_POOL) && p.pool_kernel > 2 * kMaxPoolHalo)
                 return KVC_ERR_UNSUPPORTED;
         }
+        if (!carry_ok(carry, l, p, e)) return KVC_ERR_INVALID_ARG;
         if (C == 0) continue;
         if (!x.k_in || !x.v_in || !x.k_out || !x.v_out) return KVC_ERR_INVALID_ARG;
         if (C * cpr * 2 > 0x7fffffffLL) return KVC_ERR_TOO_LARGE;
@@ -678,6 +707,7 @@ int kvc_compress_layers_ws(const kvc_shape* shape, int32_t n_layers, const kvc_l
                 d.nsb = x.n_stride_b * key_bytes(dt);
                 d.nsh = x.n_stride_h * key_bytes(dt);
             }
+            fill_carry(d.carry, carry, l0 + l, p, e);
             if (p.k_sel > 0) {
                 any_select = true;
                 any_scan |= ranked && !x.norms_in;
@@ -918,6 +948,13 @@ int kvc_slab_append(const kvc_shape* shape, int32_t n_layers, const kvc_slab_lay
 int kvc_slab_compress(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
                       const kvc_slab_layer* slabs, int32_t* const* idx_out, const int32_t* const* idx_in,
                       void* workspace, int64_t workspace_bytes, void* stream) {
+    return kvc_slab_compress_carry(shape, n_layers, plans, slabs, idx_out, idx_in, nullptr, workspace, workspace_bytes,
+                                   stream);
+}
+
+int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
+                            const kvc_slab_layer* slabs, int32_t* const* idx_out, const int32_t* const* idx_in,
+                            const kvc_carry_layer* carry, void* workspace, int64_t workspace_bytes, void* stream) {
     int cpr = 0;
     int st = check_shape(shape, &cpr);
     if (st != KVC_OK) return st;
@@ -942,6 +979,7 @@ int kvc_slab_compress(const kvc_shape* shape, int32_t n_layers, const kvc_layer_
             if ((p.score == KVC_SCORE_SNAPKV_POOL || given_score) && p.pool_kernel > 2 * kMaxPoolHalo)
                 return KVC_ERR_UNSUPPORTED;
         }
+        if (!carry_ok(carry, l, p, e)) return KVC_ERR_INVALID_ARG;
         if (p.sink + p.k_sel + p.tail == 0) continue;
         if (!sl.k || !sl.v || !sl.norms) return KVC_ERR_INVALID_ARG;
         if (((uintptr_t)sl.k | (uintptr_t)sl.v) & 15) return KVC_ERR_UNSUPPORTED;
@@ -983,6 +1021,7 @@ int kvc_slab_compress(const kvc_shape* shape, int32_t n_layers, const kvc_layer_
             d.tail = p.tail;
             d.score = p.k_sel > 0 ? p.score : KVC_SCORE_NONE;
             d.pool = p.pool_kernel;
+            fill_carry(d.carry, carry, l0 + l, p, e);
             if (p.k_sel > 0) {
                 any_select = true;
                 if (p.k_sel > max_ksel) max_ksel = p.k_sel;

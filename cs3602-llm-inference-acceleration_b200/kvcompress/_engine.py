@@ -40,6 +40,24 @@ _RANKED = (P.SCORE_L2_LOW, P.SCORE_L2_HIGH, P.SCORE_SNAPKV_POOL)  # scores deriv
 _GIVEN_SCORES = (P.SCORE_GIVEN_SCORE, P.SCORE_GIVEN_SCORE_SHARED)  # scores supplied by the caller
 
 
+_CARRY = struct.Struct("P2q2i")   # kvc_carry_layer: acc | acc_stride_b acc_stride_h | group prev_len
+assert _CARRY.size == 32
+
+
+def carry_record(li: int, spec, B: int, H: int, dtype, seq_len: int) -> bytes:
+    """The ``kvc_carry_layer`` of layer ``li`` from ``(acc, group, prev_len)``: acc a ``[B, H * group, >= seq_len]``
+    CUDA tensor of the cache dtype with a dense last dimension, compacted in place with the layer's kept rows."""
+    acc, group, prev_len = spec
+    group, prev_len = int(group), int(prev_len)
+    if group < 1 or prev_len < 0:
+        raise ValueError(f"layer {li}: carry group must be >= 1 and prev_len >= 0, got {group} and {prev_len}")
+    if not acc.is_cuda or acc.dtype != dtype or acc.dim() != 3 or acc.size(0) != B or acc.size(1) != H * group \
+            or acc.size(2) < seq_len or (acc.stride(2) != 1 and acc.size(2) > 1):
+        raise ValueError(f"layer {li}: carried state must be a CUDA {dtype} [B={B}, H*group={H * group}, >= {seq_len}] "
+                         "tensor with a dense last dimension")
+    return _CARRY.pack(acc.data_ptr(), acc.stride(0), acc.stride(1), group, prev_len)
+
+
 def _score_shape(plan, B: int, H: int) -> tuple:
     """Shape of the caller-supplied scores of a SCORE_GIVEN_SCORE(_SHARED) plan."""
     region = plan.sel_hi - plan.sel_lo
@@ -104,6 +122,13 @@ def load_library():
     lib.kvc_h2o_accumulate_qk.restype = ctypes.c_int
     lib.kvc_h2o_accumulate_qk.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_char_p, ctypes.c_float,
                                           ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
+    lib.kvc_compress_layers_carry.restype = ctypes.c_int
+    lib.kvc_compress_layers_carry.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
+                                              ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
+    lib.kvc_slab_compress_carry.restype = ctypes.c_int
+    lib.kvc_slab_compress_carry.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
+                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p,
+                                            ctypes.c_int64, ctypes.c_void_p]
     if lib.kvc_abi_version() != KVC_ABI_VERSION:
         raise RuntimeError(f"{_LIB_NAME}: ABI version {lib.kvc_abi_version()} != {KVC_ABI_VERSION} — rebuild the library")
     _lib = lib
@@ -220,7 +245,7 @@ class PlanSet:
 
 def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indices: Optional[dict] = None,
               return_indices: bool = False, given_scores: Optional[dict] = None, norms: Optional[Sequence] = None,
-              non_blocking: bool = False, output_device=None):
+              non_blocking: bool = False, output_device=None, carry: Optional[dict] = None):
     """Apply per-layer plans (a list of ``LayerPlan`` or a cached :class:`PlanSet`) to a list of (K, V) pairs.
 
     KEEP layers keep their tensor objects, VIEW layers become ``x[:, :, -n:, :]`` views (both
@@ -239,9 +264,14 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
         complete once the current stream has been synchronised.
     output_device: host-resident (pinned) caches only — a CUDA device that receives the compressed cache instead of
         pinned host memory (stream-ordered like any CUDA tensor: no synchronisation).
+    carry: {layer_idx: (acc, group, prev_len)} — per-row state that follows the kept rows, in place and in the same
+        launch (``kvc_compress_layers_carry``): ``acc[:, h*group+g, i] = acc[:, h*group+g, src(i)]`` for the kept rows
+        ``src(i) < prev_len``, 0 for the others; acc is ``[B, H * group, >= S]`` in the cache dtype (H2O accumulators,
+        :class:`~kvcompress.methods.h2o_attention.H2OScoreSlab` with ``carry_scores=True``).
     """
     ps = plans if isinstance(plans, PlanSet) else PlanSet(plans)
-    if given_indices is None and given_scores is None and not return_indices and ps.gather and not ps.views:
+    if given_indices is None and given_scores is None and not return_indices and carry is None and ps.gather \
+            and not ps.views:
         # the common per-step call: the compiled binding walks the layers (None: not built, or a case it leaves to us)
         fp = ps.fast()
         first = kv[ps.gather[0]][0] if len(kv) == len(ps.plans) else None
@@ -307,6 +337,7 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
                 offs.append(offs[-1] + sz * esz)
         plan_buf = bytearray(_PLAN.size * n)
         io_buf = bytearray(_IO.size * n)
+        carry_buf = bytearray(_CARRY.size * n) if carry else None
         host_temps = False  # pinned temporaries made here: they must outlive the launch that reads them
         for m, (li, keys, values) in enumerate(members):
             plan = ps.plans[li]
@@ -368,6 +399,8 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
                     raise RuntimeError(f"layer {li}: stored norms of a host-resident cache must be pinned")
                 norms_ptr, nsb, nsh = nt.data_ptr(), nt.stride(0), nt.stride(1)
                 keepalive.append(nt)
+            if carry_buf is not None and carry.get(li) is not None:
+                carry_buf[m * _CARRY.size:(m + 1) * _CARRY.size] = carry_record(li, carry[li], B, H, dtype, plan.seq_len)
             plan_buf[m * _PLAN.size:(m + 1) * _PLAN.size] = ps.packed[li]
             ks, vs = keys.stride(), values.stride()
             _IO.pack_into(io_buf, m * _IO.size, keys.data_ptr(), values.data_ptr(), k_out_ptr, v_out_ptr,
@@ -388,8 +421,12 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
             ws = torch.empty((need[1],), dtype=torch.uint8, device=run_device)
             keepalive.append(ws)
             ws_ptr, ws_bytes = ctypes.c_void_p(ws.data_ptr()), need[1]
-        status = lib.kvc_compress_layers_ws(shape_rec, n, plan_bytes, bytes(io_buf), ws_ptr, ws_bytes,
-                                            ctypes.c_void_p(_stream_ptr(run_device)))
+        if carry_buf is not None:
+            status = lib.kvc_compress_layers_carry(shape_rec, n, plan_bytes, bytes(io_buf), bytes(carry_buf), ws_ptr,
+                                                   ws_bytes, ctypes.c_void_p(_stream_ptr(run_device)))
+        else:
+            status = lib.kvc_compress_layers_ws(shape_rec, n, plan_bytes, bytes(io_buf), ws_ptr, ws_bytes,
+                                                ctypes.c_void_p(_stream_ptr(run_device)))
         _check(status, "kvc_compress_layers")
         if on_host and (host_temps or not (non_blocking or to_device)):
             # host tensors are read by the caller with plain loads: finish before returning, as the reference's

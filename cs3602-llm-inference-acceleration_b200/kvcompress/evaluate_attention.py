@@ -15,6 +15,14 @@ runs on the device as well: one accumulate launch per update, one compaction lau
 updates an :class:`H2OScoreSlab` (the default manager then) from the recorded queries and keys: the probabilities are
 rebuilt on the device from fp32 logits.  ``tokenizer`` only needs ``encode(text, return_tensors="pt")`` — pass
 ``input_ids=`` to skip it (offline runs).
+
+Two semantics of the scores across a compression:
+
+* ``carry_scores=False`` (the default, the reference's reset): after every compression the manager starts over, so
+  at steady state (a compression per token) the heavy hitters are ranked by the current token's attention alone;
+* ``carry_scores=True`` (cumulative H2O): an ``H2OScoreSlab(carry_scores=True)`` moves its accumulators with the kept
+  rows inside the compaction launch; the loop updates the manager once per forward, compresses without handing the
+  scores over a second time and never resets, so keys are ranked by the decayed attention of the whole generation.
 """
 
 from __future__ import annotations
@@ -38,11 +46,12 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                                         skip_layers: List[int] = [0, 1], device: Optional[torch.device] = None,
                                         show_progress: bool = True, *, input_ids: Optional[torch.Tensor] = None,
                                         cache: str = "dynamic", return_nlls: bool = False,
-                                        scores: str = "attentions") -> Dict[str, float]:
+                                        scores: str = "attentions", carry_scores: bool = False) -> Dict[str, float]:
     """PPL / accuracy / TTFT / TPOT with attention-score H2O applied after every token.  ``h2o_manager``: an
     :class:`H2OAttentionManager` (the default) or an :class:`H2OScoreSlab`; ``cache``: ``"dynamic"`` or ``"slab"``;
     ``scores``: ``"attentions"`` (``output_attentions=True``) or ``"queries"`` (:func:`kvcompress.capture_queries`, an
-    :class:`H2OScoreSlab` manager)."""
+    :class:`H2OScoreSlab` manager); ``carry_scores``: cumulative scores (an ``H2OScoreSlab(carry_scores=True)``, the
+    default manager then) instead of the reference's reset after every compression."""
     if cache not in ("dynamic", "slab"):
         raise ValueError(f"cache must be 'dynamic' or 'slab', got {cache!r}")
     if scores not in ("attentions", "queries"):
@@ -50,13 +59,17 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
     if device is None:
         device = next(model.parameters()).device
     if h2o_manager is None:
-        manager_cls = H2OScoreSlab if scores == "queries" else H2OAttentionManager
+        manager_cls = H2OScoreSlab if scores == "queries" or carry_scores else H2OAttentionManager
+        extra = dict(carry_scores=True) if carry_scores else {}
         h2o_manager = manager_cls(start_size=start_size, heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
                                   num_layers=getattr(model.config, "num_hidden_layers", 32),
-                                  num_heads=getattr(model.config, "num_attention_heads", 32), device=device)
+                                  num_heads=getattr(model.config, "num_attention_heads", 32), device=device, **extra)
     else:
         if scores == "queries" and not isinstance(h2o_manager, H2OScoreSlab):
             raise ValueError("scores='queries' needs an H2OScoreSlab manager")
+        if carry_scores and not (isinstance(h2o_manager, H2OScoreSlab) and h2o_manager.carry_scores):
+            raise ValueError("carry_scores=True needs an H2OScoreSlab(carry_scores=True) manager; "
+                             f"got {type(h2o_manager).__name__} (the torch manager keeps the reference's reset)")
         h2o_manager.reset()
     use_queries = scores == "queries"
     if input_ids is None:
@@ -98,6 +111,8 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                                 output_attentions=True)
                 attentions = outputs.attentions
                 scored = dict(attention_scores=attentions)
+            if carry_scores:  # updated once per forward below; the compaction carries the accumulators
+                scored = {}
             logits = outputs.logits[:, -1, :].view(-1, vocab)
             target = input_ids[:, idx + 1:idx + 2].view(-1)
             nlls.append(float(loss_fn(logits, target).mean().item()))
@@ -116,7 +131,8 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                     slab.compress_("h2o_attention", h2o_manager=h2o_manager, start_size=start_size,
                                    heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
                                    skip_layers=skip_layers, **scored)
-                    h2o_manager.reset()
+                    if not carry_scores:
+                        h2o_manager.reset()
             else:
                 past_key_values = outputs.past_key_values
                 update()
@@ -127,7 +143,8 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                                                       heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
                                                       skip_layers=skip_layers, **scored)
                         past_key_values = to_dynamic_cache(kept)
-                        h2o_manager.reset()
+                        if not carry_scores:
+                            h2o_manager.reset()
             token_time = time.perf_counter() - token_start
             token_times.append(token_time)
             if ttft is None:

@@ -16,6 +16,14 @@ Two managers keep the score bookkeeping:
   one ``kvc_h2o_accumulate`` launch per update for every layer, and the compaction ranks the rows from the score
   row itself (``KVC_SCORE_GIVEN_SCORE_SHARED``) — no ATen kernel and no host synchronisation on the decode path,
   and every batch entry gets its own heavy hitters.
+
+Two semantics of the accumulators across a compaction:
+
+* reset (the reference's, and the default): the caller resets the manager after every compression, so the heavy
+  hitters are ranked by the attention received since the last compaction — at steady state, by one token's attention;
+* cumulative (``H2OScoreSlab(carry_scores=True)``): the compaction moves every accumulator row with its token, in the
+  same launch (``kvc_*_carry``), and the caller never resets — keys are ranked by the decayed attention they have
+  received over the whole generation.
 """
 
 from collections.abc import Mapping
@@ -105,13 +113,32 @@ def update_manager(h2o_manager, attention_scores=None, attention_queries=None, s
         h2o_manager.update_attention_scores(attention_scores, list(skip_layers))
 
 
+def check_carry(h2o_manager, carry_scores: Optional[bool]) -> None:
+    """``carry_scores`` of a compress call (None: the manager's own setting) must agree with the manager: cumulative
+    scores need an ``H2OScoreSlab(carry_scores=True)``; the torch manager keeps the reference's reset semantics."""
+    if carry_scores is None:
+        return
+    carries = isinstance(h2o_manager, H2OScoreSlab) and h2o_manager.carry_scores
+    if bool(carry_scores) != carries:
+        raise ValueError(f"carry_scores={carry_scores} needs an h2o_manager that "
+                         f"{'is H2OScoreSlab(carry_scores=True)' if carry_scores else 'does not carry its scores'}; "
+                         f"got {type(h2o_manager).__name__}"
+                         + (f"(carry_scores={h2o_manager.carry_scores})" if isinstance(h2o_manager, H2OScoreSlab) else ""))
+
+
 def h2o_attention_compress(past_key_values, attention_scores=None, h2o_manager: Optional[H2OAttentionManager] = None,
                            start_size: int = 4, heavy_hitter_size: int = 64, recent_size: int = 444,
-                           skip_layers: List[int] = [], attention_queries=None,
+                           skip_layers: List[int] = [], attention_queries=None, carry_scores: Optional[bool] = None,
                            **kwargs) -> List[Tuple[torch.Tensor, torch.Tensor]]:
     """Sinks + heavy hitters + recent window; heavy hitters come from ``h2o_manager`` when given,
     otherwise from the lowest key norms (identical to ``h2o_l2_compress``).  ``attention_queries``: a
-    :class:`kvcompress.QueryCapture` to update an :class:`H2OScoreSlab` from, instead of ``attention_scores``."""
+    :class:`kvcompress.QueryCapture` to update an :class:`H2OScoreSlab` from, instead of ``attention_scores``.
+
+    Reset semantics (the reference's): the caller resets the manager after the compression.  Cumulative semantics:
+    with ``H2OScoreSlab(carry_scores=True)`` the manager's accumulators are compacted in place with the kept rows, in
+    the gather launch itself, and the caller does not reset (update once per forward, then compress without passing the
+    scores again).  ``carry_scores`` (default: the manager's setting) must agree with the manager."""
+    check_carry(h2o_manager, carry_scores)
     layers = as_layer_list(past_key_values)
     if not layers:
         return layers
@@ -127,9 +154,13 @@ def h2o_attention_compress(past_key_values, attention_scores=None, h2o_manager: 
         keys = next((layers[li][0] for li in plans.gather), None)
         if keys is None:
             return execute(layers, plans)
-        plans, given, scores = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,
-                                                          keys.size(0), keys.size(1), keys.dtype, keys.device)
-        return _engine.run_plans(layers, plans, given_indices=given, given_scores=scores)
+        plans, given, scores, *carry = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,
+                                                                  keys.size(0), keys.size(1), keys.dtype, keys.device)
+        carry = carry[0] if carry else None
+        out = _engine.run_plans(layers, plans, given_indices=given, given_scores=scores, carry=carry)
+        if carry is not None:
+            h2o_manager.carried(plans, carry)
+        return out
     plans, given = manager_plans(layers, plans, h2o_manager, heavy_hitter_size)
     return execute(layers, plans, given_indices=given)
 
@@ -191,11 +222,18 @@ class H2OScoreSlab:
     ``[start_size, key_len - recent_size)``.  At compression the score row is handed to the compaction as
     ``KVC_SCORE_GIVEN_SCORE_SHARED``: each batch entry keeps its own heavy hitters, shared by its KV heads (the sum
     runs over all ``Hq`` query heads, so GQA models need nothing else).  The host decides everything from integers it
-    holds — no ``.item()``, no synchronisation.  ``reset`` touches no device memory."""
+    holds — no ``.item()``, no synchronisation.  ``reset`` touches no device memory.
+
+    ``carry_scores=False`` (reset semantics, the reference's): the accumulators describe rows by position, so the
+    caller resets the manager after every compression.  ``carry_scores=True`` (cumulative semantics): every compaction
+    through this manager also moves the accumulator rows of every compressed layer it holds data for with their tokens
+    — ``acc[:, h*G+g, i] = acc[:, h*G+g, src(i)]`` in the same launch that moves K and V — after which the layer holds
+    ``C`` valid entries and its next update decays them and zero-extends the new row.  The caller then never resets:
+    keys are ranked by the decayed attention they have received over the whole generation."""
 
     def __init__(self, start_size: int = 4, heavy_hitter_size: int = 64, recent_size: int = 444,
                  num_layers: int = 32, num_heads: int = 32, decay_factor: float = 0.9, device=None,
-                 capacity: Optional[int] = None):
+                 capacity: Optional[int] = None, carry_scores: bool = False):
         self.start_size = start_size
         self.heavy_hitter_size = heavy_hitter_size
         self.recent_size = recent_size
@@ -205,6 +243,7 @@ class H2OScoreSlab:
         self.decay_factor = decay_factor
         self.device = device
         self.capacity = capacity
+        self.carry_scores = bool(carry_scores)
         self.current_seq_len = 0
         self._acc: Optional[torch.Tensor] = None    # [L, B, Hq, capacity]
         self._score: Optional[torch.Tensor] = None  # [L, B, capacity]; row l holds [B, hi - lo] densely
@@ -388,8 +427,25 @@ class H2OScoreSlab:
         of ``[batch, heads, S, D]`` ``dtype`` layers.  Returns ``(PlanSet, given_indices, given_scores)``: layers with
         accumulated scores rank ``[sel_lo, sel_lo + region)`` by their score row (``SCORE_GIVEN_SCORE_SHARED``), layers
         without data since the last reset keep evenly spaced rows (``SCORE_GIVEN_INDEX``), an empty region keeps no
-        heavy hitter.  Score rows whose region differs from the last update's are re-scored in one launch."""
+        heavy hitter.  Score rows whose region differs from the last update's are re-scored in one launch.
+        With ``carry_scores=True`` a fourth item follows: ``{layer: (acc, group, prev_len)}`` for every compressed layer
+        this manager holds accumulators for (``run_plans`` / ``apply_plans_`` ``carry=``); after the launch, hand the
+        plans and that dict to :meth:`carried`."""
         device = torch.device(device)
+        carry = None
+        if self.carry_scores:
+            carry = {}
+            held = [li for li in plans.gather if li in self._lens]
+            if held:
+                acc = self._acc
+                if acc.dtype != dtype:
+                    raise ValueError(f"H2OScoreSlab: the attention dtype {acc.dtype} differs from the cache dtype {dtype}")
+                if acc.size(1) != batch or acc.device != device or acc.size(2) % heads:
+                    raise ValueError(f"H2OScoreSlab: accumulators [B={acc.size(1)}, Hq={acc.size(2)}] on {acc.device}, "
+                                     f"cache [B={batch}, Hkv={heads}] on {device}")
+                self._ensure(batch, acc.size(2), dtype, device, max(plans.plans[li].seq_len for li in held))
+                group = self._acc.size(2) // heads
+                carry = {li: (self._acc[li], group, self._lens[li]) for li in held}
         decisions, rescore = [], []
         for li in plans.gather:
             p = plans.plans[li]
@@ -428,7 +484,7 @@ class H2OScoreSlab:
         key = (id(plans), self._gen, batch, heads, device, tuple(decisions))
         hit = self._plan_cache.get(key)
         if hit is not None and hit[0] is plans:
-            return hit[1], hit[2], hit[3]
+            return hit[1:] if carry is None else hit[1:] + (carry,)
         new_plans, given, scores = list(plans.plans), {}, {}
         for li, d in zip(plans.gather, decisions):
             if d is None:
@@ -460,7 +516,16 @@ class H2OScoreSlab:
         if len(self._plan_cache) > 64:
             self._plan_cache.clear()
         self._plan_cache[key] = (plans, ps, given or None, scores or None)
+        if carry is not None:
+            return ps, given or None, scores or None, carry
         return ps, given or None, scores or None
+
+    def carried(self, plans, carry: dict) -> None:
+        """Bookkeeping after a compaction that carried ``carry`` (from :meth:`compress_plans`) with ``plans``: each
+        carried layer now holds ``C`` valid entries, and its score row is stale."""
+        for li in carry:
+            self._lens[li] = plans.plans[li].out_len
+            self._scored.pop(li, None)
 
 
 def create_h2o_manager_from_model(model, **kwargs) -> H2OAttentionManager:
@@ -478,4 +543,4 @@ def create_h2o_manager_from_model(model, **kwargs) -> H2OAttentionManager:
 
 
 __all__ = ["H2OAttentionManager", "H2OScoreSlab", "h2o_attention_compress", "create_h2o_manager_from_model",
-           "manager_plans", "update_manager"]
+           "manager_plans", "update_manager", "check_carry"]

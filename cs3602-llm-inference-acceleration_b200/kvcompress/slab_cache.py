@@ -411,14 +411,18 @@ class KVSlabCache:
 
     def _compress_h2o_attention(self, attention_scores=None, h2o_manager=None, start_size: int = 4,
                                 heavy_hitter_size: int = 64, recent_size: int = 444, skip_layers: Sequence[int] = (),
-                                return_indices: bool = False, attention_queries=None, **_ignored):
+                                return_indices: bool = False, attention_queries=None,
+                                carry_scores: Optional[bool] = None, **_ignored):
         """``h2o_attention_compress`` in place (reference h2o_attention.py:216-363): without a manager it is exactly
         ``h2o_l2`` (:337-351); with one, its head-summed heavy hitters are the caller-supplied rows of the in-place
         compaction (they must ascend strictly — the manager sorts them, a clamp collision is refused).
-        ``attention_queries``: a ``QueryCapture`` that updates an ``H2OScoreSlab`` instead of ``attention_scores``."""
+        ``attention_queries``: a ``QueryCapture`` that updates an ``H2OScoreSlab`` instead of ``attention_scores``.
+        With ``H2OScoreSlab(carry_scores=True)`` the accumulators slide with the rows in the same launch (cumulative
+        H2O); ``carry_scores`` (default: the manager's setting) must agree with the manager."""
         from .methods._common import cached_plans
-        from .methods.h2o_attention import H2OScoreSlab, manager_plans, update_manager
+        from .methods.h2o_attention import H2OScoreSlab, check_carry, manager_plans, update_manager
 
+        check_carry(h2o_manager, carry_scores)
         if h2o_manager is None:
             if attention_queries is not None:
                 raise ValueError("attention_queries needs an H2OScoreSlab manager (h2o_manager=)")
@@ -427,9 +431,15 @@ class KVSlabCache:
         update_manager(h2o_manager, attention_scores, attention_queries, skip_layers)
         plans = cached_plans(P.plan_h2o, self.lengths, start_size, heavy_hitter_size, recent_size, skip_layers=skip_layers)
         if isinstance(h2o_manager, H2OScoreSlab):  # scores ranked on the device: no host round trip
-            plans, given, scores = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,
-                                                              self.batch, self.heads, self.dtype, self.device)
-            return self.apply_plans_(plans, given_indices=given, given_scores=scores, return_indices=return_indices)
+            plans, given, scores, *carry = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size,
+                                                                      recent_size, self.batch, self.heads, self.dtype,
+                                                                      self.device)
+            carry = carry[0] if carry else None
+            res = self.apply_plans_(plans, given_indices=given, given_scores=scores, return_indices=return_indices,
+                                    carry=carry)
+            if carry is not None:
+                h2o_manager.carried(plans, carry)
+            return res
         plans, given = manager_plans(self.to_legacy_cache(), plans, h2o_manager, heavy_hitter_size)
         for li, rows in given.items():
             if rows.size(-1) > 1 and not bool((rows[0, 0, 1:] > rows[0, 0, :-1]).all()):
@@ -447,7 +457,9 @@ class KVSlabCache:
         return self.apply_plans_(plans, return_indices=return_indices)
 
     def apply_plans_(self, plans, given_indices: Optional[dict] = None, return_indices: bool = False,
-                     given_scores: Optional[dict] = None):
+                     given_scores: Optional[dict] = None, carry: Optional[dict] = None):
+        """Compact every GATHER layer of ``plans`` in place, in one launch.  ``carry``: {layer: (acc, group,
+        prev_len)} per-row state that slides with the kept rows in the same launch (see :func:`_engine.run_plans`)."""
         ps = plans if isinstance(plans, _engine.PlanSet) else _engine.PlanSet(plans)
         if len(ps) != self.num_layers:
             raise ValueError(f"{len(ps)} plans for {self.num_layers} layers")
@@ -511,8 +523,15 @@ class KVSlabCache:
             if self._ws is None or self._ws.numel() < ws_need:
                 self._ws = torch.empty((ws_need,), dtype=torch.uint8, device=self.device)
             ws_ptr = ctypes.c_void_p(self._ws.data_ptr())
-        status = lib.kvc_slab_compress(self._shape, len(ids), plan_buf, slab_buf, idx_out, idx_in, ws_ptr, ws_need,
-                                       ctypes.c_void_p(_engine._stream_ptr(self.device)))
+        if carry:
+            carry_buf = b"".join(_engine.carry_record(i, carry[i], self.batch, self.heads, self.dtype, n)
+                                 if carry.get(i) is not None else bytes(_engine._CARRY.size)
+                                 for i, n in zip(ids, in_lens))
+            status = lib.kvc_slab_compress_carry(self._shape, len(ids), plan_buf, slab_buf, idx_out, idx_in, carry_buf,
+                                                 ws_ptr, ws_need, ctypes.c_void_p(_engine._stream_ptr(self.device)))
+        else:
+            status = lib.kvc_slab_compress(self._shape, len(ids), plan_buf, slab_buf, idx_out, idx_in, ws_ptr, ws_need,
+                                           ctypes.c_void_p(_engine._stream_ptr(self.device)))
         _engine._check(status, "kvc_slab_compress")
         for i, c in zip(ids, out_lens):
             self.lengths[i] = c

@@ -47,7 +47,7 @@ extern "C" {
 #endif
 
 /* Additions that leave every existing struct layout, enum value and entry point as it was (a new score kind, the
- * kvc_h2o_layer / kvc_h2o_qk_layer structs and their entry points) keep the version: a caller built against an older header sees the
+ * kvc_h2o_layer / kvc_h2o_qk_layer / kvc_carry_layer structs and their entry points) keep the version: a caller built against an older header sees the
  * same ABI, and a caller that uses the additions fails to link or gets KVC_ERR_INVALID_ARG from an older library. */
 #define KVC_ABI_VERSION 5
 
@@ -307,6 +307,34 @@ int64_t kvc_h2o_qk_workspace_bytes(const kvc_shape* shape, int32_t group, int32_
                                    const kvc_h2o_qk_layer* layers);
 int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers,
                           float decay, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Per-row state that moves with the kept rows (cumulative H2O: the accumulators of kvc_h2o_accumulate keep describing
+ * the token they were accumulated for across a compaction).  Per layer, batch entry b, KV head h, g < group and output
+ * row i < C = sink + k_sel + tail, with src(i) the source row of output row i for KV head h:
+ *   acc'[b, h*group+g, i] = acc[b, h*group+g, src(i)]   if src(i) < min(prev_len, seq_len)
+ *                         = 0                           otherwise
+ * The copy is bit-exact, in place, and runs in the same launch as the compaction / gather of K and V (the CTA that
+ * moves a (layer, b, h)'s rows moves its `group` accumulator rows).  Entries at and past C are unspecified afterwards.
+ * carry == NULL, or acc == NULL on every layer, is exactly kvc_slab_compress / kvc_compress_layers_ws.
+ * KVC_ERR_INVALID_ARG, before any CUDA call, on a layer with a non-NULL acc: group < 1, prev_len < 0, or acc rows not
+ * aligned to the element size (4 bytes for fp32, 2 for 16-bit). */
+typedef struct kvc_carry_layer {
+    void* acc;                          /* [B, H*group, >= seq_len] per-row state, dtype = shape->dtype, last dim dense;
+                                           NULL: nothing to carry for this layer */
+    int64_t acc_stride_b, acc_stride_h; /* elements */
+    int32_t group;                      /* rows of acc per KV head (Hq / Hkv); KV head h owns acc heads [h*group, (h+1)*group) */
+    int32_t prev_len;                   /* valid entries before the compaction (clamped to seq_len) */
+} kvc_carry_layer;
+/* kvc_slab_compress with carry[l] for layer l (carry may be NULL). */
+int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
+                            const kvc_slab_layer* slabs, int32_t* const* idx_out, const int32_t* const* idx_in,
+                            const kvc_carry_layer* carry, void* workspace, int64_t workspace_bytes, void* stream);
+/* kvc_compress_layers_ws with carry[l] for layer l (carry may be NULL); K and V are still written out of place, only
+ * acc is compacted in place. */
+int kvc_compress_layers_carry(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
+                              const kvc_layer_io* io, const kvc_carry_layer* carry, void* workspace,
+                              int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
