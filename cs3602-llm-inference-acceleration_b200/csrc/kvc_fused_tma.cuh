@@ -184,6 +184,43 @@ __device__ __forceinline__ void keys_from_values(const typename Traits<DT>::Key*
     }
 }
 
+// Kept rows of a unit (layer descriptor L: LayerDev or SlabLayerDev, ksel > 0) from per-row values in memory:
+//   GIVEN_INDEX                       caller-supplied rows (L.idx_in, [B,H,ksel]), clamped into the layer so that a bad
+//                                     index can never become a wild bulk copy;
+//   GIVEN_SCORE / GIVEN_SCORE_SHARED  caller-supplied scores of the region's rows (cache dtype, in the idx_in slot:
+//                                     [B,H,R] per-head rows or [B,R] rows shared by the heads of a batch entry), pooled,
+//                                     the highest kept;
+//   otherwise                         stored key norms (norm_row: the unit's row of them), ranked like the scan would.
+// All NT threads call.  hist and misc[kMiscMaxRaw] are reset here, behind a barrier before their first reader; sidx is
+// complete after the caller's next __syncthreads().
+template <int DT, int NT, typename Layer>
+__device__ __forceinline__ void select_from_memory(const Layer& L, const typename Traits<DT>::Key* norm_row, int b, int bh,
+                                                   typename Traits<DT>::Key* keys, uint32_t* hist, int32_t* misc,
+                                                   int32_t* sidx) {
+    using Key = typename Traits<DT>::Key;
+    const int tid = threadIdx.x;
+    const int R = L.hi - L.lo;
+    if (L.score == KVC_SCORE_GIVEN_INDEX) {
+        const int32_t* src = L.idx_in + (int64_t)bh * L.ksel;
+        for (int i = tid; i < L.ksel; i += NT) sidx[i] = min(max(src[i], 0), L.S - 1);
+        return;
+    }
+    for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;
+    if (tid == 0) misc[kMiscMaxRaw] = 0;
+    __syncthreads();
+    if (L.score == KVC_SCORE_GIVEN_SCORE || L.score == KVC_SCORE_GIVEN_SCORE_SHARED) {
+        const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)(L.score == KVC_SCORE_GIVEN_SCORE ? bh : b) * R;
+        load_keys_vectorised<DT, NT>(src, R, keys, [&](int i, uint32_t raw) { keys[i] = (Key)raw; });
+        __syncthreads();
+        snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc, /*invert=*/false);
+    } else {
+        keys_from_values<DT, NT>(norm_row + L.lo, R, L.score, keys, hist, misc);
+        __syncthreads();
+        if (L.score == KVC_SCORE_SNAPKV_POOL) snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc);
+    }
+    block_radix_select<Key, NT>(keys, R, L.ksel, hist, misc, sidx, L.lo);
+}
+
 template <int DT, int CPR, int NT, int MINB>
 __global__ void __launch_bounds__(NT, MINB) kvc_fused_tma_kernel(const __grid_constant__ BatchDev bd) {
     using Tr = Traits<DT>;
@@ -239,29 +276,11 @@ __global__ void __launch_bounds__(NT, MINB) kvc_fused_tma_kernel(const __grid_co
     if (scan && stager && warp < nblk)  // first block is in flight while the histogram is cleared
         warp_load_rows(slot, bar, kreg + (int64_t)(warp * 32 + lane) * L.kss, min(32, R - warp * 32), kdense, lane, RB);
 
-    if (ksel > 0 && score == KVC_SCORE_GIVEN_INDEX) {
-        // caller-supplied rows: clamped into the layer so that a bad index can never become a wild bulk copy
-        const int32_t* src = L.idx_in + (int64_t)bh * ksel;
-        for (int i = tid; i < ksel; i += NT) sidx[i] = min(max(src[i], 0), L.S - 1);
-    } else if (ksel > 0 && by_value) {
-        // ---------------------------------------------------------- per-row values from memory: stored key norms
-        // (ranked like the scan would rank them) or caller-supplied scores (pooled, the highest kept)
-        for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;
-        if (tid == 0) misc[kMiscMaxRaw] = 0;
-        __syncthreads();
-        if (given_score) {
-            // [B,H,R] per-head rows, or [B,R] rows shared by the heads of a batch entry
-            const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)(score == KVC_SCORE_GIVEN_SCORE ? bh : b) * R;
-            load_keys_vectorised<DT, NT>(src, R, keys, [&](int i, uint32_t raw) { keys[i] = (Key)raw; });
-            __syncthreads();
-            snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc, /*invert=*/false);
-        } else {
-            const Key* src = reinterpret_cast<const Key*>(L.n_in + (int64_t)b * L.nsb + (int64_t)h * L.nsh) + L.lo;
-            keys_from_values<DT, NT>(src, R, score, keys, hist, misc);
-            __syncthreads();
-            if (score == KVC_SCORE_SNAPKV_POOL) snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc);
-        }
-        block_radix_select<Key, NT>(keys, R, ksel, hist, misc, sidx, L.lo);
+    if (ksel > 0 && (score == KVC_SCORE_GIVEN_INDEX || by_value)) {
+        // ---------------------------------------------------------- kept rows, scores or stored key norms from memory
+        const Key* norm_row = L.n_in ? reinterpret_cast<const Key*>(L.n_in + (int64_t)b * L.nsb + (int64_t)h * L.nsh)
+                                     : nullptr;
+        select_from_memory<DT, NT>(L, norm_row, b, bh, keys, hist, misc, sidx);
     } else if (ksel > 0) {
         // ---------------------------------------------------------- K1: scan
         for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;

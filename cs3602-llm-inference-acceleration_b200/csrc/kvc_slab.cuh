@@ -234,9 +234,7 @@ __global__ void __launch_bounds__(NT, MINB) kvc_slab_compress_kernel(const __gri
     }
     __syncwarp();
 
-    const int R = L.hi - L.lo;
     const int ksel = L.ksel;
-    const int score = L.score;
     char* kbase = L.k + (int64_t)b * L.ksb + (int64_t)h * L.ksh;
     char* vbase = L.v + (int64_t)b * L.vsb + (int64_t)h * L.vsh;
     Key* nbase = reinterpret_cast<Key*>(L.n + (int64_t)b * L.nsb + (int64_t)h * L.nsh);
@@ -244,35 +242,10 @@ __global__ void __launch_bounds__(NT, MINB) kvc_slab_compress_kernel(const __gri
     const int C = sink + ksel + L.tail;
     const int tail0 = L.S - L.tail - sink - ksel;  // src row = j + tail0 for tail rows
 
-    if (tid == 0) {
-        misc[kMiscMaxRaw] = 0;
-        misc[kMiscFirst] = C;
-    }
-    if (ksel > 0 && score == KVC_SCORE_GIVEN_INDEX) {
-        // caller-supplied rows: strictly ascending absolute rows of the region (kvc.h); clamped into the slab so
-        // that a bad index can never become a wild bulk copy
-        const int32_t* src = L.idx_in + (int64_t)bh * ksel;
-        for (int i = tid; i < ksel; i += NT) sidx[i] = min(max(src[i], 0), L.S - 1);
-    } else if (ksel > 0 && (score == KVC_SCORE_GIVEN_SCORE || score == KVC_SCORE_GIVEN_SCORE_SHARED)) {
-        // caller-supplied scores of the region's rows ([B,H,R], or [B,R] shared by the heads of a batch entry; cache
-        // dtype, handed over in the idx_in slot): pooled, the highest kept (the vote mode of snapkv_lite, H2O's
-        // head-summed attention mass; same steps as the fused kernel's GIVEN_SCORE branch)
-        for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;
-        __syncthreads();
-        const Key* src = reinterpret_cast<const Key*>(L.idx_in) + (int64_t)(score == KVC_SCORE_GIVEN_SCORE ? bh : b) * R;
-        load_keys_vectorised<DT, NT>(src, R, keys, [&](int i, uint32_t raw) { keys[i] = (Key)raw; });
-        __syncthreads();
-        snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc, /*invert=*/false);
-        block_radix_select<Key, NT>(keys, R, ksel, hist, misc, sidx, L.lo);
-    } else if (ksel > 0) {
-        // ---------------------------------------------------------- keys from the stored norms
-        for (int i = tid; i < kHistBins; i += NT) hist[i] = 0;
-        __syncthreads();
-        keys_from_values<DT, NT>(nbase + L.lo, R, score, keys, hist, misc);
-        __syncthreads();
-        if (score == KVC_SCORE_SNAPKV_POOL) snapkv_transform<DT, NT>(keys, R, L.pool, hist, misc);
-        block_radix_select<Key, NT>(keys, R, ksel, hist, misc, sidx, L.lo);
-    }
+    if (tid == 0) misc[kMiscFirst] = C;
+    // kept rows (strictly ascending absolute rows of the region, kvc.h), scores (the vote mode of snapkv_lite, H2O's
+    // head-summed attention mass) or the stored norms
+    if (ksel > 0) select_from_memory<DT, NT>(L, nbase, b, bh, keys, hist, misc, sidx);
     __syncthreads();
 
     const KeepMap src_row{sidx, sink, ksel, tail0};

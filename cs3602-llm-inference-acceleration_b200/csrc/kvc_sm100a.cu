@@ -16,6 +16,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -120,6 +121,50 @@ static int cuda_fail(cudaError_t e, const char* what) {
     snprintf(g_last_error, sizeof(g_last_error), "%s: %s", what, cudaGetErrorString(e));
     return KVC_ERR_CUDA;
 }
+
+// After a kernel launch: a launch error becomes KVC_ERR_CUDA with `what` in kvc_last_cuda_error, a launch is counted.
+static int launched(const char* what) {
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, what);
+    g_launches.fetch_add(1);
+    return KVC_OK;
+}
+
+// Calls f(l0, nl) for the layers [l0, l0 + nl) of each launch (at most KVC_MAX_LAYERS_PER_LAUNCH layers); the first
+// status other than KVC_OK ends the walk and is returned.
+template <class F>
+static int for_each_chunk(int n_layers, F&& f) {
+    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
+        const int st = f(l0, std::min(n_layers - l0, KVC_MAX_LAYERS_PER_LAUNCH));
+        if (st != KVC_OK) return st;
+    }
+    return KVC_OK;
+}
+
+// Kernel tables: f(std::integral_constant<int, X>{}) for the run-time value, so that f can name the instantiation.
+// Rows of 16 B .. 2 KB: 128/160/192/256/320/512-byte rows (cpr 8/10/12/16/20/32) have kernels with compile-time widths,
+// the rest run the generic-width (0) instantiation of the same kernels.
+template <class F>
+static auto by_cpr(int cpr, F&& f) {
+    switch (cpr) {
+        case 8: return f(std::integral_constant<int, 8>{});
+        case 10: return f(std::integral_constant<int, 10>{});
+        case 12: return f(std::integral_constant<int, 12>{});
+        case 16: return f(std::integral_constant<int, 16>{});
+        case 20: return f(std::integral_constant<int, 20>{});
+        case 32: return f(std::integral_constant<int, 32>{});
+        default: return f(std::integral_constant<int, 0>{});
+    }
+}
+template <class F>
+static auto by_dtype(int dtype, F&& f) {
+    switch (dtype) {
+        case KVC_DTYPE_F32: return f(std::integral_constant<int, KVC_DTYPE_F32>{});
+        case KVC_DTYPE_F16: return f(std::integral_constant<int, KVC_DTYPE_F16>{});
+        default: return f(std::integral_constant<int, KVC_DTYPE_BF16>{});
+    }
+}
+static bool row_width_ok(int cpr) { return cpr >= 1 && cpr <= 128; }
 
 static int elem_bytes(int dtype) { return dtype == KVC_DTYPE_F32 ? 4 : 2; }
 static int key_bytes(int dtype) { return dtype == KVC_DTYPE_F32 ? 4 : 2; }
@@ -332,21 +377,11 @@ static bool onchip_plan_ok(const TmaPlan& tp, int cpr, bool light_traffic) {
 }
 
 #if KVC_HAS_CORE || KVC_HAS_FUSED_OTHER
-template <int DT, int NT, int MINB>
-static FusedFn pick_tma_cpr(int cpr) {
-    switch (cpr) {
-        case 8: return kvc_fused_tma_kernel<DT, 8, NT, MINB>;
-        case 10: return kvc_fused_tma_kernel<DT, 10, NT, MINB>;
-        case 12: return kvc_fused_tma_kernel<DT, 12, NT, MINB>;
-        case 16: return kvc_fused_tma_kernel<DT, 16, NT, MINB>;
-        case 20: return kvc_fused_tma_kernel<DT, 20, NT, MINB>;
-        case 32: return kvc_fused_tma_kernel<DT, 32, NT, MINB>;
-        default: return kvc_fused_tma_kernel<DT, 0, NT, MINB>;  // any other row width: run-time loops
-    }
-}
 template <int DT>
 static FusedFn pick_tma_nt(int cpr, int nt) {
-    return nt == 512 ? pick_tma_cpr<DT, 512, 1>(cpr) : pick_tma_cpr<DT, 256, 3>(cpr);
+    return by_cpr(cpr, [&](auto c) {
+        return nt == 512 ? FusedFn(kvc_fused_tma_kernel<DT, c, 512, 1>) : FusedFn(kvc_fused_tma_kernel<DT, c, 256, 3>);
+    });
 }
 #endif
 FusedFn pick_tma_bf16(int cpr, int nt);
@@ -362,10 +397,6 @@ FusedFn pick_tma_other(int dtype, int cpr, int nt) {
     return dtype == KVC_DTYPE_F32 ? pick_tma_nt<KVC_DTYPE_F32>(cpr, nt) : pick_tma_nt<KVC_DTYPE_F16>(cpr, nt);
 }
 #endif
-
-// Rows of 16 B .. 2 KB: 128/160/192/256/320/512-byte rows have kernels with compile-time widths, the rest run the
-// generic-width instantiation of the same kernels.
-static bool row_width_ok(int cpr) { return cpr >= 1 && cpr <= 128; }
 
 static int ensure_tma_attrs(const void* fn, int device) {
     // Function attributes are sticky per (function, device): set them once, not on every decode step.
@@ -397,21 +428,11 @@ AppendOneFn pick_append_one(int dtype, int cpr);   // thread-per-row form, one l
 AppendFn pick_append_tma(int dtype, int cpr);      // bulk-copy form (prefill-sized appends)
 
 #if KVC_HAS_SLAB || KVC_HAS_SLAB_OTHER
-template <int DT, int NT, int MINB>
-static SlabFn pick_slab_cpr(int cpr) {
-    switch (cpr) {
-        case 8: return kvc_slab_compress_kernel<DT, 8, NT, MINB>;
-        case 10: return kvc_slab_compress_kernel<DT, 10, NT, MINB>;
-        case 12: return kvc_slab_compress_kernel<DT, 12, NT, MINB>;
-        case 16: return kvc_slab_compress_kernel<DT, 16, NT, MINB>;
-        case 20: return kvc_slab_compress_kernel<DT, 20, NT, MINB>;
-        case 32: return kvc_slab_compress_kernel<DT, 32, NT, MINB>;
-        default: return kvc_slab_compress_kernel<DT, 0, NT, MINB>;
-    }
-}
 template <int DT>
 static SlabFn pick_slab_nt(int cpr, int nt) {
-    return nt == 512 ? pick_slab_cpr<DT, 512, 1>(cpr) : pick_slab_cpr<DT, 256, 3>(cpr);
+    return by_cpr(cpr, [&](auto c) {
+        return nt == 512 ? SlabFn(kvc_slab_compress_kernel<DT, c, 512, 1>) : SlabFn(kvc_slab_compress_kernel<DT, c, 256, 3>);
+    });
 }
 #endif
 #if KVC_HAS_SLAB
@@ -427,50 +448,20 @@ SlabFn pick_slab_other(int dtype, int cpr, int nt) {
 #endif
 
 #if KVC_HAS_APPEND
-template <int DT, typename Params>
-static void (*pick_append_row_cpr(int cpr))(const Params) {
-    switch (cpr) {
-        case 8: return kvc_slab_append_kernel<DT, 8, Params>;
-        case 10: return kvc_slab_append_kernel<DT, 10, Params>;
-        case 12: return kvc_slab_append_kernel<DT, 12, Params>;
-        case 16: return kvc_slab_append_kernel<DT, 16, Params>;
-        case 20: return kvc_slab_append_kernel<DT, 20, Params>;
-        case 32: return kvc_slab_append_kernel<DT, 32, Params>;
-        default: return kvc_slab_append_kernel<DT, 0, Params>;
-    }
-}
-template <int DT>
-static AppendFn pick_append_tma_cpr(int cpr) {
-    switch (cpr) {
-        case 8: return kvc_slab_append_tma_kernel<DT, 8>;
-        case 10: return kvc_slab_append_tma_kernel<DT, 10>;
-        case 12: return kvc_slab_append_tma_kernel<DT, 12>;
-        case 16: return kvc_slab_append_tma_kernel<DT, 16>;
-        case 20: return kvc_slab_append_tma_kernel<DT, 20>;
-        case 32: return kvc_slab_append_tma_kernel<DT, 32>;
-        default: return kvc_slab_append_tma_kernel<DT, 0>;
-    }
-}
 AppendOneFn pick_append_one(int dtype, int cpr) {
-    switch (dtype) {
-        case KVC_DTYPE_F32: return pick_append_row_cpr<KVC_DTYPE_F32, AppendOneDev>(cpr);
-        case KVC_DTYPE_F16: return pick_append_row_cpr<KVC_DTYPE_F16, AppendOneDev>(cpr);
-        default: return pick_append_row_cpr<KVC_DTYPE_BF16, AppendOneDev>(cpr);
-    }
+    return by_dtype(dtype, [&](auto dt) {
+        return by_cpr(cpr, [&](auto c) { return AppendOneFn(kvc_slab_append_kernel<dt, c, AppendOneDev>); });
+    });
 }
 AppendFn pick_append(int dtype, int cpr) {
-    switch (dtype) {
-        case KVC_DTYPE_F32: return pick_append_row_cpr<KVC_DTYPE_F32, AppendBatchDev>(cpr);
-        case KVC_DTYPE_F16: return pick_append_row_cpr<KVC_DTYPE_F16, AppendBatchDev>(cpr);
-        default: return pick_append_row_cpr<KVC_DTYPE_BF16, AppendBatchDev>(cpr);
-    }
+    return by_dtype(dtype, [&](auto dt) {
+        return by_cpr(cpr, [&](auto c) { return AppendFn(kvc_slab_append_kernel<dt, c, AppendBatchDev>); });
+    });
 }
 AppendFn pick_append_tma(int dtype, int cpr) {
-    switch (dtype) {
-        case KVC_DTYPE_F32: return pick_append_tma_cpr<KVC_DTYPE_F32>(cpr);
-        case KVC_DTYPE_F16: return pick_append_tma_cpr<KVC_DTYPE_F16>(cpr);
-        default: return pick_append_tma_cpr<KVC_DTYPE_BF16>(cpr);
-    }
+    return by_dtype(dtype, [&](auto dt) {
+        return by_cpr(cpr, [&](auto c) { return AppendFn(kvc_slab_append_tma_kernel<dt, c>); });
+    });
 }
 #endif  // KVC_HAS_APPEND
 
@@ -486,26 +477,136 @@ static int check_shape(const kvc_shape* shape, int* cpr_out) {
     return KVC_OK;
 }
 
-// Arguments of a layer's kvc_carry_layer (a non-NULL acc): checked before anything is enqueued.  The copy runs in place,
-// so the kept rows must be a valid in-place compaction (the slab rule: C <= S, the selection region between the sinks
-// and the tail), which makes every source row lie at or above its output row.
-static inline bool carry_ok(const kvc_carry_layer* carry, int l, const kvc_layer_plan& p, int e) {
-    if (!carry || !carry[l].acc) return true;
-    const kvc_carry_layer& c = carry[l];
-    if (c.group < 1 || c.prev_len < 0 || ((uintptr_t)c.acc % (uintptr_t)e) != 0) return false;
+// A valid in-place compaction (the slab rule: C <= S, the selection region between the sinks and the tail), which makes
+// every kept source row lie at or above its output row.
+static inline bool in_place_ok(const kvc_layer_plan& p) {
     if ((int64_t)p.sink + p.k_sel + p.tail > p.seq_len) return false;
-    if (p.k_sel > 0 && (p.sel_lo < p.sink || p.sel_hi > p.seq_len - p.tail)) return false;
-    return true;
+    return p.k_sel <= 0 || (p.sel_lo >= p.sink && p.sel_hi <= p.seq_len - p.tail);
 }
 
-static inline void fill_carry(CarryDev& d, const kvc_carry_layer* carry, int l, const kvc_layer_plan& p, int e) {
-    if (!carry || !carry[l].acc) return;  // the descriptor was zeroed: acc == nullptr
-    const kvc_carry_layer& c = carry[l];
-    d.acc = (char*)c.acc;
-    d.asb = c.acc_stride_b * e;
-    d.ash = c.acc_stride_h * e;
-    d.group = c.group;
-    d.prev = c.prev_len < p.seq_len ? c.prev_len : p.seq_len;
+// The plan checks of one layer, for both compaction forms, before anything is enqueued: KVC_OK or the status of the
+// first failing check.  in_place: the kept rows are compacted within the layer's own rows.  has_idx / has_score: the
+// caller supplied the rows a GIVEN_INDEX plan keeps / the scores a GIVEN_SCORE(_SHARED) plan ranks.  carry: the layer's
+// kvc_carry_layer or nullptr; its copy runs in place, so a non-NULL acc needs a valid in-place compaction as well.
+static int check_plan(const kvc_layer_plan& p, bool in_place, bool has_idx, bool has_score, const kvc_carry_layer* carry,
+                      int e) {
+    if (p.seq_len < 0 || p.sink < 0 || p.k_sel < 0 || p.tail < 0) return KVC_ERR_INVALID_ARG;
+    if (p.sink > p.seq_len || p.tail > p.seq_len) return KVC_ERR_INVALID_ARG;
+    if (in_place && !in_place_ok(p)) return KVC_ERR_INVALID_ARG;
+    if (p.k_sel > 0) {
+        if (p.sel_lo < 0 || p.sel_hi > p.seq_len || p.sel_lo > p.sel_hi) return KVC_ERR_INVALID_ARG;
+        if (p.k_sel > p.sel_hi - p.sel_lo) return KVC_ERR_INVALID_ARG;
+        if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE_SHARED) return KVC_ERR_INVALID_ARG;
+        const bool given_score = p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_GIVEN_SCORE_SHARED;
+        if (p.score == KVC_SCORE_GIVEN_INDEX && !has_idx) return KVC_ERR_INVALID_ARG;
+        if (given_score && !has_score) return KVC_ERR_INVALID_ARG;
+        if ((given_score || p.score == KVC_SCORE_SNAPKV_POOL) && p.pool_kernel > 2 * kMaxPoolHalo)
+            return KVC_ERR_UNSUPPORTED;
+    }
+    if (carry && carry->acc) {
+        if (carry->group < 1 || carry->prev_len < 0 || ((uintptr_t)carry->acc % (uintptr_t)e) != 0)
+            return KVC_ERR_INVALID_ARG;
+        if (!in_place_ok(p)) return KVC_ERR_INVALID_ARG;
+    }
+    return KVC_OK;
+}
+
+// The layer ranks its region by key norms (scanned from K, or stored ones the caller holds).
+static inline bool ranked(const kvc_layer_plan& p) {
+    return p.k_sel > 0 &&
+           (p.score == KVC_SCORE_L2_LOW || p.score == KVC_SCORE_L2_HIGH || p.score == KVC_SCORE_SNAPKV_POOL);
+}
+
+// What one launch (layers [0, nl) of `plans`) has to plan for.  any_scan is only known with the io records: a ranked
+// layer whose caller holds no key norms reads its region of K.
+struct ChunkStats {
+    int n_active = 0;      // layers with C > 0
+    int max_region = 0;    // largest selection region whose radix keys are built (not GIVEN_INDEX)
+    int idx_cap = 0;       // kept-index entries reserved per unit (largest k_sel, rounded up to 4)
+    bool any_select = false, any_scan = false;
+    int64_t rows_moved = 0;  // rows the units move if they scan K: the region once + kept rows of K and V read and written
+};
+static ChunkStats chunk_stats(const kvc_layer_plan* plans, const kvc_layer_io* io, int nl) {
+    ChunkStats s;
+    int max_ksel = 0;
+    for (int l = 0; l < nl; ++l) {
+        const kvc_layer_plan& p = plans[l];
+        if (p.sink + p.k_sel + p.tail == 0) continue;
+        ++s.n_active;
+        s.rows_moved += (p.k_sel > 0 ? p.sel_hi - p.sel_lo : 0) + 4LL * (p.sink + p.k_sel + p.tail);
+        if (p.k_sel > 0) {
+            s.any_select = true;
+            s.any_scan |= io != nullptr && ranked(p) && !io[l].norms_in;
+            if (p.k_sel > max_ksel) max_ksel = p.k_sel;
+            if (p.score != KVC_SCORE_GIVEN_INDEX && p.sel_hi - p.sel_lo > s.max_region) s.max_region = p.sel_hi - p.sel_lo;
+        }
+    }
+    s.idx_cap = (max_ksel + 3) & ~3;
+    return s;
+}
+
+// The launch plan of one launch.  When the on-chip plan is not good enough (onchip_plan_ok) and a workspace may be
+// used, the radix keys and kept indices go to the workspace (layout w) and shared memory keeps the histogram and slots.
+struct LaunchPlan {
+    TmaPlan tp;
+    bool ws = false;
+    WsLayout w;
+};
+static LaunchPlan plan_launch(int dtype, int cpr, const ChunkStats& s, bool light_traffic, bool in_place, int64_t units,
+                              int64_t unit_bytes, bool may_use_ws) {
+    LaunchPlan lp;
+    lp.tp = plan_tma(dtype, cpr, s.max_region, s.idx_cap, s.any_select, light_traffic, units, unit_bytes, in_place);
+    lp.ws = s.any_select && may_use_ws && !onchip_plan_ok(lp.tp, cpr, light_traffic);
+    if (lp.ws) {
+        lp.w = ws_layout(dtype, s.max_region, s.idx_cap);
+        lp.tp = plan_tma(dtype, cpr, 0, 0, true, light_traffic);
+    }
+    return lp;
+}
+
+// Zeroes the launch descriptor and fills the fields BatchDev and SlabBatchDev share from the launch plan: shape,
+// kept-index capacity, workspace, shared-memory layout.  KVC_ERR_INVALID_ARG when the plan needs more workspace than the
+// caller gave, KVC_ERR_TOO_LARGE when no plan fits.
+template <class Batch>
+static int fill_batch(Batch& bd, const kvc_shape* shape, int cpr, const ChunkStats& s, const LaunchPlan& lp,
+                      void* workspace, int64_t workspace_bytes) {
+    if (lp.ws && lp.w.unit * shape->batch * shape->heads * s.n_active > workspace_bytes) return KVC_ERR_INVALID_ARG;
+    if (!lp.tp.ok) return KVC_ERR_TOO_LARGE;
+    memset(&bd, 0, sizeof(bd));
+    bd.B = shape->batch;
+    bd.H = shape->heads;
+    bd.cpr = cpr;
+    bd.idx_cap = s.idx_cap;
+    if (lp.ws) {
+        bd.ws = (char*)workspace;
+        bd.ws_unit = lp.w.unit;
+        bd.ws_keys = lp.w.keys;
+    }
+    bd.nsw = lp.tp.nsw;
+    bd.off_hist = lp.tp.off_hist;
+    bd.off_idx = lp.tp.off_idx;
+    bd.off_keys = lp.tp.off_keys;
+    bd.off_stage = lp.tp.off_stage;
+    return KVC_OK;
+}
+
+// The fields LayerDev and SlabLayerDev share: the plan and the carry (the descriptor was zeroed: no carry, acc == nullptr).
+template <class Layer>
+static void fill_layer_plan(Layer& d, const kvc_layer_plan& p, const kvc_carry_layer* carry, int e) {
+    d.S = p.seq_len;
+    d.sink = p.sink;
+    d.lo = p.sel_lo;
+    d.hi = p.sel_hi;
+    d.ksel = p.k_sel;
+    d.tail = p.tail;
+    d.score = p.k_sel > 0 ? p.score : KVC_SCORE_NONE;
+    d.pool = p.pool_kernel;
+    if (!carry || !carry->acc) return;
+    d.carry.acc = (char*)carry->acc;
+    d.carry.asb = carry->acc_stride_b * e;
+    d.carry.ash = carry->acc_stride_h * e;
+    d.carry.group = carry->group;
+    d.carry.prev = carry->prev_len < p.seq_len ? carry->prev_len : p.seq_len;
 }
 
 }  // namespace kvc
@@ -550,44 +651,21 @@ int kvc_compress_layers(const kvc_shape* shape, int32_t n_layers, const kvc_laye
     return kvc_compress_layers_ws(shape, n_layers, plans, io, nullptr, 0, stream);
 }
 
-// Launch-chunk statistics shared by kvc_workspace_bytes and the launchers.
-static void chunk_stats(const kvc_layer_plan* plans, int nl, int* n_active, int* max_region, int* max_ksel,
-                        bool* any_select, int64_t* rows_moved = nullptr) {
-    *n_active = *max_region = *max_ksel = 0;
-    *any_select = false;
-    if (rows_moved) *rows_moved = 0;
-    for (int l = 0; l < nl; ++l) {
-        const kvc_layer_plan& p = plans[l];
-        if (p.sink + p.k_sel + p.tail == 0) continue;
-        ++*n_active;
-        // rows one unit of this layer moves if it scans K: the region once + kept rows of K and V read and written
-        if (rows_moved) *rows_moved += (p.k_sel > 0 ? p.sel_hi - p.sel_lo : 0) + 4LL * (p.sink + p.k_sel + p.tail);
-        if (p.k_sel > 0) {
-            *any_select = true;
-            if (p.k_sel > *max_ksel) *max_ksel = p.k_sel;
-            if (p.score != KVC_SCORE_GIVEN_INDEX && p.sel_hi - p.sel_lo > *max_region) *max_region = p.sel_hi - p.sel_lo;
-        }
-    }
-}
-
+// Both planning queries plan like a launch that scans K (light_traffic = false): KVSlabCache sizes the workspace of its
+// in-place compaction with kvc_workspace_bytes as well.
 int64_t kvc_workspace_bytes(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans) {
     int cpr = 0;
     if (check_shape(shape, &cpr) != KVC_OK || n_layers <= 0 || !plans || !row_width_ok(cpr)) return 0;
+    const int64_t bh = (int64_t)shape->batch * shape->heads;
     int64_t need = 0;
-    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
-        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
-        int n_active, max_region, max_ksel;
-        bool any_select;
-        int64_t rows_moved;
-        chunk_stats(plans + l0, nl, &n_active, &max_region, &max_ksel, &any_select, &rows_moved);
-        if (!any_select) continue;
-        const int idx_cap = (max_ksel + 3) & ~3;
-        const TmaPlan tp = plan_tma(shape->dtype, cpr, max_region, idx_cap, true, false,
-                                    (int64_t)shape->batch * shape->heads * n_active, rows_moved / n_active * cpr * 16);
-        if (onchip_plan_ok(tp, cpr, false)) continue;
-        const int64_t bytes = ws_layout(shape->dtype, max_region, idx_cap).unit * shape->batch * shape->heads * n_active;
-        if (bytes > need) need = bytes;
-    }
+    for_each_chunk(n_layers, [&](int l0, int nl) -> int {
+        const ChunkStats s = chunk_stats(plans + l0, nullptr, nl);
+        if (!s.any_select) return KVC_OK;
+        const LaunchPlan lp = plan_launch(shape->dtype, cpr, s, false, false, bh * s.n_active,
+                                          s.rows_moved / s.n_active * cpr * 16, true);
+        if (lp.ws) need = std::max(need, lp.w.unit * bh * s.n_active);
+        return KVC_OK;
+    });
     return need;
 }
 
@@ -597,22 +675,15 @@ int kvc_launch_shape(const kvc_shape* shape, int32_t n_layers, const kvc_layer_p
     if (st != KVC_OK) return st;
     if (n_layers <= 0 || !plans || !out) return KVC_ERR_INVALID_ARG;
     if (!row_width_ok(cpr)) return KVC_ERR_UNSUPPORTED;
-    const int nl = n_layers < KVC_MAX_LAYERS_PER_LAUNCH ? n_layers : KVC_MAX_LAYERS_PER_LAUNCH;
-    int n_active, max_region, max_ksel;
-    bool any_select;
-    int64_t rows_moved;
-    chunk_stats(plans, nl, &n_active, &max_region, &max_ksel, &any_select, &rows_moved);
-    if (n_active == 0) return KVC_ERR_INVALID_ARG;
-    const int idx_cap = (max_ksel + 3) & ~3;
-    TmaPlan tp = plan_tma(shape->dtype, cpr, max_region, idx_cap, any_select, false,
-                          (int64_t)shape->batch * shape->heads * n_active, rows_moved / n_active * cpr * 16);
-    const bool ws = any_select && !onchip_plan_ok(tp, cpr, false);
-    if (ws) tp = plan_tma(shape->dtype, cpr, 0, 0, true, false);
-    if (!tp.ok) return KVC_ERR_TOO_LARGE;
-    out[0] = tp.nt;
-    out[1] = tp.ctas;
-    out[2] = tp.nsw;
-    out[3] = ws ? 1 : 0;
+    const ChunkStats s = chunk_stats(plans, nullptr, std::min(n_layers, KVC_MAX_LAYERS_PER_LAUNCH));
+    if (s.n_active == 0) return KVC_ERR_INVALID_ARG;
+    const int64_t units = (int64_t)shape->batch * shape->heads * s.n_active;
+    const LaunchPlan lp = plan_launch(shape->dtype, cpr, s, false, false, units, s.rows_moved / s.n_active * cpr * 16, true);
+    if (!lp.tp.ok) return KVC_ERR_TOO_LARGE;
+    out[0] = lp.tp.nt;
+    out[1] = lp.tp.ctas;
+    out[2] = lp.tp.nsw;
+    out[3] = lp.ws ? 1 : 0;
     return KVC_OK;
 }
 
@@ -637,20 +708,9 @@ int kvc_compress_layers_carry(const kvc_shape* shape, int32_t n_layers, const kv
     for (int l = 0; l < n_layers; ++l) {
         const kvc_layer_plan& p = plans[l];
         const kvc_layer_io& x = io[l];
+        st = check_plan(p, false, x.idx_in != nullptr, x.score_in != nullptr, carry ? carry + l : nullptr, e);
+        if (st != KVC_OK) return st;
         const int64_t C = (int64_t)p.sink + p.k_sel + p.tail;
-        if (p.seq_len < 0 || p.sink < 0 || p.k_sel < 0 || p.tail < 0) return KVC_ERR_INVALID_ARG;
-        if (p.sink > p.seq_len || p.tail > p.seq_len) return KVC_ERR_INVALID_ARG;
-        if (p.k_sel > 0) {
-            if (p.sel_lo < 0 || p.sel_hi > p.seq_len || p.sel_lo > p.sel_hi) return KVC_ERR_INVALID_ARG;
-            if (p.k_sel > p.sel_hi - p.sel_lo) return KVC_ERR_INVALID_ARG;
-            if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE_SHARED) return KVC_ERR_INVALID_ARG;
-            const bool given_score = p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_GIVEN_SCORE_SHARED;
-            if (p.score == KVC_SCORE_GIVEN_INDEX && !x.idx_in) return KVC_ERR_INVALID_ARG;
-            if (given_score && !x.score_in) return KVC_ERR_INVALID_ARG;
-            if ((given_score || p.score == KVC_SCORE_SNAPKV_POOL) && p.pool_kernel > 2 * kMaxPoolHalo)
-                return KVC_ERR_UNSUPPORTED;
-        }
-        if (!carry_ok(carry, l, p, e)) return KVC_ERR_INVALID_ARG;
         if (C == 0) continue;
         if (!x.k_in || !x.v_in || !x.k_out || !x.v_out) return KVC_ERR_INVALID_ARG;
         if (C * cpr * 2 > 0x7fffffffLL) return KVC_ERR_TOO_LARGE;
@@ -663,22 +723,24 @@ int kvc_compress_layers_carry(const kvc_shape* shape, int32_t n_layers, const kv
     NvtxRange nvtx_range("kvc_compress_layers_ws");
     if (guard.status != KVC_OK) return guard.status;
 
-    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
-        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+    return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
+        const ChunkStats s = chunk_stats(plans + l0, io + l0, nl);
+        if (s.n_active == 0) return KVC_OK;
+        // no K scan in this launch (stored norms, caller-supplied scores or rows, pure slices with a select next to
+        // them): only kept rows move -> residency over slot depth
+        const bool light = s.any_select && !s.any_scan;
+        const LaunchPlan lp = plan_launch(dt, cpr, s, light, false, (int64_t)B * H * s.n_active,
+                                          s.rows_moved / s.n_active * cpr * 16, workspace != nullptr);
         BatchDev bd;
-        memset(&bd, 0, sizeof(bd));
-        bd.B = B;
-        bd.H = H;
-        bd.cpr = cpr;
-        int n_active = 0, max_region = 0, max_ksel = 0;
-        int64_t rows_moved = 0;
-        bool any_select = false, any_scan = false;
-        for (int l = 0; l < nl; ++l) {
-            const kvc_layer_plan& p = plans[l0 + l];
-            const kvc_layer_io& x = io[l0 + l];
+        int st = fill_batch(bd, shape, cpr, s, lp, workspace, workspace_bytes);
+        if (st != KVC_OK) return st;
+        bd.upc = lp.tp.upc;
+        int m = 0;
+        for (int l = l0; l < l0 + nl; ++l) {
+            const kvc_layer_plan& p = plans[l];
+            const kvc_layer_io& x = io[l];
             if (p.sink + p.k_sel + p.tail == 0) continue;
-            rows_moved += (p.k_sel > 0 ? p.sel_hi - p.sel_lo : 0) + 4LL * (p.sink + p.k_sel + p.tail);
-            LayerDev& d = bd.layers[n_active++];
+            LayerDev& d = bd.layers[m++];
             d.k_in = (const char*)x.k_in;
             d.v_in = (const char*)x.v_in;
             d.k_out = (char*)x.k_out;
@@ -692,63 +754,20 @@ int kvc_compress_layers_carry(const kvc_shape* shape, int32_t n_layers, const kv
             d.vsb = x.v_stride_b * e;
             d.vsh = x.v_stride_h * e;
             d.vss = x.v_stride_s * e;
-            d.S = p.seq_len;
-            d.sink = p.sink;
-            d.lo = p.sel_lo;
-            d.hi = p.sel_hi;
-            d.ksel = p.k_sel;
-            d.tail = p.tail;
-            d.score = p.k_sel > 0 ? p.score : KVC_SCORE_NONE;
-            d.pool = p.pool_kernel;
-            const bool ranked = p.k_sel > 0 && (p.score == KVC_SCORE_L2_LOW || p.score == KVC_SCORE_L2_HIGH ||
-                                                p.score == KVC_SCORE_SNAPKV_POOL);
-            if (ranked && x.norms_in) {  // the caller holds the key norms: the scan is skipped
+            if (ranked(p) && x.norms_in) {  // the caller holds the key norms: the scan is skipped
                 d.n_in = (const char*)x.norms_in;
                 d.nsb = x.n_stride_b * key_bytes(dt);
                 d.nsh = x.n_stride_h * key_bytes(dt);
             }
-            fill_carry(d.carry, carry, l0 + l, p, e);
-            if (p.k_sel > 0) {
-                any_select = true;
-                any_scan |= ranked && !x.norms_in;
-                if (p.k_sel > max_ksel) max_ksel = p.k_sel;
-                if (p.score != KVC_SCORE_GIVEN_INDEX && p.sel_hi - p.sel_lo > max_region)
-                    max_region = p.sel_hi - p.sel_lo;
-            }
+            fill_layer_plan(d, p, carry ? carry + l : nullptr, e);
         }
-        if (n_active == 0) continue;
-        bd.idx_cap = (max_ksel + 3) & ~3;
-        // no K scan in this launch (stored norms, caller-supplied scores or rows, pure slices with a select next to
-        // them): only kept rows move -> residency over slot depth
-        const bool light = any_select && !any_scan;
-        TmaPlan tp = plan_tma(dt, cpr, max_region, bd.idx_cap, any_select, light, (int64_t)B * H * n_active,
-                              rows_moved / n_active * cpr * 16);
-        if (any_select && workspace != nullptr && !onchip_plan_ok(tp, cpr, light)) {
-            // keys and kept indices go to the workspace; shared memory keeps the histogram and the slots
-            const WsLayout w = ws_layout(dt, max_region, bd.idx_cap);
-            if (w.unit * B * H * n_active > workspace_bytes) return KVC_ERR_INVALID_ARG;
-            bd.ws = (char*)workspace;
-            bd.ws_unit = w.unit;
-            bd.ws_keys = w.keys;
-            tp = plan_tma(dt, cpr, 0, 0, true, light);
-        }
-        if (!tp.ok) return KVC_ERR_TOO_LARGE;
-        FusedFn fn = pick_tma(dt, cpr, tp.nt);
-        bd.nsw = tp.nsw;
-        bd.off_hist = tp.off_hist;
-        bd.off_idx = tp.off_idx;
-        bd.off_keys = tp.off_keys;
-        bd.off_stage = tp.off_stage;
-        bd.upc = tp.upc;
-        dim3 grid((unsigned)(((int64_t)B * H + tp.upc - 1) / tp.upc), (unsigned)n_active, 1);
+        FusedFn fn = pick_tma(dt, cpr, lp.tp.nt);
+        dim3 grid((unsigned)(((int64_t)B * H + lp.tp.upc - 1) / lp.tp.upc), (unsigned)s.n_active, 1);
         st = ensure_tma_attrs((const void*)fn, shape->device);
         if (st != KVC_OK) return st;
-        fn<<<grid, tp.nt, tp.smem, (cudaStream_t)stream>>>(bd);
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_fused_tma_kernel launch");
-        g_launches.fetch_add(1);
-    }
-    return KVC_OK;
+        fn<<<grid, lp.tp.nt, lp.tp.smem, (cudaStream_t)stream>>>(bd);
+        return launched("kvc_fused_tma_kernel launch");
+    });
 }
 
 int kvc_key_norms(const kvc_shape* shape, const void* k_in, int64_t stride_b, int64_t stride_h, int64_t stride_s,
@@ -775,24 +794,11 @@ int kvc_key_norms(const kvc_shape* shape, const void* k_in, int64_t stride_b, in
     if (blocks > cap) blocks = cap;
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t sb = stride_b * e, sh = stride_h * e, ss = stride_s * e;
-    switch (dt) {
-        case KVC_DTYPE_F32:
-            kvc_norm_kernel<KVC_DTYPE_F32><<<(unsigned)blocks, 256, 0, s>>>((const char*)k_in, sb, sh, ss, H, row_lo, R,
-                                                                           total, lpr, cpl, (uint32_t*)norms_out);
-            break;
-        case KVC_DTYPE_F16:
-            kvc_norm_kernel<KVC_DTYPE_F16><<<(unsigned)blocks, 256, 0, s>>>((const char*)k_in, sb, sh, ss, H, row_lo, R,
-                                                                           total, lpr, cpl, (uint16_t*)norms_out);
-            break;
-        default:
-            kvc_norm_kernel<KVC_DTYPE_BF16><<<(unsigned)blocks, 256, 0, s>>>((const char*)k_in, sb, sh, ss, H, row_lo,
-                                                                            R, total, lpr, cpl, (uint16_t*)norms_out);
-            break;
-    }
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return cuda_fail(err, "kvc_norm_kernel launch");
-    g_launches.fetch_add(1);
-    return KVC_OK;
+    by_dtype(dt, [&](auto d) {
+        kvc_norm_kernel<d><<<(unsigned)blocks, 256, 0, s>>>((const char*)k_in, sb, sh, ss, H, row_lo, R, total, lpr, cpl,
+                                                            (typename Traits<d>::Key*)norms_out);
+    });
+    return launched("kvc_norm_kernel launch");
 }
 
 int kvc_select(int32_t dtype, int32_t device, const void* scores, int64_t n_rows, int32_t n, int32_t k,
@@ -806,34 +812,13 @@ int kvc_select(int32_t dtype, int32_t device, const void* scores, int64_t n_rows
     DeviceGuard guard(device);
     NvtxRange nvtx_range("kvc_select");
     if (guard.status != KVC_OK) return guard.status;
-    int st = KVC_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    const void* fn = nullptr;
-    switch (dtype) {
-        case KVC_DTYPE_F32: fn = (const void*)kvc_select_kernel<KVC_DTYPE_F32, kNT>; break;
-        case KVC_DTYPE_F16: fn = (const void*)kvc_select_kernel<KVC_DTYPE_F16, kNT>; break;
-        default: fn = (const void*)kvc_select_kernel<KVC_DTYPE_BF16, kNT>; break;
-    }
-    st = ensure_smem(fn, smem);
-    if (st != KVC_OK) return st;
-    switch (dtype) {
-        case KVC_DTYPE_F32:
-            kvc_select_kernel<KVC_DTYPE_F32, kNT>
-                <<<(unsigned)n_rows, kNT, smem, s>>>((const uint32_t*)scores, n, k, largest, idx_out);
-            break;
-        case KVC_DTYPE_F16:
-            kvc_select_kernel<KVC_DTYPE_F16, kNT>
-                <<<(unsigned)n_rows, kNT, smem, s>>>((const uint16_t*)scores, n, k, largest, idx_out);
-            break;
-        default:
-            kvc_select_kernel<KVC_DTYPE_BF16, kNT>
-                <<<(unsigned)n_rows, kNT, smem, s>>>((const uint16_t*)scores, n, k, largest, idx_out);
-            break;
-    }
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return cuda_fail(err, "kvc_select_kernel launch");
-    g_launches.fetch_add(1);
-    return KVC_OK;
+    return by_dtype(dtype, [&](auto d) -> int {
+        const int st = ensure_smem((const void*)kvc_select_kernel<d, kNT>, smem);
+        if (st != KVC_OK) return st;
+        kvc_select_kernel<d, kNT><<<(unsigned)n_rows, kNT, smem, (cudaStream_t)stream>>>(
+            (const typename Traits<d>::Key*)scores, n, k, largest, idx_out);
+        return launched("kvc_select_kernel launch");
+    });
 }
 
 #endif  // KVC_HAS_CORE
@@ -896,14 +881,10 @@ int kvc_slab_append(const kvc_shape* shape, int32_t n_layers, const kvc_slab_lay
         fill(one.layers[0], slabs[0], rows[0]);
         const int64_t threads = (int64_t)B * H * rows[0].n_new;
         pick_append_one(dt, cpr)<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(one);
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_slab_append_kernel launch");
-        g_launches.fetch_add(1);
-        return KVC_OK;
+        return launched("kvc_slab_append_kernel launch");
     }
     AppendFn fn = pick_append(dt, cpr);
-    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
-        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+    return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
         AppendBatchDev bd;
         memset(&bd, 0, sizeof(bd));
         bd.B = B;
@@ -916,14 +897,13 @@ int kvc_slab_append(const kvc_shape* shape, int32_t n_layers, const kvc_slab_lay
             fill(bd.layers[n_active++], sl, r);
             if (r.n_new > max_new) max_new = r.n_new;
         }
-        if (n_active == 0) continue;
+        if (n_active == 0) return KVC_OK;
         bd.max_new = max_new;
         bd.cpr = cpr;
-        cudaError_t err;
         if (max_new >= 32) {
             // prefill / chunked prefill: rows move 32 at a time through shared memory with bulk copies
             AppendFn tfn = pick_append_tma(dt, cpr);
-            st = ensure_tma_attrs((const void*)tfn, shape->device);
+            const int st = ensure_tma_attrs((const void*)tfn, shape->device);
             if (st != KVC_OK) return st;
             const size_t smem = 128 + (size_t)8 * 32 * cpr * 16;
             const int64_t items = (int64_t)B * H * ((max_new + 31) / 32);
@@ -932,17 +912,13 @@ int kvc_slab_append(const kvc_shape* shape, int32_t n_layers, const kvc_slab_lay
             if (blocks > cap) blocks = cap;
             dim3 grid((unsigned)blocks, (unsigned)n_active, 1);
             tfn<<<grid, 256, smem, (cudaStream_t)stream>>>(bd);
-            err = cudaGetLastError();
         } else {
             const int64_t threads = (int64_t)B * H * max_new;
             dim3 grid((unsigned)((threads + 127) / 128), (unsigned)n_active, 1);
             fn<<<grid, 128, 0, (cudaStream_t)stream>>>(bd);
-            err = cudaGetLastError();
         }
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_slab_append_kernel launch");
-        g_launches.fetch_add(1);
-    }
-    return KVC_OK;
+        return launched("kvc_slab_append_kernel launch");
+    });
 }
 
 int kvc_slab_compress(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
@@ -966,20 +942,9 @@ int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_
     for (int l = 0; l < n_layers; ++l) {
         const kvc_layer_plan& p = plans[l];
         const kvc_slab_layer& sl = slabs[l];
-        if (p.seq_len < 0 || p.sink < 0 || p.k_sel < 0 || p.tail < 0) return KVC_ERR_INVALID_ARG;
-        if (p.sink > p.seq_len || p.tail > p.seq_len) return KVC_ERR_INVALID_ARG;
-        if ((int64_t)p.sink + p.k_sel + p.tail > p.seq_len) return KVC_ERR_INVALID_ARG;
-        if (p.k_sel > 0) {
-            if (p.sel_lo < p.sink || p.sel_hi > p.seq_len - p.tail || p.sel_lo > p.sel_hi) return KVC_ERR_INVALID_ARG;
-            if (p.k_sel > p.sel_hi - p.sel_lo) return KVC_ERR_INVALID_ARG;
-            if (p.score <= KVC_SCORE_NONE || p.score > KVC_SCORE_GIVEN_SCORE_SHARED) return KVC_ERR_INVALID_ARG;
-            const bool given_score = p.score == KVC_SCORE_GIVEN_SCORE || p.score == KVC_SCORE_GIVEN_SCORE_SHARED;
-            if ((p.score == KVC_SCORE_GIVEN_INDEX || given_score) && (!idx_in || !idx_in[l]))
-                return KVC_ERR_INVALID_ARG;
-            if ((p.score == KVC_SCORE_SNAPKV_POOL || given_score) && p.pool_kernel > 2 * kMaxPoolHalo)
-                return KVC_ERR_UNSUPPORTED;
-        }
-        if (!carry_ok(carry, l, p, e)) return KVC_ERR_INVALID_ARG;
+        const bool given = idx_in && idx_in[l];  // kept rows or scores travel in the idx_in slot
+        st = check_plan(p, true, given, given, carry ? carry + l : nullptr, e);
+        if (st != KVC_OK) return st;
         if (p.sink + p.k_sel + p.tail == 0) continue;
         if (!sl.k || !sl.v || !sl.norms) return KVC_ERR_INVALID_ARG;
         if (((uintptr_t)sl.k | (uintptr_t)sl.v) & 15) return KVC_ERR_UNSUPPORTED;
@@ -988,73 +953,39 @@ int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_
     DeviceGuard guard(shape->device);
     NvtxRange nvtx_range("kvc_slab_compress");
     if (guard.status != KVC_OK) return guard.status;
-    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
-        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+    return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
+        const ChunkStats s = chunk_stats(plans + l0, nullptr, nl);
+        if (s.n_active == 0) return KVC_OK;
+        const LaunchPlan lp = plan_launch(dt, cpr, s, /*light_traffic=*/true, /*in_place=*/true, 0, 0, workspace != nullptr);
         SlabBatchDev bd;
-        memset(&bd, 0, sizeof(bd));
-        bd.B = B;
-        bd.H = H;
-        bd.cpr = cpr;
-        int n_active = 0, max_region = 0, max_ksel = 0;
-        bool any_select = false;
-        for (int l = 0; l < nl; ++l) {
-            const kvc_layer_plan& p = plans[l0 + l];
-            const kvc_slab_layer& sl = slabs[l0 + l];
+        int st = fill_batch(bd, shape, cpr, s, lp, workspace, workspace_bytes);
+        if (st != KVC_OK) return st;
+        int m = 0;
+        for (int l = l0; l < l0 + nl; ++l) {
+            const kvc_layer_plan& p = plans[l];
+            const kvc_slab_layer& sl = slabs[l];
             if (p.sink + p.k_sel + p.tail == 0) continue;
-            SlabLayerDev& d = bd.layers[n_active++];
+            SlabLayerDev& d = bd.layers[m++];
             d.k = (char*)sl.k;
             d.v = (char*)sl.v;
             d.n = (char*)sl.norms;
-            d.idx_out = idx_out ? idx_out[l0 + l] : nullptr;
-            d.idx_in = idx_in ? idx_in[l0 + l] : nullptr;
+            d.idx_out = idx_out ? idx_out[l] : nullptr;
+            d.idx_in = idx_in ? idx_in[l] : nullptr;
             d.ksb = sl.k_stride_b * e;
             d.ksh = sl.k_stride_h * e;
             d.vsb = sl.v_stride_b * e;
             d.vsh = sl.v_stride_h * e;
             d.nsb = sl.n_stride_b * key_bytes(dt);
             d.nsh = sl.n_stride_h * key_bytes(dt);
-            d.S = p.seq_len;
-            d.sink = p.sink;
-            d.lo = p.sel_lo;
-            d.hi = p.sel_hi;
-            d.ksel = p.k_sel;
-            d.tail = p.tail;
-            d.score = p.k_sel > 0 ? p.score : KVC_SCORE_NONE;
-            d.pool = p.pool_kernel;
-            fill_carry(d.carry, carry, l0 + l, p, e);
-            if (p.k_sel > 0) {
-                any_select = true;
-                if (p.k_sel > max_ksel) max_ksel = p.k_sel;
-                if (p.score != KVC_SCORE_GIVEN_INDEX && p.sel_hi - p.sel_lo > max_region) max_region = p.sel_hi - p.sel_lo;
-            }
+            fill_layer_plan(d, p, carry ? carry + l : nullptr, e);
         }
-        if (n_active == 0) continue;
-        bd.idx_cap = (max_ksel + 3) & ~3;
-        TmaPlan tp = plan_tma(dt, cpr, max_region, bd.idx_cap, any_select, /*light_traffic=*/true, 0, 0, /*in_place=*/true);
-        if (any_select && workspace != nullptr && !onchip_plan_ok(tp, cpr, true)) {
-            const WsLayout w = ws_layout(dt, max_region, bd.idx_cap);
-            if (w.unit * B * H * n_active > workspace_bytes) return KVC_ERR_INVALID_ARG;
-            bd.ws = (char*)workspace;
-            bd.ws_unit = w.unit;
-            bd.ws_keys = w.keys;
-            tp = plan_tma(dt, cpr, 0, 0, true, /*light_traffic=*/true);
-        }
-        if (!tp.ok) return KVC_ERR_TOO_LARGE;
-        SlabFn fn = pick_slab(dt, cpr, tp.nt);
-        bd.nsw = tp.nsw;
-        bd.off_hist = tp.off_hist;
-        bd.off_idx = tp.off_idx;
-        bd.off_keys = tp.off_keys;
-        bd.off_stage = tp.off_stage;
+        SlabFn fn = pick_slab(dt, cpr, lp.tp.nt);
         st = ensure_tma_attrs((const void*)fn, shape->device);
         if (st != KVC_OK) return st;
-        dim3 grid((unsigned)((int64_t)B * H), (unsigned)n_active, 1);
-        fn<<<grid, tp.nt, tp.smem, (cudaStream_t)stream>>>(bd);
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_slab_compress_kernel launch");
-        g_launches.fetch_add(1);
-    }
-    return KVC_OK;
+        dim3 grid((unsigned)((int64_t)B * H), (unsigned)s.n_active, 1);
+        fn<<<grid, lp.tp.nt, lp.tp.smem, (cudaStream_t)stream>>>(bd);
+        return launched("kvc_slab_compress_kernel launch");
+    });
 }
 
 #endif  // KVC_HAS_SLAB
@@ -1169,29 +1100,43 @@ static int launch_vote_tma(const kvc_shape* shape, int32_t n_layers, const kvc_v
         }
         dim3 grid((unsigned)((int64_t)B * H), (unsigned)nl, 1);
         fn<<<grid, 576, smem, (cudaStream_t)stream>>>(bd);
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_snapkv_vote_tma_kernel launch");
-        g_launches.fetch_add(1);
+        st = launched("kvc_snapkv_vote_tma_kernel launch");
+        if (st != KVC_OK) return st;
     }
+    return KVC_OK;
+}
+
+// The call-wide checks both vote entry points make (the fused form's plans / io present: `more_ok`); KVC_OK with
+// n_layers == 0 means there is nothing to do.
+static int check_vote_call(const kvc_shape* shape, int32_t n_layers, const kvc_vote_layer* layers, bool more_ok,
+                           int32_t group, int32_t window, int* cpr) {
+    const int st = check_shape(shape, cpr);
+    if (st != KVC_OK) return st;
+    if (n_layers < 0 || (n_layers > 0 && (!layers || !more_ok)) || group <= 0 || window <= 0) return KVC_ERR_INVALID_ARG;
+    if (n_layers == 0) return KVC_OK;
+    if (shape->dtype == KVC_DTYPE_F32) return KVC_ERR_UNSUPPORTED;
+    if (*cpr != 8 && *cpr != 10 && *cpr != 16) return KVC_ERR_UNSUPPORTED;
+    if ((int64_t)group * window > kVoteM) return KVC_ERR_UNSUPPORTED;
+    return KVC_OK;
+}
+
+// The checks of one kvc_vote_layer both vote entry points make.
+static int check_vote_layer(const kvc_vote_layer& v, int32_t window) {
+    if (!v.k_in || !v.q_obs || !v.votes_out || v.seq_len <= window) return KVC_ERR_INVALID_ARG;
+    if (((uintptr_t)v.k_in | (uintptr_t)v.q_obs) & 15) return KVC_ERR_UNSUPPORTED;
+    const int64_t sb = v.k_stride_b | v.k_stride_h | v.k_stride_s | v.q_stride_b | v.q_stride_h | v.q_stride_s;
+    if ((sb * 2) & 15) return KVC_ERR_UNSUPPORTED;
     return KVC_OK;
 }
 
 int kvc_snapkv_vote(const kvc_shape* shape, int32_t n_layers, const kvc_vote_layer* layers, int32_t group,
                     int32_t window, void* stream) {
     int cpr = 0;
-    int st = check_shape(shape, &cpr);
-    if (st != KVC_OK) return st;
-    if (n_layers < 0 || (n_layers > 0 && !layers) || group <= 0 || window <= 0) return KVC_ERR_INVALID_ARG;
-    if (n_layers == 0) return KVC_OK;
-    if (shape->dtype == KVC_DTYPE_F32) return KVC_ERR_UNSUPPORTED;
-    if (cpr != 8 && cpr != 10 && cpr != 16) return KVC_ERR_UNSUPPORTED;
-    if ((int64_t)group * window > kVoteM) return KVC_ERR_UNSUPPORTED;
+    int st = check_vote_call(shape, n_layers, layers, true, group, window, &cpr);
+    if (st != KVC_OK || n_layers == 0) return st;
     for (int l = 0; l < n_layers; ++l) {
-        const kvc_vote_layer& v = layers[l];
-        if (!v.k_in || !v.q_obs || !v.votes_out || v.seq_len <= window) return KVC_ERR_INVALID_ARG;
-        if (((uintptr_t)v.k_in | (uintptr_t)v.q_obs) & 15) return KVC_ERR_UNSUPPORTED;
-        const int64_t sb = v.k_stride_b | v.k_stride_h | v.k_stride_s | v.q_stride_b | v.q_stride_h | v.q_stride_s;
-        if ((sb * 2) & 15) return KVC_ERR_UNSUPPORTED;
+        st = check_vote_layer(layers[l], window);
+        if (st != KVC_OK) return st;
     }
     DeviceGuard guard(shape->device);
     NvtxRange nvtx_range("kvc_snapkv_vote");
@@ -1205,23 +1150,15 @@ int kvc_snapkv_vote_compress(const kvc_shape* shape, int32_t n_layers, const kvc
                              const kvc_layer_plan* plans, const kvc_layer_io* io, int32_t group, int32_t window,
                              void* stream) {
     int cpr = 0;
-    int st = check_shape(shape, &cpr);
-    if (st != KVC_OK) return st;
-    if (n_layers < 0 || (n_layers > 0 && (!layers || !plans || !io)) || group <= 0 || window <= 0)
-        return KVC_ERR_INVALID_ARG;
-    if (n_layers == 0) return KVC_OK;
-    if (shape->dtype == KVC_DTYPE_F32) return KVC_ERR_UNSUPPORTED;
-    if (cpr != 8 && cpr != 10 && cpr != 16) return KVC_ERR_UNSUPPORTED;
-    if ((int64_t)group * window > kVoteM) return KVC_ERR_UNSUPPORTED;
+    int st = check_vote_call(shape, n_layers, layers, plans && io, group, window, &cpr);
+    if (st != KVC_OK || n_layers == 0) return st;
     const size_t ring_bytes = (size_t)vote_tma_ring(cpr) * ((size_t)(cpr / 8) * kVoteTile * 128 + (size_t)(cpr % 8) * kVoteTile * 16);
     for (int l = 0; l < n_layers; ++l) {
         const kvc_vote_layer& v = layers[l];
         const kvc_layer_plan& p = plans[l];
         const kvc_layer_io& x = io[l];
-        if (!v.k_in || !v.q_obs || !v.votes_out || v.seq_len <= window) return KVC_ERR_INVALID_ARG;
-        if (((uintptr_t)v.k_in | (uintptr_t)v.q_obs) & 15) return KVC_ERR_UNSUPPORTED;
-        const int64_t sb = v.k_stride_b | v.k_stride_h | v.k_stride_s | v.q_stride_b | v.q_stride_h | v.q_stride_s;
-        if ((sb * 2) & 15) return KVC_ERR_UNSUPPORTED;
+        st = check_vote_layer(v, window);
+        if (st != KVC_OK) return st;
         // the plan of snapkv_lite in vote mode: no sinks, the prefix [0, S - W) ranked by pooled votes, the window kept
         if (p.seq_len != v.seq_len || p.sink != 0 || p.sel_lo != 0 || p.sel_hi != v.seq_len - window || p.k_sel <= 0 ||
             p.k_sel > p.sel_hi || p.tail < 0 || p.tail > window || p.score != KVC_SCORE_GIVEN_SCORE)
@@ -1263,8 +1200,7 @@ int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_l
     NvtxRange nvtx_range("kvc_h2o_accumulate");
     if (guard.status != KVC_OK) return guard.status;
     const int tc = 32 * (16 / e);  // key columns per CTA
-    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
-        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+    return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
         H2oBatchDev bd;
         memset(&bd, 0, sizeof(bd));
         bd.B = B;
@@ -1292,18 +1228,11 @@ int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_l
             const int tiles = (x.key_len + tc - 1) / tc;
             if (tiles > max_tiles) max_tiles = tiles;
         }
-        if (n_active == 0) continue;
+        if (n_active == 0) return KVC_OK;
         dim3 grid((unsigned)max_tiles, (unsigned)B, (unsigned)n_active);
-        switch (dt) {
-            case KVC_DTYPE_F32: kvc_h2o_accumulate_kernel<KVC_DTYPE_F32><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); break;
-            case KVC_DTYPE_F16: kvc_h2o_accumulate_kernel<KVC_DTYPE_F16><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); break;
-            default: kvc_h2o_accumulate_kernel<KVC_DTYPE_BF16><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); break;
-        }
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_h2o_accumulate_kernel launch");
-        g_launches.fetch_add(1);
-    }
-    return KVC_OK;
+        by_dtype(dt, [&](auto d) { kvc_h2o_accumulate_kernel<d><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); });
+        return launched("kvc_h2o_accumulate_kernel launch");
+    });
 }
 
 // ------------------------------------------------------------------ kvc_h2o_accumulate_qk
@@ -1378,8 +1307,7 @@ int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layer
     const int e = elem_bytes(dt);
     const int rb = D * e, pitch = ((rb / 16) | 1) * 16;
     char* ws = (char*)workspace;
-    for (int l0 = 0; l0 < n_layers; l0 += KVC_MAX_LAYERS_PER_LAUNCH) {
-        const int nl = (n_layers - l0) < KVC_MAX_LAYERS_PER_LAUNCH ? (n_layers - l0) : KVC_MAX_LAYERS_PER_LAUNCH;
+    return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
         H2oQkBatchDev bd;
         memset(&bd, 0, sizeof(bd));
         bd.B = B;
@@ -1424,15 +1352,14 @@ int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layer
             if (tiles > max_tiles) max_tiles = tiles;
             if (gt > max_gt) max_gt = gt;
         }
-        if (n_active == 0) continue;
+        if (n_active == 0) return KVC_OK;
         // queries per register tile: the work of a (query, key) pair does not depend on it, only the speed does
         const int qt = max_gt >= 8 ? 8 : max_gt >= 4 ? 4 : 1;
         QkFn stats, accum;
-        switch (dt) {
-            case KVC_DTYPE_F32: stats = pick_qk<KVC_DTYPE_F32>(true, qt); accum = pick_qk<KVC_DTYPE_F32>(false, qt); break;
-            case KVC_DTYPE_F16: stats = pick_qk<KVC_DTYPE_F16>(true, qt); accum = pick_qk<KVC_DTYPE_F16>(false, qt); break;
-            default: stats = pick_qk<KVC_DTYPE_BF16>(true, qt); accum = pick_qk<KVC_DTYPE_BF16>(false, qt); break;
-        }
+        by_dtype(dt, [&](auto d) {
+            stats = pick_qk<d>(true, qt);
+            accum = pick_qk<d>(false, qt);
+        });
         const size_t smem_k = 128 + 2 * (size_t)kQkRows * pitch;
         const size_t smem1 = smem_k + (size_t)kQkQ1 * D * 4 + 2 * (size_t)kQkQ1 * kQkThreads * 4;
         const size_t smem2 = smem_k + (size_t)kQkQ2 * D * 4 + (size_t)kQkQ2 * 4;
@@ -1442,15 +1369,11 @@ int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layer
         if (st != KVC_OK) return st;
         stats<<<dim3((unsigned)max_x1, (unsigned)(B * Hkv), (unsigned)n_active), kQkThreads, smem1,
                  (cudaStream_t)stream>>>(bd);
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_h2o_qk_stats_kernel launch");
-        g_launches.fetch_add(1);
+        st = launched("kvc_h2o_qk_stats_kernel launch");
+        if (st != KVC_OK) return st;
         accum<<<dim3((unsigned)max_tiles, (unsigned)B, (unsigned)n_active), kQkThreads, smem2, (cudaStream_t)stream>>>(bd);
-        err = cudaGetLastError();
-        if (err != cudaSuccess) return cuda_fail(err, "kvc_h2o_qk_accumulate_kernel launch");
-        g_launches.fetch_add(1);
-    }
-    return KVC_OK;
+        return launched("kvc_h2o_qk_accumulate_kernel launch");
+    });
 }
 #endif  // KVC_HAS_H2O
 

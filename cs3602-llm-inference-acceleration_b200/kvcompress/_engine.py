@@ -421,12 +421,10 @@ def run_plans(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans, given_indi
             ws = torch.empty((need[1],), dtype=torch.uint8, device=run_device)
             keepalive.append(ws)
             ws_ptr, ws_bytes = ctypes.c_void_p(ws.data_ptr()), need[1]
-        if carry_buf is not None:
-            status = lib.kvc_compress_layers_carry(shape_rec, n, plan_bytes, bytes(io_buf), bytes(carry_buf), ws_ptr,
-                                                   ws_bytes, ctypes.c_void_p(_stream_ptr(run_device)))
-        else:
-            status = lib.kvc_compress_layers_ws(shape_rec, n, plan_bytes, bytes(io_buf), ws_ptr, ws_bytes,
-                                                ctypes.c_void_p(_stream_ptr(run_device)))
+        # a NULL carry is exactly kvc_compress_layers_ws (kvc.h)
+        status = lib.kvc_compress_layers_carry(shape_rec, n, plan_bytes, bytes(io_buf),
+                                               None if carry_buf is None else bytes(carry_buf), ws_ptr, ws_bytes,
+                                               ctypes.c_void_p(_stream_ptr(run_device)))
         _check(status, "kvc_compress_layers")
         if on_host and (host_temps or not (non_blocking or to_device)):
             # host tensors are read by the caller with plain loads: finish before returning, as the reference's

@@ -523,15 +523,13 @@ class KVSlabCache:
             if self._ws is None or self._ws.numel() < ws_need:
                 self._ws = torch.empty((ws_need,), dtype=torch.uint8, device=self.device)
             ws_ptr = ctypes.c_void_p(self._ws.data_ptr())
+        carry_buf = None  # a NULL carry is exactly kvc_slab_compress (kvc.h)
         if carry:
             carry_buf = b"".join(_engine.carry_record(i, carry[i], self.batch, self.heads, self.dtype, n)
                                  if carry.get(i) is not None else bytes(_engine._CARRY.size)
                                  for i, n in zip(ids, in_lens))
-            status = lib.kvc_slab_compress_carry(self._shape, len(ids), plan_buf, slab_buf, idx_out, idx_in, carry_buf,
-                                                 ws_ptr, ws_need, ctypes.c_void_p(_engine._stream_ptr(self.device)))
-        else:
-            status = lib.kvc_slab_compress(self._shape, len(ids), plan_buf, slab_buf, idx_out, idx_in, ws_ptr, ws_need,
-                                           ctypes.c_void_p(_engine._stream_ptr(self.device)))
+        status = lib.kvc_slab_compress_carry(self._shape, len(ids), plan_buf, slab_buf, idx_out, idx_in, carry_buf,
+                                             ws_ptr, ws_need, ctypes.c_void_p(_engine._stream_ptr(self.device)))
         _engine._check(status, "kvc_slab_compress")
         for i, c in zip(ids, out_lens):
             self.lengths[i] = c
