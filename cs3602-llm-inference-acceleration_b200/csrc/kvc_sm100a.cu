@@ -25,6 +25,7 @@
 #include "kvc_device.cuh"
 #include "kvc_fused_tma.cuh"
 #include "kvc_h2o.cuh"
+#include "kvc_h2o_tc.cuh"
 #include "kvc_slab.cuh"
 #include "kvc_vote.cuh"
 
@@ -32,7 +33,8 @@
 // times in parallel, each pass keeping one group of entry points (and only the kernels they launch), and links the
 // objects.  KVC_PART is a bit mask: 1 = compress / select / norms entry points (+ the library-wide state) and the
 // bf16 fused kernels, 2 = slab entry points and the bf16 in-place kernels, 4 = vote, 8 = slab append kernels,
-// 16 = f16/f32 fused kernels, 32 = f16/f32 in-place kernels, 64 = H2O score accumulation.
+// 16 = f16/f32 fused kernels, 32 = f16/f32 in-place kernels, 64 = H2O score accumulation (CUDA-core and tensor-core
+// forms).
 #ifndef KVC_PART
 #define KVC_PART 127
 #endif
@@ -991,22 +993,6 @@ int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_
 #endif  // KVC_HAS_SLAB
 
 #if KVC_HAS_VOTE
-// cuTensorMapEncodeTiled through the runtime (the library links cudart statically and never links libcuda).
-using EncodeTiledFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn tensor_map_encoder() {
-    static EncodeTiledFn fn = [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-            q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return (EncodeTiledFn)p;
-    }();
-    return fn;
-}
-
 // Shared-memory bytes the fused tail needs inside the (dead) key-tile ring: histogram, kept indices, radix keys
 // of the prefix, at least one staging slot of 32 rows.
 static size_t vote_tail_bytes(int cpr, int prefix_rows, int idx_cap) {
@@ -1056,21 +1042,9 @@ static int launch_vote_tma(const kvc_shape* shape, int32_t n_layers, const kvc_v
             const cuuint64_t dims[4] = {(cuuint64_t)D, (cuuint64_t)v.seq_len, (cuuint64_t)H, (cuuint64_t)B};
             const cuuint64_t strides[3] = {(cuuint64_t)v.k_stride_s * 2, (cuuint64_t)v.k_stride_h * 2,
                                            (cuuint64_t)v.k_stride_b * 2};
-            const cuuint32_t box[4] = {64, (cuuint32_t)kVoteTile, 1, 1};
-            const cuuint32_t estr[4] = {1, 1, 1, 1};
-            const CUresult r = encode(&d.map, dt == KVC_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16,
-                                      4, const_cast<void*>(v.k_in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) return KVC_ERR_UNSUPPORTED;
-            if (cpr % 8) {  // D = 80: the last 16 elements of every row through a 32-byte-swizzled box
-                const cuuint32_t box_tail[4] = {16, (cuuint32_t)kVoteTile, 1, 1};
-                const CUresult r2 = encode(&d.map_tail, dt == KVC_DTYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16,
-                                           4, const_cast<void*>(v.k_in), dims, strides, box_tail, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                           CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-                if (r2 != CUDA_SUCCESS) return KVC_ERR_UNSUPPORTED;
-            }
+            // D = 80: the last 16 elements of every row through the 32-byte-swizzled tail map
+            if (!encode_row_maps(encode, &d.map, &d.map_tail, dt == KVC_DTYPE_BF16, v.k_in, dims, strides, kVoteTile, 1))
+                return KVC_ERR_UNSUPPORTED;
             d.q = (const char*)v.q_obs;
             d.votes = (char*)v.votes_out;
             d.lse = v.lse;
@@ -1180,25 +1154,10 @@ int kvc_snapkv_vote_compress(const kvc_shape* shape, int32_t n_layers, const kvc
 #endif  // KVC_HAS_VOTE
 
 #if KVC_HAS_H2O
-int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_layer* layers, float decay,
-                       void* stream) {
-    if (!shape || n_layers < 0 || (n_layers > 0 && !layers)) return KVC_ERR_INVALID_ARG;
-    const int B = shape->batch, H = shape->heads, dt = shape->dtype;
-    if (B <= 0 || H <= 0 || B > 65535) return KVC_ERR_INVALID_ARG;
-    if (dt != KVC_DTYPE_F32 && dt != KVC_DTYPE_F16 && dt != KVC_DTYPE_BF16) return KVC_ERR_UNSUPPORTED;
-    if (n_layers == 0) return KVC_OK;
+// kvc_h2o_accumulate's launches, arguments already checked (also the score-row launch of kvc_h2o_accumulate_qk_tc).
+static int launch_h2o_accumulate(int B, int H, int dt, int32_t n_layers, const kvc_h2o_layer* layers, float decay,
+                                 void* stream) {
     const int e = elem_bytes(dt);
-    for (int l = 0; l < n_layers; ++l) {
-        const kvc_h2o_layer& x = layers[l];
-        if (x.key_len < 0 || !x.acc) return KVC_ERR_INVALID_ARG;
-        if (x.attn && x.n_query <= 0) return KVC_ERR_INVALID_ARG;
-        if (x.score_lo < 0 || x.score_hi < x.score_lo || x.score_hi > x.key_len) return KVC_ERR_INVALID_ARG;
-        if (x.score_hi > x.score_lo && !x.score_out) return KVC_ERR_INVALID_ARG;
-        if (((uintptr_t)x.attn | (uintptr_t)x.acc | (uintptr_t)x.score_out) % e) return KVC_ERR_UNSUPPORTED;
-    }
-    DeviceGuard guard(shape->device);
-    NvtxRange nvtx_range("kvc_h2o_accumulate");
-    if (guard.status != KVC_OK) return guard.status;
     const int tc = 32 * (16 / e);  // key columns per CTA
     return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
         H2oBatchDev bd;
@@ -1233,6 +1192,28 @@ int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_l
         by_dtype(dt, [&](auto d) { kvc_h2o_accumulate_kernel<d><<<grid, kH2oThreads, 0, (cudaStream_t)stream>>>(bd); });
         return launched("kvc_h2o_accumulate_kernel launch");
     });
+}
+
+int kvc_h2o_accumulate(const kvc_shape* shape, int32_t n_layers, const kvc_h2o_layer* layers, float decay,
+                       void* stream) {
+    if (!shape || n_layers < 0 || (n_layers > 0 && !layers)) return KVC_ERR_INVALID_ARG;
+    const int B = shape->batch, H = shape->heads, dt = shape->dtype;
+    if (B <= 0 || H <= 0 || B > 65535) return KVC_ERR_INVALID_ARG;
+    if (dt != KVC_DTYPE_F32 && dt != KVC_DTYPE_F16 && dt != KVC_DTYPE_BF16) return KVC_ERR_UNSUPPORTED;
+    if (n_layers == 0) return KVC_OK;
+    const int e = elem_bytes(dt);
+    for (int l = 0; l < n_layers; ++l) {
+        const kvc_h2o_layer& x = layers[l];
+        if (x.key_len < 0 || !x.acc) return KVC_ERR_INVALID_ARG;
+        if (x.attn && x.n_query <= 0) return KVC_ERR_INVALID_ARG;
+        if (x.score_lo < 0 || x.score_hi < x.score_lo || x.score_hi > x.key_len) return KVC_ERR_INVALID_ARG;
+        if (x.score_hi > x.score_lo && !x.score_out) return KVC_ERR_INVALID_ARG;
+        if (((uintptr_t)x.attn | (uintptr_t)x.acc | (uintptr_t)x.score_out) % e) return KVC_ERR_UNSUPPORTED;
+    }
+    DeviceGuard guard(shape->device);
+    NvtxRange nvtx_range("kvc_h2o_accumulate");
+    if (guard.status != KVC_OK) return guard.status;
+    return launch_h2o_accumulate(B, H, dt, n_layers, layers, decay, stream);
 }
 
 // ------------------------------------------------------------------ kvc_h2o_accumulate_qk
@@ -1374,6 +1355,143 @@ int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layer
         accum<<<dim3((unsigned)max_tiles, (unsigned)B, (unsigned)n_active), kQkThreads, smem2, (cudaStream_t)stream>>>(bd);
         return launched("kvc_h2o_qk_accumulate_kernel launch");
     });
+}
+
+// ------------------------------------------------------------------ kvc_h2o_accumulate_qk_tc
+// Query tiles of a layer: tb = 128 / G positions each (G heads x tb positions = at most 128 MMA rows).
+static int tc_query_tiles(int group, int n_query) { return (n_query + 128 / group - 1) / (128 / group); }
+
+static int64_t tc_layer_ws(const kvc_shape* shape, int group, const kvc_h2o_qk_layer& x) {
+    if (x.key_len <= 0) return 0;
+    const int64_t bytes = (int64_t)shape->batch * shape->heads * tc_query_tiles(group, x.n_query) * kTcRows * 4;
+    return (bytes + 255) & ~(int64_t)255;
+}
+
+// qk_validate's checks, then what the tensor-core form does not cover: fp32, head_dim outside {64, 80, 128}, more than
+// 128 query heads per KV head, and q / K layouts a tensor map cannot describe (16-byte aligned base and strides).
+static int tc_validate(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers) {
+    const int v = qk_validate(shape, group, n_layers, layers);
+    if (v != KVC_OK) return v;
+    const int D = shape->head_dim;
+    if (shape->dtype == KVC_DTYPE_F32 || (D != 64 && D != 80 && D != 128) || group > kTcRows) return KVC_ERR_UNSUPPORTED;
+    for (int l = 0; l < n_layers; ++l) {
+        const kvc_h2o_qk_layer& x = layers[l];
+        if ((uintptr_t)x.q % 16 || (x.q_stride_b * 2) % 16 || (x.q_stride_h * 2) % 16 || (x.q_stride_t * 2) % 16)
+            return KVC_ERR_UNSUPPORTED;
+    }
+    return KVC_OK;
+}
+
+int64_t kvc_h2o_qk_tc_workspace_bytes(const kvc_shape* shape, int32_t group, int32_t n_layers,
+                                      const kvc_h2o_qk_layer* layers) {
+    if (tc_validate(shape, group, n_layers, layers) != KVC_OK) return -1;
+    int64_t total = 0;
+    for (int l = 0; l < n_layers; ++l) total += tc_layer_ws(shape, group, layers[l]);
+    return total;
+}
+
+using TcFn = void (*)(const H2oTcBatchDev);
+
+extern "C++" {
+template <int DT>
+static TcFn pick_tc(bool cols, int cpr) {
+    if (cols) return cpr == 8 ? kvc_h2o_tc_kernel<DT, 8, true> : cpr == 10 ? kvc_h2o_tc_kernel<DT, 10, true>
+                                                                           : kvc_h2o_tc_kernel<DT, 16, true>;
+    return cpr == 8 ? kvc_h2o_tc_kernel<DT, 8, false> : cpr == 10 ? kvc_h2o_tc_kernel<DT, 10, false>
+                                                                  : kvc_h2o_tc_kernel<DT, 16, false>;
+}
+}
+
+int kvc_h2o_accumulate_qk_tc(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers,
+                             float decay, void* workspace, int64_t workspace_bytes, void* stream) {
+    const int v = tc_validate(shape, group, n_layers, layers);
+    if (v != KVC_OK) return v;
+    int64_t need = 0;
+    for (int l = 0; l < n_layers; ++l) need += tc_layer_ws(shape, group, layers[l]);
+    if (need > 0 && (!workspace || workspace_bytes < need || (uintptr_t)workspace % 16)) return KVC_ERR_INVALID_ARG;
+    if (need == 0) return KVC_OK;  // every layer has key_len 0
+    DeviceGuard guard(shape->device);
+    NvtxRange nvtx_range("kvc_h2o_accumulate_qk_tc");
+    if (guard.status != KVC_OK) return guard.status;
+    EncodeTiledFn encode = tensor_map_encoder();
+    if (!encode) return KVC_ERR_UNSUPPORTED;
+    const int B = shape->batch, Hkv = shape->heads, D = shape->head_dim, dt = shape->dtype;
+    const int cpr = D * 2 / 16, tb = kTcRows / group;
+    const bool bf16 = dt == KVC_DTYPE_BF16;
+    const TcFn rows = bf16 ? pick_tc<KVC_DTYPE_BF16>(false, cpr) : pick_tc<KVC_DTYPE_F16>(false, cpr);
+    const TcFn cols = bf16 ? pick_tc<KVC_DTYPE_BF16>(true, cpr) : pick_tc<KVC_DTYPE_F16>(true, cpr);
+    const size_t smem = (size_t)tc_smem_bytes(cpr, group);
+    int st = ensure_tma_attrs((const void*)rows, shape->device);
+    if (st != KVC_OK) return st;
+    st = ensure_tma_attrs((const void*)cols, shape->device);
+    if (st != KVC_OK) return st;
+    char* ws = (char*)workspace;
+    for (int l0 = 0; l0 < n_layers; l0 += kTcLayers) {
+        const int nl = std::min(n_layers - l0, kTcLayers);
+        H2oTcBatchDev bd;
+        memset(&bd, 0, sizeof(bd));
+        bd.B = B;
+        bd.Hkv = Hkv;
+        bd.G = group;
+        bd.tb = tb;
+        bd.decay = decay;
+        kvc_h2o_layer rescore[kTcLayers];
+        int n_active = 0, n_scored = 0, max_qt = 0, max_kt = 0;
+        for (int l = 0; l < nl; ++l) {
+            const kvc_h2o_qk_layer& x = layers[l0 + l];
+            if (x.key_len == 0) continue;
+            H2oTcLayerDev& d = bd.layers[n_active++];
+            const cuuint64_t qdims[4] = {(cuuint64_t)D, (cuuint64_t)x.n_query, (cuuint64_t)Hkv * group, (cuuint64_t)B};
+            const cuuint64_t qstr[3] = {(cuuint64_t)x.q_stride_t * 2, (cuuint64_t)x.q_stride_h * 2,
+                                        (cuuint64_t)x.q_stride_b * 2};
+            const cuuint64_t kdims[4] = {(cuuint64_t)D, (cuuint64_t)x.key_len, (cuuint64_t)Hkv, (cuuint64_t)B};
+            const cuuint64_t kstr[3] = {(cuuint64_t)x.k_stride_s * 2, (cuuint64_t)x.k_stride_h * 2,
+                                        (cuuint64_t)x.k_stride_b * 2};
+            if (!encode_row_maps(encode, &d.qmap, &d.qmap_tail, bf16, x.q, qdims, qstr, tb, group) ||
+                !encode_row_maps(encode, &d.kmap, &d.kmap_tail, bf16, x.k, kdims, kstr, kTcRows, 1))
+                return KVC_ERR_UNSUPPORTED;
+            d.mask = x.mask;
+            d.msb = x.m_stride_b;
+            d.mst = x.m_stride_t;
+            d.acc = (char*)x.acc;
+            d.csb = x.acc_stride_b * 2;
+            d.csh = x.acc_stride_h * 2;
+            d.lse = (float*)ws;
+            ws += tc_layer_ws(shape, group, x);
+            d.c2 = x.scaling * 1.4426950408889634f;
+            d.T = x.n_query;
+            d.K = x.key_len;
+            d.prev = x.prev_len;
+            d.n_qt = tc_query_tiles(group, x.n_query);
+            d.n_kt = (x.key_len + kTcRows - 1) / kTcRows;
+            max_qt = std::max(max_qt, d.n_qt);
+            max_kt = std::max(max_kt, d.n_kt);
+            if (x.score_hi > x.score_lo) {  // the score row: kvc_h2o_accumulate's re-score of the updated accumulators
+                kvc_h2o_layer& r = rescore[n_scored++];
+                memset(&r, 0, sizeof(r));
+                r.acc = x.acc;
+                r.acc_stride_b = x.acc_stride_b;
+                r.acc_stride_h = x.acc_stride_h;
+                r.score_out = x.score_out;
+                r.key_len = x.key_len;
+                r.prev_len = x.key_len;
+                r.score_lo = x.score_lo;
+                r.score_hi = x.score_hi;
+            }
+        }
+        if (n_active == 0) continue;
+        rows<<<dim3((unsigned)max_qt, (unsigned)(B * Hkv), (unsigned)n_active), kTcThreads, smem, (cudaStream_t)stream>>>(bd);
+        st = launched("kvc_h2o_tc_kernel (rows) launch");
+        if (st != KVC_OK) return st;
+        cols<<<dim3((unsigned)max_kt, (unsigned)(B * Hkv), (unsigned)n_active), kTcThreads, smem, (cudaStream_t)stream>>>(bd);
+        st = launched("kvc_h2o_tc_kernel (columns) launch");
+        if (st != KVC_OK) return st;
+        if (n_scored > 0) {
+            st = launch_h2o_accumulate(B, Hkv * group, dt, n_scored, rescore, decay, stream);
+            if (st != KVC_OK) return st;
+        }
+    }
+    return KVC_OK;
 }
 #endif  // KVC_HAS_H2O
 

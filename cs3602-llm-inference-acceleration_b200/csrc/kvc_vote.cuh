@@ -32,11 +32,11 @@
 // Intensity is ~2*128 flop per key byte at most: the kernel stays HBM/MUFU-bound, not tensor-bound
 // (SURVEY.md §7 "SnapKV vote spec gap") — the tensor pipe is reported, not chased.
 #pragma once
-#include <cuda.h>  // CUtensorMap (type only; the encoder is fetched through cudaGetDriverEntryPoint)
 #include <type_traits>
 
 #include "kvc_device.cuh"
 #include "kvc_fused_tma.cuh"
+#include "kvc_tcgen05.cuh"
 #include "kvc_tma.cuh"
 
 namespace kvc {
@@ -44,74 +44,6 @@ namespace kvc {
 constexpr int kVoteM = 128;     // rows of both MMA shapes
 constexpr int kVoteTile = 128;  // keys per tile
 
-// ---------------------------------------------------------------- tcgen05 wrappers
-__device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-// D[tmem] (+)= A[smem] . B[smem]^T, bf16/fp16 inputs, fp32 accumulate; issued by ONE thread.
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// mbarrier arrive once every previously issued tcgen05.mma of this thread has completed.
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread (lane = TMEM lane base + laneid).
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr)
-        : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// 32 lanes x 16 consecutive fp32 columns, asynchronous: tmem_ld_wait() before the registers are read.
-__device__ __forceinline__ void tmem_ld16_async(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// K-major, no swizzle: 8x16-byte core matrices; LBO = step between the two 16-byte K chunks of one
-// K=16 instruction, SBO = step between 8-row groups (cute/arch/mma_sm100_desc.hpp, SmemDescriptor).
-__device__ __forceinline__ uint64_t umma_smem_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3fff);
-    d |= (uint64_t)((lbo_bytes >> 4) & 0x3fff) << 16;
-    d |= (uint64_t)((sbo_bytes >> 4) & 0x3fff) << 32;
-    d |= (uint64_t)1 << 46;  // descriptor version (Blackwell)
-    return d;                // base_offset 0, lbo_mode 0, layout_type 0 = SWIZZLE_NONE
-}
-// Instruction descriptor (cute/arch/mma_sm100_desc.hpp, InstrDescriptor): fp32 accumulate, K-major A and B.
-__host__ __device__ constexpr uint32_t umma_idesc_f16(int fmt /*0 f16, 1 bf16*/, int m, int n) {
-    return (1u << 4) | ((uint32_t)fmt << 7) | ((uint32_t)fmt << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-
-__device__ __forceinline__ float ex2(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
 // Lab build only.  KVC_VOTE_DEBUG=6: the exponentials of both passes replaced by the identity (everything but the MUFU
 // work is timed); KVC_T0 / KVC_TACC: cycles a role spends inside its mbarrier waits, per CTA, into lab_timeline.
 #ifdef KVC_LAB
@@ -149,10 +81,6 @@ __device__ __forceinline__ void tile_item(int q, int& r, int& c) {
 // followed by the tiles of pass 2 (P keys, A = keys); the copy and MMA threads run ahead across the pass boundary,
 // only the math groups meet there to merge the row statistics.  (A cp.async-fed variant of this layout, four copy
 // warps, was measured at 21.6 ms on c4_vote against 15.6 ms for the TMA-fed one and removed.)
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-
 // ---------------------------------------------------------------------------------------------
 // TMA-fed warp-specialised form (head_dim * 2 bytes a multiple of 128: D = 64, 128).  Stage isolation of the
 // cp.async-fed kernels showed the copy stage alone at 4.3 TB/s (16 of 22 ms at c4): 16-byte copies into the
@@ -184,34 +112,6 @@ struct VoteTmaBatchDev {
     long long* lab_timeline;  // lab build: [CTAs][8] cycle counters, or nullptr
     VoteTmaLayerDev layers[32];
 };
-
-__device__ __forceinline__ void tma_load_4d(uint32_t dst_smem, const CUtensorMap* map, int c0, int c1, int c2, int c3,
-                                            uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-        ::"r"(dst_smem), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar)
-        : "memory");
-}
-// K-major, 32-byte swizzle: rows 32 B apart inside an 8-row atom, atoms 256 B apart (SBO), LBO = 16 B.
-__device__ __forceinline__ uint64_t umma_smem_desc_sw32(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3fff);
-    d |= (uint64_t)1 << 16;
-    d |= (uint64_t)(256 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)6 << 61;  // layout type SWIZZLE_32B
-    return d;
-}
-// K-major, 128-byte swizzle: rows 128 B apart inside an 8-row atom, atoms 1024 B apart (SBO), LBO = 16 B.
-__device__ __forceinline__ uint64_t umma_smem_desc_sw128(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3fff);
-    d |= (uint64_t)1 << 16;           // leading byte offset 16 B (unused by swizzled K-major layouts)
-    d |= (uint64_t)(1024 >> 4) << 32;  // stride byte offset: 8 rows x 128 B
-    d |= (uint64_t)1 << 46;           // descriptor version (Blackwell)
-    d |= (uint64_t)2 << 61;           // layout type SWIZZLE_128B
-    return d;
-}
 
 // Ring depth of the TMA-fed kernel.  A slot is held from the issue of its load until its MMAs have completed, ~3 us,
 // so the ring depth bounds the tile rate: 5 slots of 20 KB (D = 80) left the MHA shape latency-bound (copies alone

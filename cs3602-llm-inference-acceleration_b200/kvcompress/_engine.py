@@ -122,6 +122,10 @@ def load_library():
     lib.kvc_h2o_accumulate_qk.restype = ctypes.c_int
     lib.kvc_h2o_accumulate_qk.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_char_p, ctypes.c_float,
                                           ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
+    lib.kvc_h2o_qk_tc_workspace_bytes.restype = ctypes.c_int64
+    lib.kvc_h2o_qk_tc_workspace_bytes.argtypes = lib.kvc_h2o_qk_workspace_bytes.argtypes
+    lib.kvc_h2o_accumulate_qk_tc.restype = ctypes.c_int
+    lib.kvc_h2o_accumulate_qk_tc.argtypes = lib.kvc_h2o_accumulate_qk.argtypes
     lib.kvc_compress_layers_carry.restype = ctypes.c_int
     lib.kvc_compress_layers_carry.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
                                               ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
@@ -660,7 +664,7 @@ _H2O_QK = struct.Struct("P3qP3qP2qP2qPf5i")  # kvc_h2o_qk_layer: q | 3 strides |
 assert _H2O_QK.size == 144                    # 2 strides | score_out | scaling | n_query key_len prev_len score_lo score_hi
 
 
-def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspace) -> None:
+def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspace, tensor_cores: bool = False) -> None:
     """H2O attention-score bookkeeping from queries and keys (``kvc_h2o_accumulate_qk``): two launches for all layers.
 
     layers: ``(q, k, mask, acc, score_out, prev_len, score_lo, score_hi, scaling)`` per layer —
@@ -703,6 +707,9 @@ def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspa
         if not _rows_ok(k):
             k = k.contiguous()
             keep.append(k)
+        if tensor_cores and not _rows_ok(q):  # a tensor map needs 16-byte aligned strides, size-1 dimensions included
+            q = q.clone(memory_format=torch.contiguous_format)
+            keep.append(q)
         m_ptr, m_st = 0, (0, 0)
         if mask is not None:
             if mask.dtype != torch.bool or mask.device != dev or mask.dim() != 3 or mask.size(0) != B \
@@ -725,11 +732,14 @@ def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspa
     recs = bytes(buf)
     shape = _SHAPE.pack(B, Hkv, D, KVC_DTYPE[dt], dev.index)
     lib = load_library()
-    need = int(lib.kvc_h2o_qk_workspace_bytes(shape, group, len(layers), recs))
+    name = "kvc_h2o_accumulate_qk_tc" if tensor_cores else "kvc_h2o_accumulate_qk"
+    run = getattr(lib, name)
+    sizer = lib.kvc_h2o_qk_tc_workspace_bytes if tensor_cores else lib.kvc_h2o_qk_workspace_bytes
+    need = int(sizer(shape, group, len(layers), recs))
     if need < 0:
-        status = lib.kvc_h2o_accumulate_qk(shape, group, len(layers), recs, float(decay), None, 0, None)
-        _check(status, "kvc_h2o_accumulate_qk")
-        raise ValueError("kvc_h2o_qk_workspace_bytes: invalid arguments")
+        status = run(shape, group, len(layers), recs, float(decay), None, 0, None)
+        _check(status, name)
+        raise ValueError(f"{name}: invalid arguments")
     ws = workspace(need) if callable(workspace) else workspace
     ws_ptr, ws_bytes = 0, 0
     if ws is not None:
@@ -737,7 +747,16 @@ def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspa
             raise ValueError(f"workspace must be a contiguous tensor on {dev}")
         ws_ptr, ws_bytes = ws.data_ptr(), ws.numel() * ws.element_size()
     if ws_bytes < need:
-        raise ValueError(f"workspace of {ws_bytes} bytes, kvc_h2o_accumulate_qk needs {need}")
-    status = lib.kvc_h2o_accumulate_qk(shape, group, len(layers), recs, float(decay), ctypes.c_void_p(ws_ptr), ws_bytes,
-                                       ctypes.c_void_p(_stream_ptr(dev)))
-    _check(status, "kvc_h2o_accumulate_qk")
+        raise ValueError(f"workspace of {ws_bytes} bytes, {name} needs {need}")
+    status = run(shape, group, len(layers), recs, float(decay), ctypes.c_void_p(ws_ptr), ws_bytes,
+                 ctypes.c_void_p(_stream_ptr(dev)))
+    _check(status, name)
+
+
+def h2o_accumulate_qk_tc(layers: Sequence[tuple], decay: float, group: int, workspace) -> None:
+    """:func:`h2o_accumulate_qk` on the tensor cores (``kvc_h2o_accumulate_qk_tc``): the same records and workspace
+    callback, logits from ``tcgen05.mma`` (16-bit q and K, fp32 accumulation) and ``p = round(exp2(a * c - lse2))``,
+    ``c = scaling * log2(e)``; the query sum, the decay update and the head sum are the CUDA-core form's.  bf16 / f16
+    only, head_dim 64, 80 or 128, q and K with 16-byte aligned base and strides (``ValueError`` otherwise).  Two launches
+    for every 32 layers, plus one for the score rows."""
+    h2o_accumulate_qk(layers, decay, group, workspace, tensor_cores=True)

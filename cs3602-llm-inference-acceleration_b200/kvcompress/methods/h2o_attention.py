@@ -229,11 +229,16 @@ class H2OScoreSlab:
     through this manager also moves the accumulator rows of every compressed layer it holds data for with their tokens
     — ``acc[:, h*G+g, i] = acc[:, h*G+g, src(i)]`` in the same launch that moves K and V — after which the layer holds
     ``C`` valid entries and its next update decays them and zero-extends the new row.  The caller then never resets:
-    keys are ranked by the decayed attention they have received over the whole generation."""
+    keys are ranked by the decayed attention they have received over the whole generation.
+
+    ``tensor_cores=True`` sends every :meth:`update_from_queries` through ``kvc_h2o_accumulate_qk_tc``: the logits come
+    from the tensor cores (16-bit q and K, fp32 accumulation) and the exponentials from ``exp2``, so its bits differ from
+    the default CUDA-core form (both stay within 2 ulps of fp64 logits).  It is the form to use for prompt-sized query
+    counts; bf16 / f16 models with head_dim 64, 80 or 128 only (``ValueError`` otherwise)."""
 
     def __init__(self, start_size: int = 4, heavy_hitter_size: int = 64, recent_size: int = 444,
                  num_layers: int = 32, num_heads: int = 32, decay_factor: float = 0.9, device=None,
-                 capacity: Optional[int] = None, carry_scores: bool = False):
+                 capacity: Optional[int] = None, carry_scores: bool = False, tensor_cores: bool = False):
         self.start_size = start_size
         self.heavy_hitter_size = heavy_hitter_size
         self.recent_size = recent_size
@@ -244,6 +249,7 @@ class H2OScoreSlab:
         self.device = device
         self.capacity = capacity
         self.carry_scores = bool(carry_scores)
+        self.tensor_cores = bool(tensor_cores)
         self.current_seq_len = 0
         self._acc: Optional[torch.Tensor] = None    # [L, B, Hq, capacity]
         self._score: Optional[torch.Tensor] = None  # [L, B, capacity]; row l holds [B, hi - lo] densely
@@ -351,7 +357,8 @@ class H2OScoreSlab:
         (causal: the queries are the last T positions) or a bool ``[B, 1, T, key_len]`` / ``[B, T, key_len]`` mask,
         True = visible.  ``scaling``: the logit scale, one float or one per layer (default ``D ** -0.5``).  The
         probabilities are ``softmax(fp32 logits).to(dtype)``: HF eager attention in a 16-bit model rounds the logits to
-        the model dtype first, SDPA and flash do not.  Two launches for every non-skipped layer with queries and keys;
+        the model dtype first, SDPA and flash do not.  Two launches for every non-skipped layer with queries and keys
+        (three with ``tensor_cores=True``: statistics, column sums, score rows);
         no synchronisation (:func:`kvcompress.capture_queries` records these arguments from a model's forward)."""
         if queries is None:
             return
@@ -387,6 +394,13 @@ class H2OScoreSlab:
             return
         q0, k0 = work[0][1], work[0][2]
         _engine._require_cuda(q0, "queries")
+        if self.tensor_cores:
+            if q0.dtype not in (torch.bfloat16, torch.float16):
+                raise ValueError(f"H2OScoreSlab(tensor_cores=True): {q0.dtype} queries; the tensor-core form takes "
+                                 "bfloat16 / float16 (use tensor_cores=False for float32)")
+            if q0.size(3) not in (64, 80, 128):
+                raise ValueError(f"H2OScoreSlab(tensor_cores=True): head_dim {q0.size(3)} is not 64, 80 or 128 (use "
+                                 "tensor_cores=False)")
         self._ensure(q0.size(0), q0.size(1), q0.dtype, q0.device, max(k.size(2) for _, _, k, _, _ in work))
         recs = []
         for layer_idx, q, k, mask, s in work:
@@ -398,8 +412,8 @@ class H2OScoreSlab:
             self._lens[layer_idx] = key_len
             self._scored[layer_idx] = (lo, hi)
             self.current_seq_len = key_len
-        _engine.h2o_accumulate_qk(recs, self.decay_factor, q0.size(1) // k0.size(1),
-                                  lambda n: self._workspace(n, q0.device))
+        update = _engine.h2o_accumulate_qk_tc if self.tensor_cores else _engine.h2o_accumulate_qk
+        update(recs, self.decay_factor, q0.size(1) // k0.size(1), lambda n: self._workspace(n, q0.device))
 
     def get_heavy_hitter_indices(self, layer_idx: int, seq_len: int) -> torch.Tensor:
         """Indices (relative to the middle region, ascending) of its heaviest tokens — what

@@ -308,6 +308,28 @@ int64_t kvc_h2o_qk_workspace_bytes(const kvc_shape* shape, int32_t group, int32_
 int kvc_h2o_accumulate_qk(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers,
                           float decay, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* The same update with the logits on the 5th-generation tensor cores, for prompt-sized n_query (opt-in: its bits differ
+ * from kvc_h2o_accumulate_qk's).  The same records and the same visibility, prev_len and score rules; per layer:
+ *   a[t,j]   = sum_d q[b,h,t,d] * k[b,h/G,j,d]    tcgen05.mma kind::f16: 16-bit operands, fp32 accumulation in the
+ *              tensor core's order
+ *   c        = fp32(scaling * log2(e))
+ *   lse2[t]  = m + log2(sum_{vis} exp2(fma(a[t,j], c, -m))),  m = max_{vis} a[t,j] * c   (online over 128-key tiles in
+ *              ascending order; +inf for a query that sees no key)
+ *   attn     = round(exp2(fma(a[t,j], c, -lse2[t]))) where visible, 0 elsewhere   (exp2: ex2.approx.ftz.f32)
+ * then exactly kvc_h2o_accumulate_qk's tail: one __fadd_rn chain over ascending t per (head, key), h2o_update_acc, and
+ * the score row as the sum of the updated accumulators in ascending h (a kvc_h2o_accumulate launch with attn = NULL).
+ * Only the logits and the exponential differ from the CUDA-core form; against fp64 logits -> softmax -> round the
+ * accumulators agree within 2 ulps of the attention dtype.  Launches per 32 layers: a statistics pass, a column-sum
+ * pass, and the score-row launch when a layer asks for a score row.  Every tile depends only on (key_len, n_query,
+ * group, head_dim, dtype): a layer's bits do not depend on B, the other layers of the call or the device.  The entry
+ * point allocates nothing and never synchronises.  Refusals, before any CUDA call: everything kvc_h2o_accumulate_qk
+ * refuses; KVC_ERR_UNSUPPORTED for fp32, head_dim outside {64, 80, 128}, group > 128, and q or K whose base or
+ * b / h / t strides are not 16-byte multiples (a tensor map cannot describe them). */
+int64_t kvc_h2o_qk_tc_workspace_bytes(const kvc_shape* shape, int32_t group, int32_t n_layers,
+                                      const kvc_h2o_qk_layer* layers);
+int kvc_h2o_accumulate_qk_tc(const kvc_shape* shape, int32_t group, int32_t n_layers, const kvc_h2o_qk_layer* layers,
+                             float decay, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Per-row state that moves with the kept rows (cumulative H2O: the accumulators of kvc_h2o_accumulate keep describing
  * the token they were accumulated for across a compaction).  Per layer, batch entry b, KV head h, g < group and output

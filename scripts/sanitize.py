@@ -2,7 +2,8 @@
 """Small-shape exerciser for compute-sanitizer (memcheck / racecheck / synccheck / initcheck) over every kernel
 family of the library: the fused kernel (scan, stored norms, caller rows, caller scores, workspace, generic row
 width), slab append (both forms), in-place compaction (overlapping source / destination), the tcgen05 vote (two
-passes, single pass, fused tail).  Results are checked against torch so a sanitizer-clean run is also a correct one.
+passes, single pass, fused tail), the tensor-core H2O query update (both passes, causal and masked tiles).  Results
+are checked against torch (or the CUDA-core form) so a sanitizer-clean run is also a correct one.
 
     compute-sanitizer --tool racecheck python scripts/sanitize.py
 """
@@ -64,6 +65,21 @@ def main():
         out, idx = _engine.snapkv_vote_compress([(k, v)], plan, [q], W, return_indices=True)
         gathered = torch.gather(v, 2, idx[0].long().unsqueeze(-1).expand(-1, -1, -1, D))
         assert torch.equal(out[0][1], gathered)
+    # the tensor-core H2O query update: both passes (causal and masked tiles, D = 80 tail boxes, GQA) + the score row,
+    # against the CUDA-core form
+    from kvcompress import H2OScoreSlab
+    for (B, Hkv, G, T, S, D, dt) in ((1, 2, 4, 40, 300, 128, torch.bfloat16), (2, 1, 1, 130, 200, 80, torch.float16),
+                                     (1, 2, 8, 1, 150, 64, torch.bfloat16)):
+        q = (2 * torch.randn(B, Hkv * G, T, D, generator=gen, device="cuda")).to(dt)
+        k = torch.randn(B, Hkv, S, D, generator=gen, device="cuda").to(dt)
+        mask = torch.rand(B, T, S, generator=gen, device="cuda") > 0.3
+        for m in (None, mask):
+            kw = dict(start_size=4, heavy_hitter_size=16, recent_size=40, num_layers=1, num_heads=Hkv * G)
+            tc, cc = H2OScoreSlab(tensor_cores=True, **kw), H2OScoreSlab(**kw)
+            tc.update_from_queries([q], [k], masks=[m])
+            cc.update_from_queries([q], [k], masks=[m])
+            a, b = tc.accumulated_attention[0].double(), cc.accumulated_attention[0].double()
+            assert torch.all((a - b).abs() <= 2.0 ** -5 * a.abs().maximum(b.abs()) + 1e-6)
     torch.cuda.synchronize()
     print(f"sanitize.py ok: {_engine.launch_count() - n0} launches")
 
