@@ -1151,6 +1151,52 @@ int kvc_snapkv_vote_compress(const kvc_shape* shape, int32_t n_layers, const kvc
     return launch_vote_tma(shape, n_layers, layers, group, window, cpr, plans, io, stream);
 }
 
+int kvc_query_window_push(const kvc_shape* shape, int32_t window, int32_t n_layers, const kvc_qwin_layer* layers,
+                          void* stream) {
+    int cpr = 0;
+    const int st = check_shape(shape, &cpr);
+    if (st != KVC_OK) return st;
+    if (window < 1 || window > kQwinMaxRows || n_layers < 0 || (n_layers > 0 && !layers)) return KVC_ERR_INVALID_ARG;
+    if (shape->dtype == KVC_DTYPE_F32) return KVC_ERR_UNSUPPORTED;
+    for (int l = 0; l < n_layers; ++l) {
+        const kvc_qwin_layer& x = layers[l];
+        if (!x.q_new || !x.window || x.filled < 0 || x.filled > window || x.n_new < 0) return KVC_ERR_INVALID_ARG;
+        if (((uintptr_t)x.q_new | (uintptr_t)x.window) & 15) return KVC_ERR_UNSUPPORTED;
+        if (((x.q_stride_b | x.q_stride_h | x.q_stride_s | x.w_stride_b | x.w_stride_h) * 2) & 15)
+            return KVC_ERR_UNSUPPORTED;
+    }
+    if (n_layers == 0) return KVC_OK;
+    DeviceGuard guard(shape->device);
+    NvtxRange nvtx_range("kvc_query_window_push");
+    if (guard.status != KVC_OK) return guard.status;
+    return for_each_chunk(n_layers, [&](int l0, int nl) -> int {
+        QwinBatchDev bd;
+        memset(&bd, 0, sizeof(bd));
+        bd.Hq = shape->heads;
+        bd.cpr = cpr;
+        bd.window = window;
+        int n_active = 0;
+        for (int l = l0; l < l0 + nl; ++l) {
+            const kvc_qwin_layer& x = layers[l];
+            if (x.n_new == 0) continue;
+            QwinLayerDev& d = bd.layers[n_active++];
+            d.q = (const char*)x.q_new;
+            d.qsb = x.q_stride_b * 2;
+            d.qsh = x.q_stride_h * 2;
+            d.qss = x.q_stride_s * 2;
+            d.w = (char*)x.window;
+            d.wsb = x.w_stride_b * 2;
+            d.wsh = x.w_stride_h * 2;
+            d.filled = x.filled;
+            d.n_new = x.n_new;
+        }
+        if (n_active == 0) return KVC_OK;
+        dim3 grid((unsigned)((int64_t)shape->batch * shape->heads), (unsigned)n_active, 1);
+        kvc_query_window_push_kernel<kQwinChunks><<<grid, kQwinThreads, 0, (cudaStream_t)stream>>>(bd);
+        return launched("kvc_query_window_push_kernel launch");
+    });
+}
+
 #endif  // KVC_HAS_VOTE
 
 #if KVC_HAS_H2O

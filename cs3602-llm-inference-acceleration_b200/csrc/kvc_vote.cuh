@@ -526,4 +526,63 @@ __global__ void __launch_bounds__(576, 1) kvc_snapkv_vote_tma_kernel(const __gri
     }
 }
 
+
+// ------------------------------------------------------------------ observation window: kvc_query_window_push
+// Per (layer, b, hq) the window holds the queries of the last `filled` positions in rows [0, filled).  A push of n_new
+// rows leaves keep = min(W, filled + n_new) rows: output row r is row drop + r of window[:filled] ++ q_new, with
+// drop = filled + n_new - keep.  Kept window rows only move towards row 0, but a new row can land on a window row that
+// is still to be read, so every window row that moves is staged in shared memory before anything is written.  One CTA
+// per unit; rows move in 16-byte chunks, kQwinChunks chunks of every row per round (all of a 256-byte row at once).
+constexpr int kQwinMaxRows = 128;
+constexpr int kQwinChunks = 16;
+constexpr int kQwinThreads = 256;
+
+struct QwinLayerDev {
+    const char* q;          // new rows of unit (0, 0)
+    int64_t qsb, qsh, qss;  // bytes
+    char* w;                // window rows of unit (0, 0), rows dense
+    int64_t wsb, wsh;       // bytes
+    int filled, n_new;
+};
+struct QwinBatchDev {
+    QwinLayerDev layers[KVC_MAX_LAYERS_PER_LAUNCH];
+    int Hq, cpr, window;
+};
+static_assert(sizeof(QwinBatchDev) < 32 * 1024, "kernel parameters are limited to 32 KB");
+
+// CHUNKS = kQwinChunks; a template so that only the object that launches the kernel compiles it.
+template <int CHUNKS>
+__global__ void __launch_bounds__(kQwinThreads) kvc_query_window_push_kernel(const __grid_constant__ QwinBatchDev bd) {
+    __shared__ uint4 stage[kQwinMaxRows * CHUNKS];
+    const QwinLayerDev& L = bd.layers[blockIdx.y];
+    const int b = blockIdx.x / bd.Hq, h = blockIdx.x - b * bd.Hq;
+    const int keep = min(bd.window, L.filled + L.n_new);
+    const int drop = L.filled + L.n_new - keep;
+    const int from_win = max(0, L.filled - drop);  // window[drop, filled) -> rows [0, from_win)
+    const bool slide = from_win > 0 && drop > 0;   // without a slide the kept window rows stay where they are
+    const int64_t row = (int64_t)bd.cpr * 16;
+    char* w = L.w + b * L.wsb + h * L.wsh;
+    const char* q = L.q + b * L.qsb + h * L.qsh;
+    for (int c0 = 0; c0 < bd.cpr; c0 += CHUNKS) {
+        const int nc = min(CHUNKS, bd.cpr - c0);
+        if (slide) {
+            for (int i = threadIdx.x; i < from_win * nc; i += kQwinThreads) {
+                const int r = i / nc, c = i - r * nc;
+                stage[r * CHUNKS + c] = *reinterpret_cast<const uint4*>(w + (drop + r) * row + (c0 + c) * 16);
+            }
+            __syncthreads();
+            for (int i = threadIdx.x; i < from_win * nc; i += kQwinThreads) {
+                const int r = i / nc, c = i - r * nc;
+                *reinterpret_cast<uint4*>(w + r * row + (c0 + c) * 16) = stage[r * CHUNKS + c];
+            }
+        }
+        for (int i = threadIdx.x; i < (keep - from_win) * nc; i += kQwinThreads) {
+            const int r = from_win + i / nc, c = i % nc;
+            *reinterpret_cast<uint4*>(w + r * row + (c0 + c) * 16) =
+                *reinterpret_cast<const uint4*>(q + (drop + r - L.filled) * L.qss + (c0 + c) * 16);
+        }
+        __syncthreads();  // the next round reuses `stage`
+    }
+}
+
 }  // namespace kvc

@@ -30,6 +30,7 @@ from .methods import (
 )
 from .slab_cache import KVSlabCache
 from .capture import capture_queries, QueryCapture
+from .query_window import SnapKVQueryWindow
 from .evaluate import evaluate_with_compression, evaluate_baseline, compare_methods
 from .benchmark import benchmark, measure_generation_metrics, run_benchmark_suite, print_benchmark_summary
 from .utils import (
@@ -49,7 +50,7 @@ __all__ = [
     "to_dynamic_cache", "normalize_kv_cache", "get_cache_size_mb", "get_cache_info", "get_seq_len",
     "evaluate_with_compression", "evaluate_baseline", "compare_methods",
     "benchmark", "measure_generation_metrics", "run_benchmark_suite", "print_benchmark_summary",
-    "KVSlabCache", "capture_queries", "QueryCapture",
+    "KVSlabCache", "capture_queries", "QueryCapture", "SnapKVQueryWindow",
 ]
 
 __version__ = "2.0.0"

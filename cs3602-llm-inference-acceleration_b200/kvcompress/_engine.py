@@ -129,6 +129,9 @@ def load_library():
     lib.kvc_compress_layers_carry.restype = ctypes.c_int
     lib.kvc_compress_layers_carry.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
                                               ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]
+    lib.kvc_query_window_push.restype = ctypes.c_int
+    lib.kvc_query_window_push.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_char_p,
+                                          ctypes.c_void_p]
     lib.kvc_slab_compress_carry.restype = ctypes.c_int
     lib.kvc_slab_compress_carry.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
                                             ctypes.c_void_p, ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p,
@@ -610,6 +613,45 @@ def snapkv_vote_compress(kv: Sequence[Tuple[torch.Tensor, torch.Tensor]], plans,
     if return_votes:
         ret.append(votes_by_layer)
     return ret[0] if len(ret) == 1 else tuple(ret)
+
+
+_QWIN = struct.Struct("P3qP2q2i")  # kvc_qwin_layer: q_new | 3 strides | window | 2 strides | filled n_new
+assert _QWIN.size == 64
+
+
+def query_window_push(layers: Sequence[tuple], window: int) -> None:
+    """Append new query rows to per-layer observation windows, ONE ``kvc_query_window_push`` launch for every layer.
+
+    layers: ``(q_new, buf, filled)`` per layer — q_new ``[B, Hq, n_new, D]`` 16-bit CUDA tensor with a dense last
+    dimension (any other strides), buf the ``[B, Hq, window, D]`` window (same dtype and device, rows dense) whose first
+    ``filled`` rows are valid.  Afterwards buf holds the last ``min(window, filled + n_new)`` rows of
+    ``buf[:, :, :filled] ++ q_new`` at rows ``[0, min(window, filled + n_new))``.  Nothing is synchronised."""
+    if not layers:
+        return
+    buf0 = layers[0][1]
+    _require_cuda(buf0, "query window")
+    B, Hq, _, D = buf0.shape
+    keep, recs = [], bytearray(_QWIN.size * len(layers))
+    for m, (q, buf, filled) in enumerate(layers):
+        _require_cuda(q, f"layer {m} queries")
+        if q.dim() != 4 or q.shape[:2] != (B, Hq) or q.size(3) != D or q.dtype != buf0.dtype or q.device != buf0.device:
+            raise ValueError(f"layer {m}: queries must be a {buf0.dtype} [B={B}, Hq={Hq}, T, D={D}] tensor on "
+                             f"{buf0.device}, got {q.dtype} {tuple(q.shape)}")
+        if buf.shape != buf0.shape or buf.dtype != buf0.dtype or buf.device != buf0.device or buf.stride(3) != 1 \
+                or buf.stride(2) != D:
+            raise ValueError(f"layer {m}: the window must be a dense-row {tuple(buf0.shape)} {buf0.dtype} tensor")
+        if q.size(2) > window:  # only the last `window` rows can survive the push
+            q = q[:, :, -window:]
+        if q.size(2) > 0 and not _rows_ok(q):
+            q = q.contiguous()
+            keep.append(q)
+        qs, ws = q.stride(), buf.stride()
+        _QWIN.pack_into(recs, m * _QWIN.size, q.data_ptr(), qs[0], qs[1], qs[2], buf.data_ptr(), ws[0], ws[1],
+                        int(filled), q.size(2))
+    shape = _SHAPE.pack(B, Hq, D, KVC_DTYPE[buf0.dtype], buf0.device.index)
+    status = load_library().kvc_query_window_push(shape, int(window), len(layers), bytes(recs),
+                                                  ctypes.c_void_p(_stream_ptr(buf0.device)))
+    _check(status, "kvc_query_window_push")
 
 
 _H2O = struct.Struct("P3qP2qP6i")  # kvc_h2o_layer: attn | 3 strides | acc | 2 strides | score_out | n_query key_len prev_len

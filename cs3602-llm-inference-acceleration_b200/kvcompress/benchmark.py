@@ -13,7 +13,8 @@ from typing import Callable, Dict, List, Optional
 
 import torch
 
-from .evaluate import evaluate_with_compression, method_name_of, new_slab_for_model
+from .evaluate import _check_scores, _forward, evaluate_with_compression, method_name_of, new_slab_for_model
+from .query_window import window_for_harness
 from .utils import normalize_kv_cache, to_dynamic_cache
 
 
@@ -21,8 +22,11 @@ def measure_generation_metrics(model, tokenizer=None, text: str = "", compress_f
                                compress_kwargs: Optional[Dict] = None, max_new_tokens: int = 1000,
                                max_input_tokens: int = 3000, skip_layers: List[int] = [0, 1],
                                device: Optional[torch.device] = None, *, input_ids: Optional[torch.Tensor] = None,
-                               cache: str = "dynamic") -> Dict[str, float]:
-    """TTFT / TPOT / throughput of greedy generation with compression after the prefill and after every token."""
+                               cache: str = "dynamic", scores: str = "norms") -> Dict[str, float]:
+    """TTFT / TPOT / throughput of greedy generation with compression after the prefill and after every token.
+    ``scores="queries"``: snapkv_lite votes with the model's own queries (the prompt's last ``observation_window``
+    queries after the prefill, then one more per decode step; see ``evaluate.py``)."""
+    _check_scores(scores)
     if device is None:
         device = next(model.parameters()).device
     compress_kwargs = dict(compress_kwargs or {})
@@ -31,6 +35,10 @@ def measure_generation_metrics(model, tokenizer=None, text: str = "", compress_f
     input_ids = input_ids[:, :max_input_tokens].to(device)
     input_length = input_ids.shape[1]
     eos = getattr(tokenizer, "eos_token_id", None) if tokenizer is not None else None
+    window = None
+    if scores == "queries" and compress_fn is not None:
+        window = window_for_harness(model, compress_fn, compress_kwargs, input_ids.shape[0])
+        compress_kwargs["obs_queries"] = window
 
     slab = method = None
     past_key_values = None
@@ -54,7 +62,7 @@ def measure_generation_metrics(model, tokenizer=None, text: str = "", compress_f
     generated = []
     total_start = time.perf_counter()
     with torch.inference_mode():
-        outputs = model(input_ids, past_key_values=past_key_values, use_cache=True, return_dict=True)
+        outputs = _forward(model, window, input_ids, past_key_values=past_key_values, use_cache=True, return_dict=True)
         next_token = torch.argmax(outputs.logits[:, -1, :], dim=-1, keepdim=True)
         generated.append(next_token)
         if device.type == "cuda":
@@ -62,7 +70,8 @@ def measure_generation_metrics(model, tokenizer=None, text: str = "", compress_f
         ttft = time.perf_counter() - total_start
         past_key_values = compress(outputs.past_key_values)
         for _ in range(max_new_tokens - 1):
-            outputs = model(next_token, past_key_values=past_key_values, use_cache=True, return_dict=True)
+            outputs = _forward(model, window, next_token, past_key_values=past_key_values, use_cache=True,
+                              return_dict=True)
             next_token = torch.argmax(outputs.logits[:, -1, :], dim=-1, keepdim=True)
             generated.append(next_token)
             if eos is not None and next_token.numel() == 1 and next_token.item() == eos:

@@ -12,6 +12,15 @@ Two cache paths run the identical loop:
 ``cache="slab"``     a :class:`KVSlabCache` is the model's cache object: HF's ``update`` appends in place, and
                      ``compress_`` compacts every layer in place in one launch (SURVEY.md §8f rank 1).
 
+Two score sources for ``snapkv_lite_compress``:
+
+``scores="norms"``   the reference's SnapKV-lite: prefix keys ranked by pooled inverted key norms;
+``scores="queries"`` SnapKV proper: every forward runs under :func:`kvcompress.capture_queries`, a
+                     :class:`SnapKVQueryWindow` keeps each layer's queries of the last ``observation_window``
+                     positions on the device, and the prefix keys are ranked by the attention mass those queries give
+                     them (the tcgen05 vote, ``obs_queries=window``).  16-bit models, ``compress_fn`` snapkv_lite or
+                     ``None``, ``G * observation_window <= 128``.
+
 ``tokenizer`` only needs ``encode(text, return_tensors="pt")``; pass ``input_ids=`` to skip it (offline runs).
 """
 
@@ -24,6 +33,8 @@ from typing import Callable, Dict, List, Optional
 import torch
 from torch.nn import CrossEntropyLoss
 
+from .capture import capture_queries
+from .query_window import window_for_harness
 from .slab_cache import KVSlabCache
 from .utils import normalize_kv_cache, to_dynamic_cache
 
@@ -50,6 +61,21 @@ def new_slab_for_model(model, batch: int, capacity: int, dtype=None, device=None
     return KVSlabCache(cfg.num_hidden_layers, batch, heads, head_dim, capacity, dtype or p.dtype, device or p.device)
 
 
+def _check_scores(scores: str) -> None:
+    if scores not in ("norms", "queries"):
+        raise ValueError(f"scores must be 'norms' or 'queries', got {scores!r}")
+
+
+def _forward(model, window, *args, **kwargs):
+    """``model(*args, **kwargs)``; with a query window, under :func:`capture_queries`, the queries pushed after."""
+    if window is None:
+        return model(*args, **kwargs)
+    with capture_queries(model) as capture:
+        outputs = model(*args, **kwargs)
+    window.push(capture)
+    return outputs
+
+
 def _final_cache_size(lengths: List[int], skip_layers) -> int:
     for layer_idx, n in enumerate(lengths):  # a layer that is actually compressed (reference :205-216)
         if layer_idx not in skip_layers:
@@ -61,10 +87,13 @@ def evaluate_with_compression(model, tokenizer=None, text: str = "", compress_fn
                               compress_kwargs: Optional[Dict] = None, max_tokens: int = 3000,
                               skip_layers: List[int] = [0, 1], device: Optional[torch.device] = None,
                               show_progress: bool = True, *, input_ids: Optional[torch.Tensor] = None,
-                              cache: str = "dynamic", return_nlls: bool = False) -> Dict[str, float]:
-    """PPL / accuracy / TTFT / TPOT with ``compress_fn`` applied after every token (reference evaluate.py:26-226)."""
+                              cache: str = "dynamic", return_nlls: bool = False,
+                              scores: str = "norms") -> Dict[str, float]:
+    """PPL / accuracy / TTFT / TPOT with ``compress_fn`` applied after every token (reference evaluate.py:26-226).
+    ``scores="queries"``: snapkv_lite votes with the model's own queries (module docstring)."""
     if cache not in ("dynamic", "slab"):
         raise ValueError(f"cache must be 'dynamic' or 'slab', got {cache!r}")
+    _check_scores(scores)
     if device is None:
         device = next(model.parameters()).device
     compress_kwargs = dict(compress_kwargs or {})
@@ -72,6 +101,10 @@ def evaluate_with_compression(model, tokenizer=None, text: str = "", compress_fn
         input_ids = tokenizer.encode(text, return_tensors="pt")
     input_ids = input_ids[:, :max_tokens].to(device)
     seq_len = input_ids.shape[1]
+    window = None
+    if scores == "queries" and compress_fn is not None:
+        window = window_for_harness(model, compress_fn, compress_kwargs, input_ids.shape[0])
+        compress_kwargs["obs_queries"] = window
     if seq_len < 2:
         return dict(_EMPTY)
 
@@ -102,7 +135,8 @@ def evaluate_with_compression(model, tokenizer=None, text: str = "", compress_fn
     with torch.inference_mode():
         for idx in steps:
             token_start = time.perf_counter()
-            outputs = model(input_ids[:, idx:idx + 1], past_key_values=past_key_values, use_cache=True)
+            outputs = _forward(model, window, input_ids[:, idx:idx + 1], past_key_values=past_key_values,
+                              use_cache=True)
             logits = outputs.logits[:, -1, :].view(-1, vocab)
             target = input_ids[:, idx + 1:idx + 2].view(-1)
             nll = loss_fn(logits, target)

@@ -1,11 +1,12 @@
 """SnapKV-lite: pooled inverted-norm voting + observation window (reference methods/snapkv_lite.py:24-154)."""
 
 from dataclasses import replace
-from typing import List, Optional, Sequence, Tuple
+from typing import List, Tuple
 
 import torch
 
 from .. import _engine, _planner
+from ..query_window import SnapKVQueryWindow
 from ._common import as_layer_list, cached_plans, execute, seq_lens, stored_norms
 
 
@@ -21,8 +22,10 @@ def snapkv_lite_compress(past_key_values, observation_window: int = 32, keep_siz
     becomes the SnapKV vote ``softmax(q.K^T / sqrt(D)).sum(window queries, group heads)`` computed on the tensor
     cores, pooled, selected and gathered exactly as above — all in ONE launch (``_engine.snapkv_vote_compress``).
     ``obs_lse=`` (optional, with ``obs_queries``): per layer the ``[B, H*G, W]`` float32 log-sum-exp of those queries'
-    attention rows, as returned by a flash-attention forward; the kernel then reads K once instead of twice."""
-    obs_queries: Optional[Sequence[Optional[torch.Tensor]]] = kwargs.get("obs_queries")
+    attention rows, as returned by a flash-attention forward; the kernel then reads K once instead of twice.
+    ``obs_queries`` may also be a :class:`kvcompress.SnapKVQueryWindow` fed by the model's own forwards: its window must
+    be ``observation_window`` long and full on every layer that votes (``ValueError`` otherwise)."""
+    obs_queries = kwargs.get("obs_queries")
     layers = as_layer_list(past_key_values)
     if not layers:
         return layers
@@ -31,9 +34,11 @@ def snapkv_lite_compress(past_key_values, observation_window: int = 32, keep_siz
     if obs_queries is None:
         return execute(layers, plans, norms=stored_norms(past_key_values),
                    non_blocking=kwargs.get("non_blocking", False), output_device=kwargs.get("output_device"))
+    voted = [li for li, p in enumerate(plans) if p.kind == _planner.GATHER and p.k_sel > 0]
+    if isinstance(obs_queries, SnapKVQueryWindow):
+        obs_queries = obs_queries.queries_for(observation_window, voted)
     if len(obs_queries) != len(layers):
         raise ValueError(f"obs_queries: {len(obs_queries)} entries for {len(layers)} layers")
-    voted = [li for li, p in enumerate(plans) if p.kind == _planner.GATHER and p.k_sel > 0]
     for li in voted:
         if obs_queries[li] is None:
             raise ValueError(f"obs_queries[{li}] is missing for a layer that is compressed")

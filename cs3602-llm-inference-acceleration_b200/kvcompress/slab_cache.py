@@ -36,6 +36,7 @@ import torch
 
 from . import _engine
 from . import _planner as P
+from .query_window import SnapKVQueryWindow
 
 _SLAB = struct.Struct("3P6q")    # kvc_slab_layer: k v norms | k_stride_b k_stride_h v_stride_b v_stride_h n_stride_b n_stride_h
 _ROWS = struct.Struct("2P6q2i")  # kvc_slab_new_rows: k_new v_new | 6 strides | cur_len n_new
@@ -394,10 +395,12 @@ class KVSlabCache:
         if self.pinned:
             raise RuntimeError("the q.K^T vote reads the keys through TMA tensor maps: device-resident slabs only")
         plans = self.plans_for("snapkv_lite", **kwargs)
-        if len(obs_queries) != self.num_layers:
-            raise ValueError(f"obs_queries: {len(obs_queries)} entries for {self.num_layers} layers")
         window = kwargs.get("observation_window", _method_defaults("snapkv_lite")["observation_window"])
         voted = [li for li, p in enumerate(plans) if p.kind == P.GATHER and p.k_sel > 0]
+        if isinstance(obs_queries, SnapKVQueryWindow):
+            obs_queries = obs_queries.queries_for(window, voted)
+        if len(obs_queries) != self.num_layers:
+            raise ValueError(f"obs_queries: {len(obs_queries)} entries for {self.num_layers} layers")
         for li in voted:
             if obs_queries[li] is None:
                 raise ValueError(f"obs_queries[{li}] is missing for a layer that is compressed")

@@ -47,7 +47,7 @@ extern "C" {
 #endif
 
 /* Additions that leave every existing struct layout, enum value and entry point as it was (a new score kind, the
- * kvc_h2o_layer / kvc_h2o_qk_layer / kvc_carry_layer structs and their entry points) keep the version: a caller built against an older header sees the
+ * kvc_h2o_layer / kvc_h2o_qk_layer / kvc_carry_layer / kvc_qwin_layer structs and their entry points) keep the version: a caller built against an older header sees the
  * same ABI, and a caller that uses the additions fails to link or gets KVC_ERR_INVALID_ARG from an older library. */
 #define KVC_ABI_VERSION 5
 
@@ -190,6 +190,24 @@ int kvc_snapkv_vote(const kvc_shape* shape, int32_t n_layers, const kvc_vote_lay
 int kvc_snapkv_vote_compress(const kvc_shape* shape, int32_t n_layers, const kvc_vote_layer* layers,
                              const kvc_layer_plan* plans, const kvc_layer_io* io, int32_t group, int32_t window,
                              void* stream);
+
+/* The vote's observation window kept on the device across forwards.  Per layer, batch entry b and query head hq
+ * (shape->heads = Hq, the QUERY heads), window[b, hq, 0:filled) holds the queries of the last `filled` <= W positions
+ * in position order.  A push appends n_new rows from q_new[b, hq, 0:n_new) and keeps the last min(W, filled + n_new)
+ * rows of window[:filled] ++ q_new at rows [0, min(W, filled + n_new)), byte for byte; with n_new > W only the last W
+ * new rows are read.  The slide is in place.  One launch covers every layer (KVC_MAX_LAYERS_PER_LAUNCH chunks); layers
+ * with n_new == 0 are not touched.  16-bit dtypes only (the vote's).  Refused before any CUDA call:
+ * KVC_ERR_INVALID_ARG for a NULL pointer, window outside [1, 128], filled outside [0, window], n_new < 0;
+ * KVC_ERR_UNSUPPORTED for fp32, and for row widths, bases or b / h / s strides that are not 16-byte multiples. */
+typedef struct kvc_qwin_layer {
+    const void* q_new;                          /* [B, Hq, n_new, D] new queries, last dim dense (e.g. HF's q.transpose(1, 2)) */
+    int64_t q_stride_b, q_stride_h, q_stride_s; /* elements */
+    void* window;                               /* [B, Hq, W, D] window, rows dense */
+    int64_t w_stride_b, w_stride_h;             /* elements */
+    int32_t filled, n_new;
+} kvc_qwin_layer;
+int kvc_query_window_push(const kvc_shape* shape, int32_t window, int32_t n_layers, const kvc_qwin_layer* layers,
+                          void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Slab cache: the container step on both sides of the compress call (SURVEY.md §8f rank 1).

@@ -2,7 +2,7 @@
 """Small-shape exerciser for compute-sanitizer (memcheck / racecheck / synccheck / initcheck) over every kernel
 family of the library: the fused kernel (scan, stored norms, caller rows, caller scores, workspace, generic row
 width), slab append (both forms), in-place compaction (overlapping source / destination), the tcgen05 vote (two
-passes, single pass, fused tail), the tensor-core H2O query update (both passes, causal and masked tiles).  Results
+passes, single pass, fused tail), the tensor-core H2O query update (both passes, causal and masked tiles), the SnapKV observation-window push.  Results
 are checked against torch (or the CUDA-core form) so a sanitizer-clean run is also a correct one.
 
     compute-sanitizer --tool racecheck python scripts/sanitize.py
@@ -80,6 +80,18 @@ def main():
             cc.update_from_queries([q], [k], masks=[m])
             a, b = tc.accumulated_attention[0].double(), cc.accumulated_attention[0].double()
             assert torch.all((a - b).abs() <= 2.0 ** -5 * a.abs().maximum(b.abs()) + 1e-6)
+    # the observation-window push: a prompt longer than the window, a decode push that slides every row, a partial
+    # window, an HF-strided view, and a row wider than one 256-byte round
+    from kvcompress import SnapKVQueryWindow
+    for (B, Hq, D, W, dt) in ((2, 4, 80, 32, torch.bfloat16), (1, 2, 256, 8, torch.float16)):
+        win = SnapKVQueryWindow(2, B, Hq, D, W, dt, "cuda")
+        ref = [torch.empty(B, Hq, 0, D, dtype=dt, device="cuda") for _ in range(2)]
+        for T in (5, 3 * W, 1, W - 1):
+            qs = [torch.randn(B, T, Hq, D, generator=gen, device="cuda").to(dt).transpose(1, 2) for _ in range(2)]
+            win.push(qs)
+            ref = [torch.cat([r, q], 2)[:, :, -W:] for r, q in zip(ref, qs)]
+            for l in range(2):
+                assert torch.equal(win.queries[l][:, :, :win.filled[l]], ref[l])
     torch.cuda.synchronize()
     print(f"sanitize.py ok: {_engine.launch_count() - n0} launches")
 
