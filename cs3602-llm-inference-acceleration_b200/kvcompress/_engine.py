@@ -658,6 +658,21 @@ _H2O = struct.Struct("P3qP2qP6i")  # kvc_h2o_layer: attn | 3 strides | acc | 2 s
 assert _H2O.size == 88             #                score_lo score_hi reserved
 
 
+def _h2o_outputs(m: int, acc: torch.Tensor, score: Optional[torch.Tensor], B: int, Hq: int, key_len: int, region: int,
+                 dtype: torch.dtype, device: torch.device) -> int:
+    """Check layer ``m``'s accumulators and score row for an H2O update; returns the score row's address (0: none)."""
+    if acc.dtype != dtype or acc.device != device or acc.dim() != 3 or acc.size(0) != B or acc.size(1) != Hq \
+            or acc.size(2) < key_len or acc.stride(2) != 1:
+        raise ValueError(f"layer {m}: acc must be a [B={B}, Hq={Hq}, >= {key_len}] {dtype} tensor on {device} with a "
+                         "dense last dimension")
+    if score is None:
+        return 0
+    if score.dtype != dtype or score.device != device or not score.is_contiguous() or score.numel() < B * region:
+        raise ValueError(f"layer {m}: score_out must be a contiguous {dtype} tensor of >= B * region elements on "
+                         f"{device}")
+    return score.data_ptr()
+
+
 def h2o_accumulate(layers: Sequence[tuple], decay: float) -> None:
     """H2O attention-score bookkeeping for several layers in ONE ``kvc_h2o_accumulate`` launch.
 
@@ -675,10 +690,7 @@ def h2o_accumulate(layers: Sequence[tuple], decay: float) -> None:
     B, Hq = acc0.size(0), acc0.size(1)
     buf = bytearray(_H2O.size * len(layers))
     for m, (attn, acc, score, prev_len, key_len, lo, hi) in enumerate(layers):
-        if acc.dtype != acc0.dtype or acc.device != acc0.device or acc.dim() != 3 or acc.size(0) != B \
-                or acc.size(1) != Hq or acc.size(2) < key_len or acc.stride(2) != 1:
-            raise ValueError(f"layer {m}: acc must be a [B={B}, Hq={Hq}, >= {key_len}] {acc0.dtype} tensor on "
-                             f"{acc0.device} with a dense last dimension")
+        s_ptr = _h2o_outputs(m, acc, score, B, Hq, key_len, hi - lo, acc0.dtype, acc0.device)
         a_ptr, a_st, n_query = 0, (0, 0, 0), 0
         if attn is not None:
             _require_cuda(attn, f"layer {m} attention")
@@ -687,13 +699,6 @@ def h2o_accumulate(layers: Sequence[tuple], decay: float) -> None:
                 raise ValueError(f"layer {m}: attention must be a [B={B}, Hq={Hq}, n_query, {key_len}] {acc0.dtype} "
                                  f"tensor on {acc0.device} with a dense last dimension")
             a_ptr, a_st, n_query = attn.data_ptr(), attn.stride()[:3], attn.size(2)
-        s_ptr = 0
-        if score is not None:
-            if score.dtype != acc0.dtype or score.device != acc0.device or not score.is_contiguous() \
-                    or score.numel() < B * (hi - lo):
-                raise ValueError(f"layer {m}: score_out must be a contiguous {acc0.dtype} tensor of >= B * region "
-                                 f"elements on {acc0.device}")
-            s_ptr = score.data_ptr()
         _H2O.pack_into(buf, m * _H2O.size, a_ptr, a_st[0], a_st[1], a_st[2], acc.data_ptr(), acc.stride(0),
                        acc.stride(1), s_ptr, n_query, key_len, prev_len, lo, hi, 0)
     shape = _SHAPE.pack(B, Hq, 0, KVC_DTYPE[acc0.dtype], acc0.device.index)
@@ -742,10 +747,7 @@ def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspa
             raise ValueError(f"layer {m}: queries must be a [B={B}, Hq={Hq}, T, D={D}] {dt} tensor on {dev} with a dense "
                              "last dimension")
         T = q.size(2)
-        if acc.dtype != dt or acc.device != dev or acc.dim() != 3 or acc.size(0) != B or acc.size(1) != Hq \
-                or acc.size(2) < key_len or acc.stride(2) != 1:
-            raise ValueError(f"layer {m}: acc must be a [B={B}, Hq={Hq}, >= {key_len}] {dt} tensor on {dev} with a dense "
-                             "last dimension")
+        s_ptr = _h2o_outputs(m, acc, score, B, Hq, key_len, hi - lo, dt, dev)
         if not _rows_ok(k):
             k = k.contiguous()
             keep.append(k)
@@ -761,12 +763,6 @@ def h2o_accumulate_qk(layers: Sequence[tuple], decay: float, group: int, workspa
             m_ptr, m_st = mask.data_ptr(), mask.stride()[:2]
         elif T > key_len:
             raise ValueError(f"layer {m}: {T} queries over {key_len} keys need a mask")
-        s_ptr = 0
-        if score is not None:
-            if score.dtype != dt or score.device != dev or not score.is_contiguous() or score.numel() < B * (hi - lo):
-                raise ValueError(f"layer {m}: score_out must be a contiguous {dt} tensor of >= B * region elements on "
-                                 f"{dev}")
-            s_ptr = score.data_ptr()
         qs, ks = q.stride(), k.stride()
         _H2O_QK.pack_into(buf, m * _H2O_QK.size, q.data_ptr(), qs[0], qs[1], qs[2], k.data_ptr(), ks[0], ks[1], ks[2],
                           m_ptr, m_st[0], m_st[1], acc.data_ptr(), acc.stride(0), acc.stride(1), s_ptr, float(scaling),

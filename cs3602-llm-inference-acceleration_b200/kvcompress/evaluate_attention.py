@@ -36,7 +36,8 @@ from torch.nn import CrossEntropyLoss
 
 from .evaluate import _EMPTY, _final_cache_size, evaluate_with_compression, new_slab_for_model
 from .capture import capture_queries
-from .methods.h2o_attention import H2OAttentionManager, H2OScoreSlab, h2o_attention_compress
+from .methods.h2o_attention import (H2OAttentionManager, H2OScoreSlab, check_carry, h2o_attention_compress,
+                                    update_manager)
 from .utils import normalize_kv_cache, to_dynamic_cache
 
 
@@ -67,9 +68,8 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
     else:
         if scores == "queries" and not isinstance(h2o_manager, H2OScoreSlab):
             raise ValueError("scores='queries' needs an H2OScoreSlab manager")
-        if carry_scores and not (isinstance(h2o_manager, H2OScoreSlab) and h2o_manager.carry_scores):
-            raise ValueError("carry_scores=True needs an H2OScoreSlab(carry_scores=True) manager; "
-                             f"got {type(h2o_manager).__name__} (the torch manager keeps the reference's reset)")
+        if carry_scores:
+            check_carry(h2o_manager, True)
         h2o_manager.reset()
     use_queries = scores == "queries"
     if input_ids is None:
@@ -104,29 +104,20 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
             if use_queries:
                 with capture_queries(model) as capture:
                     outputs = model(input_ids[:, idx:idx + 1], past_key_values=past_key_values, use_cache=True)
-                attentions = None
-                scored = dict(attention_queries=capture)
+                inputs = dict(attention_queries=capture)
             else:
                 outputs = model(input_ids[:, idx:idx + 1], past_key_values=past_key_values, use_cache=True,
                                 output_attentions=True)
-                attentions = outputs.attentions
-                scored = dict(attention_scores=attentions)
-            if carry_scores:  # updated once per forward below; the compaction carries the accumulators
-                scored = {}
+                inputs = dict(attention_scores=outputs.attentions)
+            # cumulative scores: updated once per forward below, the compaction carries the accumulators
+            scored = {} if carry_scores else inputs
             logits = outputs.logits[:, -1, :].view(-1, vocab)
             target = input_ids[:, idx + 1:idx + 2].view(-1)
             nlls.append(float(loss_fn(logits, target).mean().item()))
             correct.append(float((torch.argmax(logits, dim=-1) == target).float().mean().item()))
 
-            def update():
-                if use_queries:
-                    h2o_manager.update_from_queries(capture.queries, capture.keys, capture.masks, capture.scaling,
-                                                    skip_layers)
-                else:
-                    h2o_manager.update_attention_scores(attentions, skip_layers)
-
             if slab is not None:
-                update()
+                update_manager(h2o_manager, skip_layers=skip_layers, **inputs)
                 if slab.lengths[0] > budget:
                     slab.compress_("h2o_attention", h2o_manager=h2o_manager, start_size=start_size,
                                    heavy_hitter_size=heavy_hitter_size, recent_size=recent_size,
@@ -135,7 +126,7 @@ def evaluate_with_attention_compression(model, tokenizer=None, text: str = "",
                         h2o_manager.reset()
             else:
                 past_key_values = outputs.past_key_values
-                update()
+                update_manager(h2o_manager, skip_layers=skip_layers, **inputs)
                 if past_key_values is not None:
                     kv_list = list(normalize_kv_cache(past_key_values))
                     if kv_list and kv_list[0][0].size(2) > budget:

@@ -27,12 +27,23 @@ Two semantics of the accumulators across a compaction:
 """
 
 from collections.abc import Mapping
+from functools import partial
 from typing import Dict, List, Optional, Tuple
 
 import torch
 
 from .. import _engine, _planner
-from ._common import as_layer_list, cached_plans, execute, seq_lens
+from ._common import as_layer_list, cached_plans, seq_lens
+from .h2o_l2 import h2o_l2_compress
+
+
+def _evenly_spaced(seq_len: int, start_size: int, heavy_hitter_size: int, recent_size: int) -> range:
+    """The heavy hitters of a layer without data since the last reset: evenly spaced rows of the middle region,
+    relative to it (reference h2o_attention.py:167-177)."""
+    middle_len = (seq_len - recent_size) - start_size
+    if middle_len <= 0:
+        return range(0)
+    return range(0, middle_len, max(1, middle_len // heavy_hitter_size))[:heavy_hitter_size]
 
 
 class H2OAttentionManager:
@@ -80,12 +91,9 @@ class H2OAttentionManager:
     def get_heavy_hitter_indices(self, layer_idx: int, seq_len: int) -> torch.Tensor:
         """Indices (relative to the middle region, ascending) of its heaviest tokens  (:153-213)."""
         acc = self.accumulated_attention.get(layer_idx)
-        if acc is None:  # no data: evenly spaced  (:167-177)
-            middle_len = (seq_len - self.recent_size) - self.start_size
-            if middle_len <= 0:
-                return torch.tensor([], dtype=torch.long)
-            step = max(1, middle_len // self.heavy_hitter_size)
-            return torch.arange(0, middle_len, step)[: self.heavy_hitter_size]
+        if acc is None:
+            rows = _evenly_spaced(seq_len, self.start_size, self.heavy_hitter_size, self.recent_size)
+            return torch.arange(rows.start, rows.stop, rows.step)
         middle_end = min(seq_len, acc.size(-1)) - self.recent_size
         if middle_end <= self.start_size:
             return torch.tensor([], dtype=torch.long, device=acc.device)
@@ -96,6 +104,30 @@ class H2OAttentionManager:
         _, top = torch.topk(per_token, k, dim=-1)
         top, _ = torch.sort(top, dim=-1)
         return top
+
+    def compress_plans(self, plans, start_size: int, heavy_hitter_size: int, recent_size: int, batch: int, heads: int,
+                       dtype: torch.dtype, device):
+        """:meth:`H2OScoreSlab.compress_plans` for this manager (reference h2o_attention.py:318-331): the head-summed
+        top-k rows of each compressed layer become caller-supplied rows (``SCORE_GIVEN_INDEX``).  Returns
+        ``(plans, {layer: int32 [batch, heads, count] ascending absolute rows on device}, None)``."""
+        new_plans = list(plans)  # the manager rewrites per-layer plans below: never touch the cached set
+        given = {}
+        for li, plan in enumerate(plans):
+            if plan.kind != _planner.GATHER or plan.region == 0:
+                continue
+            middle_len = plan.sel_hi - plan.sel_lo
+            picked = self.get_heavy_hitter_indices(li, plan.seq_len)
+            count = min(len(picked), heavy_hitter_size, middle_len)  # :321
+            if count > 0 and picked.dim() != 1:
+                raise ValueError("h2o_attention: the manager's indices are shared across the batch; batch > 1 "
+                                 "is not supported (the reference fails on it as well)")
+            rows = picked[:count].clamp(0, middle_len - 1).to(device) + plan.sel_lo  # :324-326
+            new_plans[li] = _planner.LayerPlan(_planner.GATHER, plan.seq_len, sink=plan.sink, sel_lo=plan.sel_lo,
+                                               sel_hi=plan.sel_hi, k_sel=count, tail=plan.tail,
+                                               score=_planner.SCORE_GIVEN_INDEX if count > 0 else _planner.SCORE_NONE)
+            if count > 0:
+                given[li] = rows.to(torch.int32).view(1, 1, count).expand(batch, heads, count).contiguous()
+        return new_plans, given, None
 
 
 def update_manager(h2o_manager, attention_scores=None, attention_queries=None, skip_layers=()) -> None:
@@ -142,54 +174,29 @@ def h2o_attention_compress(past_key_values, attention_scores=None, h2o_manager: 
     layers = as_layer_list(past_key_values)
     if not layers:
         return layers
-    if attention_queries is not None and h2o_manager is None:
-        raise ValueError("attention_queries needs an H2OScoreSlab manager (h2o_manager=)")
-    update_manager(h2o_manager, attention_scores, attention_queries, skip_layers)
-    plans = cached_plans(_planner.plan_h2o, seq_lens(layers), start_size, heavy_hitter_size, recent_size,
-                         skip_layers=skip_layers)
     if h2o_manager is None:
-        return execute(layers, plans)
-
-    if isinstance(h2o_manager, H2OScoreSlab):
-        keys = next((layers[li][0] for li in plans.gather), None)
-        if keys is None:
-            return execute(layers, plans)
-        plans, given, scores, *carry = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size,
-                                                                  keys.size(0), keys.size(1), keys.dtype, keys.device)
-        carry = carry[0] if carry else None
-        out = _engine.run_plans(layers, plans, given_indices=given, given_scores=scores, carry=carry)
-        if carry is not None:
-            h2o_manager.carried(plans, carry)
-        return out
-    plans, given = manager_plans(layers, plans, h2o_manager, heavy_hitter_size)
-    return execute(layers, plans, given_indices=given)
+        if attention_queries is not None:
+            raise ValueError("attention_queries needs an H2OScoreSlab manager (h2o_manager=)")
+        return h2o_l2_compress(layers, start_size, heavy_hitter_size, recent_size, skip_layers)
+    keys = layers[0][0]
+    return compress_with_manager(partial(_engine.run_plans, layers), seq_lens(layers),
+                                 (keys.size(0), keys.size(1), keys.dtype, keys.device), h2o_manager, start_size,
+                                 heavy_hitter_size, recent_size, skip_layers, attention_scores, attention_queries)
 
 
-def manager_plans(layers, plans, h2o_manager: H2OAttentionManager, heavy_hitter_size: int):
-    """Rewrite the h2o plans with the manager's heavy hitters (reference h2o_attention.py:318-331): per compressed
-    layer the head-summed top-k rows become caller-supplied rows of the gather (``SCORE_GIVEN_INDEX``).  Returns
-    (plans, {layer: int32 [B, H, count] absolute rows, ascending}).  Shared by the function and by
-    ``KVSlabCache.compress_("h2o_attention", h2o_manager=...)``."""
-    plans = list(plans)  # the manager rewrites per-layer plans below: never touch the cached set
-    given = {}
-    for li, plan in enumerate(plans):
-        if plan.kind != _planner.GATHER or plan.region == 0:
-            continue
-        keys = layers[li][0]
-        batch, heads, seq_len, _ = keys.shape
-        middle_len = plan.sel_hi - plan.sel_lo
-        picked = h2o_manager.get_heavy_hitter_indices(li, seq_len)
-        count = min(len(picked), heavy_hitter_size, middle_len)  # :321
-        if count > 0 and picked.dim() != 1:
-            raise ValueError("h2o_attention: the manager's indices are shared across the batch; batch > 1 "
-                             "is not supported (the reference fails on it as well)")
-        rows = picked[:count].clamp(0, middle_len - 1).to(keys.device) + plan.sel_lo  # :324-326
-        plans[li] = _planner.LayerPlan(_planner.GATHER, seq_len, sink=plan.sink, sel_lo=plan.sel_lo,
-                                       sel_hi=plan.sel_hi, k_sel=count, tail=plan.tail,
-                                       score=_planner.SCORE_GIVEN_INDEX if count > 0 else _planner.SCORE_NONE)
-        if count > 0:
-            given[li] = rows.to(torch.int32).view(1, 1, count).expand(batch, heads, count).contiguous()
-    return plans, given
+def compress_with_manager(run, lens, shape, h2o_manager, start_size: int, heavy_hitter_size: int, recent_size: int,
+                          skip_layers, attention_scores=None, attention_queries=None):
+    """h2o_attention with a manager, for the function and ``KVSlabCache.compress_``: update the manager, plan ``lens``,
+    let the manager rewrite the plans for a ``(batch, heads, dtype, device)`` cache, compact with ``run(plans,
+    given_indices=, given_scores=, carry=)`` (``run_plans`` or ``apply_plans_``) and book what was carried."""
+    update_manager(h2o_manager, attention_scores, attention_queries, skip_layers)
+    plans = cached_plans(_planner.plan_h2o, lens, start_size, heavy_hitter_size, recent_size, skip_layers=skip_layers)
+    plans, given, scores, *carry = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size, recent_size, *shape)
+    carry = carry[0] if carry else None
+    out = run(plans, given_indices=given, given_scores=scores, carry=carry)
+    if carry is not None:
+        h2o_manager.carried(plans, carry)
+    return out
 
 
 class _AccumulatorViews(Mapping):
@@ -308,6 +315,28 @@ class H2OScoreSlab:
             self._scored[li] = (lo, hi)
         _engine.h2o_accumulate(recs, self.decay_factor)
 
+    def _takes(self, layer_idx: int, skip_layers, missing: bool) -> bool:
+        """Whether an update takes a layer (not skipped, no input missing); refuses one past ``num_layers``."""
+        if missing or layer_idx in skip_layers:
+            return False
+        if layer_idx >= self.num_layers:
+            raise ValueError(f"H2OScoreSlab: layer {layer_idx} >= num_layers={self.num_layers}")
+        return True
+
+    def _record(self, layers: List[Tuple[int, int]], like: torch.Tensor) -> List[tuple]:
+        """Book an update of ``(layer_idx, key_len)`` pairs from ``[B, Hq, ...]`` tensors like ``like``; returns
+        ``(acc, score_out, prev_len, lo, hi)`` per layer for the launch records."""
+        self._ensure(like.size(0), like.size(1), like.dtype, like.device, max(n for _, n in layers))
+        out = []
+        for layer_idx, key_len in layers:
+            lo, hi, _ = _planner.h2o_score_region(key_len, key_len, self.start_size, self.heavy_hitter_size,
+                                                  self.recent_size)
+            out.append((self._acc[layer_idx], self._score[layer_idx], self._lens.get(layer_idx, -1), lo, hi))
+            self._lens[layer_idx] = key_len
+            self._scored[layer_idx] = (lo, hi)
+            self.current_seq_len = key_len
+        return out
+
     # ------------------------------------------------------------------ the manager's interface
     def update_attention_scores(self, attentions, skip_layers: List[int] = []) -> None:
         """acc <- decay * acc (zero-extended, or reset if the cache shrank) + attn.sum(query dim), and the score row of
@@ -316,29 +345,17 @@ class H2OScoreSlab:
             return
         work = []
         for layer_idx, attn in enumerate(attentions):
-            if layer_idx in skip_layers or attn is None:
+            if not self._takes(layer_idx, skip_layers, attn is None):
                 continue
-            if layer_idx >= self.num_layers:
-                raise ValueError(f"H2OScoreSlab: layer {layer_idx} >= num_layers={self.num_layers}")
             if attn.dim() != 4:
                 raise ValueError(f"layer {layer_idx}: attention must be [B, Hq, n_query, key_len]")
             work.append((layer_idx, attn if attn.stride(-1) == 1 else attn.contiguous()))
         if not work:
             return
-        a0 = work[0][1]
-        _engine._require_cuda(a0, "attention")
-        self._ensure(a0.size(0), a0.size(1), a0.dtype, a0.device, max(a.size(3) for _, a in work))
-        recs = []
-        for layer_idx, attn in work:
-            key_len = attn.size(3)
-            lo, hi, _ = _planner.h2o_score_region(key_len, key_len, self.start_size, self.heavy_hitter_size,
-                                                  self.recent_size)
-            recs.append((attn, self._acc[layer_idx], self._score[layer_idx], self._lens.get(layer_idx, -1), key_len,
-                         lo, hi))
-            self._lens[layer_idx] = key_len
-            self._scored[layer_idx] = (lo, hi)
-            self.current_seq_len = key_len
-        _engine.h2o_accumulate(recs, self.decay_factor)
+        _engine._require_cuda(work[0][1], "attention")
+        booked = self._record([(layer_idx, attn.size(3)) for layer_idx, attn in work], work[0][1])
+        _engine.h2o_accumulate([(attn, acc, score, prev_len, attn.size(3), lo, hi)
+                                for (_, attn), (acc, score, prev_len, lo, hi) in zip(work, booked)], self.decay_factor)
 
     def _workspace(self, nbytes: int, device: torch.device) -> torch.Tensor:
         """The query path's workspace: kept between updates, grown by doubling, so a steady step allocates nothing."""
@@ -365,10 +382,8 @@ class H2OScoreSlab:
         work = []
         for layer_idx, q in enumerate(queries):
             k = keys[layer_idx] if layer_idx < len(keys) else None
-            if layer_idx in skip_layers or q is None or k is None:
+            if not self._takes(layer_idx, skip_layers, q is None or k is None):
                 continue
-            if layer_idx >= self.num_layers:
-                raise ValueError(f"H2OScoreSlab: layer {layer_idx} >= num_layers={self.num_layers}")
             if q.dim() != 4 or k.dim() != 4 or k.size(1) == 0 or q.size(1) % k.size(1):
                 raise ValueError(f"layer {layer_idx}: queries must be [B, Hq, T, D] and keys [B, Hkv, key_len, D] with "
                                  f"Hkv dividing Hq, got {tuple(q.shape)} and {tuple(k.shape)}")
@@ -401,17 +416,9 @@ class H2OScoreSlab:
             if q0.size(3) not in (64, 80, 128):
                 raise ValueError(f"H2OScoreSlab(tensor_cores=True): head_dim {q0.size(3)} is not 64, 80 or 128 (use "
                                  "tensor_cores=False)")
-        self._ensure(q0.size(0), q0.size(1), q0.dtype, q0.device, max(k.size(2) for _, _, k, _, _ in work))
-        recs = []
-        for layer_idx, q, k, mask, s in work:
-            key_len = k.size(2)
-            lo, hi, _ = _planner.h2o_score_region(key_len, key_len, self.start_size, self.heavy_hitter_size,
-                                                  self.recent_size)
-            recs.append((q, k, mask, self._acc[layer_idx], self._score[layer_idx], self._lens.get(layer_idx, -1), lo, hi,
-                         s))
-            self._lens[layer_idx] = key_len
-            self._scored[layer_idx] = (lo, hi)
-            self.current_seq_len = key_len
+        booked = self._record([(layer_idx, k.size(2)) for layer_idx, _, k, _, _ in work], q0)
+        recs = [(q, k, mask, acc, score, prev_len, lo, hi, s)
+                for (_, q, k, mask, s), (acc, score, prev_len, lo, hi) in zip(work, booked)]
         update = _engine.h2o_accumulate_qk_tc if self.tensor_cores else _engine.h2o_accumulate_qk
         update(recs, self.decay_factor, q0.size(1) // k0.size(1), lambda n: self._workspace(n, q0.device))
 
@@ -419,12 +426,9 @@ class H2OScoreSlab:
         """Indices (relative to the middle region, ascending) of its heaviest tokens — what
         :meth:`H2OAttentionManager.get_heavy_hitter_indices` returns, selected on the device (``kvc_select``)."""
         n = self._lens.get(layer_idx)
-        if n is None:  # no data: evenly spaced  (:167-177)
-            middle_len = (seq_len - self.recent_size) - self.start_size
-            if middle_len <= 0:
-                return torch.tensor([], dtype=torch.long)
-            step = max(1, middle_len // self.heavy_hitter_size)
-            return torch.arange(0, middle_len, step)[: self.heavy_hitter_size]
+        if n is None:
+            rows = _evenly_spaced(seq_len, self.start_size, self.heavy_hitter_size, self.recent_size)
+            return torch.arange(rows.start, rows.stop, rows.step)
         lo, hi, k = _planner.h2o_score_region(seq_len, n, self.start_size, self.heavy_hitter_size, self.recent_size)
         if k == 0:
             return torch.tensor([], dtype=torch.long, device=self._acc.device)
@@ -435,6 +439,16 @@ class H2OScoreSlab:
         return top.squeeze(0) if batch == 1 else top
 
     # ------------------------------------------------------------------ compaction
+    def _check_cache(self, batch: int, heads: int, dtype: torch.dtype, device: torch.device) -> None:
+        """The accumulators against the cache a compaction runs on: the same dtype, batch and device and, to carry them
+        with the rows, ``heads`` dividing their ``Hq``."""
+        acc = self._acc
+        if acc.dtype != dtype:
+            raise ValueError(f"H2OScoreSlab: the attention dtype {acc.dtype} differs from the cache dtype {dtype}")
+        if acc.size(1) != batch or acc.device != device or (self.carry_scores and acc.size(2) % heads):
+            raise ValueError(f"H2OScoreSlab: accumulators of batch {acc.size(1)} with Hq={acc.size(2)} on "
+                             f"{acc.device}, cache of batch {batch} with Hkv={heads} on {device}")
+
     def compress_plans(self, plans, start_size: int, heavy_hitter_size: int, recent_size: int, batch: int, heads: int,
                        dtype: torch.dtype, device):
         """The h2o plans rewritten with this manager's heavy hitters (reference h2o_attention.py:318-331) for a cache
@@ -451,15 +465,11 @@ class H2OScoreSlab:
             carry = {}
             held = [li for li in plans.gather if li in self._lens]
             if held:
-                acc = self._acc
-                if acc.dtype != dtype:
-                    raise ValueError(f"H2OScoreSlab: the attention dtype {acc.dtype} differs from the cache dtype {dtype}")
-                if acc.size(1) != batch or acc.device != device or acc.size(2) % heads:
-                    raise ValueError(f"H2OScoreSlab: accumulators [B={acc.size(1)}, Hq={acc.size(2)}] on {acc.device}, "
-                                     f"cache [B={batch}, Hkv={heads}] on {device}")
-                self._ensure(batch, acc.size(2), dtype, device, max(plans.plans[li].seq_len for li in held))
+                self._check_cache(batch, heads, dtype, device)
+                self._ensure(batch, self._acc.size(2), dtype, device, max(plans.plans[li].seq_len for li in held))
                 group = self._acc.size(2) // heads
                 carry = {li: (self._acc[li], group, self._lens[li]) for li in held}
+        checked = carry is not None  # every layer scored below is held, so checked above
         decisions, rescore = [], []
         for li in plans.gather:
             p = plans.plans[li]
@@ -469,10 +479,8 @@ class H2OScoreSlab:
             S, middle_len = p.seq_len, p.sel_hi - p.sel_lo
             n = self._lens.get(li)
             if n is None:
-                m_len = (S - self.recent_size) - self.start_size
-                picked = range(0, m_len, max(1, m_len // self.heavy_hitter_size))[: self.heavy_hitter_size] \
-                    if m_len > 0 else range(0)
-                decisions.append(("even", m_len, len(picked), min(len(picked), heavy_hitter_size, middle_len)))
+                picked = _evenly_spaced(S, self.start_size, self.heavy_hitter_size, self.recent_size)
+                decisions.append(("even", picked[:min(heavy_hitter_size, middle_len)]))
                 continue
             lo, hi, k = _planner.h2o_score_region(S, n, self.start_size, self.heavy_hitter_size, self.recent_size)
             if k == 0:
@@ -484,12 +492,9 @@ class H2OScoreSlab:
                 raise ValueError(f"layer {li}: H2OScoreSlab(start_size={self.start_size}, heavy_hitter_size="
                                  f"{self.heavy_hitter_size}, recent_size={self.recent_size}) selects {k} of {region} rows, "
                                  f"the compression keeps {count} of {middle_len}: use the same sizes for both")
-            if self._acc.dtype != dtype:
-                raise ValueError(f"H2OScoreSlab: the attention dtype {self._acc.dtype} differs from the cache dtype "
-                                 f"{dtype}")
-            if self._acc.size(1) != batch or self._acc.device != device:
-                raise ValueError(f"H2OScoreSlab: accumulators of batch {self._acc.size(1)} on {self._acc.device}, "
-                                 f"cache of batch {batch} on {device}")
+            if not checked:
+                self._check_cache(batch, heads, dtype, device)
+                checked = True
             if self._scored.get(li) != (lo, hi):
                 rescore.append((li, lo, hi))
             decisions.append(("score", region, count))
@@ -505,22 +510,20 @@ class H2OScoreSlab:
                 continue
             p = plans.plans[li]
             middle_len = p.sel_hi - p.sel_lo
-            count = 0 if d[0] == "none" else d[-1]
-            score = _planner.SCORE_NONE
-            sel_hi = p.sel_hi
-            if count > 0 and d[0] == "even":
-                m_len, n_picked = d[1], d[2]
-                step = max(1, m_len // self.heavy_hitter_size)
-                rows = [min(max(x, 0), middle_len - 1) + p.sel_lo for x in range(0, m_len, step)[:count]]
+            count, score, sel_hi = 0, _planner.SCORE_NONE, p.sel_hi
+            if d[0] == "even" and d[1]:
+                picked = d[1]
+                count = len(picked)
+                rows = [min(max(x, 0), middle_len - 1) + p.sel_lo for x in picked]
                 if any(b <= a for a, b in zip(rows, rows[1:])):
                     raise ValueError(f"layer {li}: evenly spaced rows {rows[:4]}... collide after clamping into the "
                                      f"region of {middle_len} rows")
-                given[li] = (torch.arange(0, m_len, step, device=device, dtype=torch.int32)[:count]
+                given[li] = (torch.arange(picked.start, picked.stop, picked.step, device=device, dtype=torch.int32)
                              .clamp_(0, middle_len - 1).add_(p.sel_lo)
                              .view(1, 1, count).expand(batch, heads, count).contiguous())
                 score = _planner.SCORE_GIVEN_INDEX
-            elif count > 0:
-                region = d[1]
+            elif d[0] == "score":
+                _, region, count = d
                 sel_hi = p.sel_lo + region
                 scores[li] = self._score_row(li, batch, region)
                 score = _planner.SCORE_GIVEN_SCORE_SHARED
@@ -557,4 +560,4 @@ def create_h2o_manager_from_model(model, **kwargs) -> H2OAttentionManager:
 
 
 __all__ = ["H2OAttentionManager", "H2OScoreSlab", "h2o_attention_compress", "create_h2o_manager_from_model",
-           "manager_plans", "update_manager", "check_carry"]
+           "compress_with_manager", "update_manager", "check_carry"]

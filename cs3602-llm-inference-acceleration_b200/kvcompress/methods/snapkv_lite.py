@@ -34,16 +34,34 @@ def snapkv_lite_compress(past_key_values, observation_window: int = 32, keep_siz
     if obs_queries is None:
         return execute(layers, plans, norms=stored_norms(past_key_values),
                    non_blocking=kwargs.get("non_blocking", False), output_device=kwargs.get("output_device"))
+    plans, obs_queries = vote_plans(plans, obs_queries, observation_window, len(layers))
+    return _engine.snapkv_vote_compress(layers, plans, obs_queries, observation_window, lse=kwargs.get("obs_lse"))
+
+
+_VOTE_PLANS = {}
+
+
+def vote_plans(plans, obs_queries, window: int, n_layers: int):
+    """The snapkv ``plans`` of a vote (function and ``KVSlabCache.compress_``): every compressed layer ranks its prefix
+    by its votes (``SCORE_GIVEN_SCORE``).  Returns ``(PlanSet, per-layer queries)``, a :class:`SnapKVQueryWindow`
+    resolved; ``ValueError`` unless there is one entry per layer and every layer that votes has one."""
     voted = [li for li, p in enumerate(plans) if p.kind == _planner.GATHER and p.k_sel > 0]
     if isinstance(obs_queries, SnapKVQueryWindow):
-        obs_queries = obs_queries.queries_for(observation_window, voted)
-    if len(obs_queries) != len(layers):
-        raise ValueError(f"obs_queries: {len(obs_queries)} entries for {len(layers)} layers")
+        obs_queries = obs_queries.queries_for(window, voted)
+    if len(obs_queries) != n_layers:
+        raise ValueError(f"obs_queries: {len(obs_queries)} entries for {n_layers} layers")
     for li in voted:
         if obs_queries[li] is None:
             raise ValueError(f"obs_queries[{li}] is missing for a layer that is compressed")
-    plans = [replace(p, score=_planner.SCORE_GIVEN_SCORE) if li in voted else p for li, p in enumerate(plans)]
-    return _engine.snapkv_vote_compress(layers, plans, obs_queries, observation_window, lse=kwargs.get("obs_lse"))
+    # a decode loop votes with the same (cached) plans every step: rewrite them once, not ahead of every vote launch
+    hit = _VOTE_PLANS.get(id(plans))
+    if hit is None or hit[0] is not plans:
+        hit = (plans, _engine.PlanSet([replace(p, score=_planner.SCORE_GIVEN_SCORE) if li in voted else p
+                                       for li, p in enumerate(plans)]))
+        if len(_VOTE_PLANS) > 64:
+            _VOTE_PLANS.clear()
+        _VOTE_PLANS[id(plans)] = hit
+    return hit[1], obs_queries
 
 
 __all__ = ["snapkv_lite_compress"]

@@ -36,7 +36,6 @@ import torch
 
 from . import _engine
 from . import _planner as P
-from .query_window import SnapKVQueryWindow
 
 _SLAB = struct.Struct("3P6q")    # kvc_slab_layer: k v norms | k_stride_b k_stride_h v_stride_b v_stride_h n_stride_b n_stride_h
 _ROWS = struct.Struct("2P6q2i")  # kvc_slab_new_rows: k_new v_new | 6 strides | cur_len n_new
@@ -390,27 +389,19 @@ class KVSlabCache:
         """snapkv_lite in vote mode, in place: the tcgen05 q.K^T vote over the slab's keys (one launch), then pool ->
         top-k -> slide inside the slab with the votes as caller-supplied scores (one launch).  Keeps the rows
         ``snapkv_lite_compress(cache, obs_queries=...)`` keeps."""
-        from dataclasses import replace
+        from .methods.snapkv_lite import vote_plans
 
         if self.pinned:
             raise RuntimeError("the q.K^T vote reads the keys through TMA tensor maps: device-resident slabs only")
-        plans = self.plans_for("snapkv_lite", **kwargs)
         window = kwargs.get("observation_window", _method_defaults("snapkv_lite")["observation_window"])
-        voted = [li for li, p in enumerate(plans) if p.kind == P.GATHER and p.k_sel > 0]
-        if isinstance(obs_queries, SnapKVQueryWindow):
-            obs_queries = obs_queries.queries_for(window, voted)
-        if len(obs_queries) != self.num_layers:
-            raise ValueError(f"obs_queries: {len(obs_queries)} entries for {self.num_layers} layers")
-        for li in voted:
-            if obs_queries[li] is None:
-                raise ValueError(f"obs_queries[{li}] is missing for a layer that is compressed")
+        plans, obs_queries = vote_plans(self.plans_for("snapkv_lite", **kwargs), obs_queries, window, self.num_layers)
+        voted = [li for li, p in enumerate(plans) if p.score == P.SCORE_GIVEN_SCORE]
         scores = {}
         if voted:
             votes = _engine.snapkv_votes([(self[li][0], obs_queries[li]) for li in voted], window,
                                          lse=None if obs_lse is None else [obs_lse[li] for li in voted])
             scores = dict(zip(voted, votes))
-        new_plans = [replace(p, score=P.SCORE_GIVEN_SCORE) if li in scores else p for li, p in enumerate(plans)]
-        return self.apply_plans_(new_plans, given_scores=scores, return_indices=return_indices)
+        return self.apply_plans_(plans, given_scores=scores, return_indices=return_indices)
 
     def _compress_h2o_attention(self, attention_scores=None, h2o_manager=None, start_size: int = 4,
                                 heavy_hitter_size: int = 64, recent_size: int = 444, skip_layers: Sequence[int] = (),
@@ -422,8 +413,7 @@ class KVSlabCache:
         ``attention_queries``: a ``QueryCapture`` that updates an ``H2OScoreSlab`` instead of ``attention_scores``.
         With ``H2OScoreSlab(carry_scores=True)`` the accumulators slide with the rows in the same launch (cumulative
         H2O); ``carry_scores`` (default: the manager's setting) must agree with the manager."""
-        from .methods._common import cached_plans
-        from .methods.h2o_attention import H2OScoreSlab, check_carry, manager_plans, update_manager
+        from .methods.h2o_attention import H2OAttentionManager, check_carry, compress_with_manager
 
         check_carry(h2o_manager, carry_scores)
         if h2o_manager is None:
@@ -431,23 +421,18 @@ class KVSlabCache:
                 raise ValueError("attention_queries needs an H2OScoreSlab manager (h2o_manager=)")
             return self.compress_("h2o_l2", return_indices=return_indices, start_size=start_size,
                                   heavy_hitter_size=heavy_hitter_size, recent_size=recent_size, skip_layers=skip_layers)
-        update_manager(h2o_manager, attention_scores, attention_queries, skip_layers)
-        plans = cached_plans(P.plan_h2o, self.lengths, start_size, heavy_hitter_size, recent_size, skip_layers=skip_layers)
-        if isinstance(h2o_manager, H2OScoreSlab):  # scores ranked on the device: no host round trip
-            plans, given, scores, *carry = h2o_manager.compress_plans(plans, start_size, heavy_hitter_size,
-                                                                      recent_size, self.batch, self.heads, self.dtype,
-                                                                      self.device)
-            carry = carry[0] if carry else None
-            res = self.apply_plans_(plans, given_indices=given, given_scores=scores, return_indices=return_indices,
-                                    carry=carry)
-            if carry is not None:
-                h2o_manager.carried(plans, carry)
-            return res
-        plans, given = manager_plans(self.to_legacy_cache(), plans, h2o_manager, heavy_hitter_size)
-        for li, rows in given.items():
-            if rows.size(-1) > 1 and not bool((rows[0, 0, 1:] > rows[0, 0, :-1]).all()):
-                raise ValueError(f"layer {li}: the manager's rows must ascend strictly for the in-place compaction")
-        return self.apply_plans_(plans, given_indices=given, return_indices=return_indices)
+
+        def compact(plans, given_indices, **kwargs):
+            if isinstance(h2o_manager, H2OAttentionManager):  # rows sorted by torch; H2OScoreSlab checks its own
+                for li, rows in given_indices.items():
+                    if rows.size(-1) > 1 and not bool((rows[0, 0, 1:] > rows[0, 0, :-1]).all()):
+                        raise ValueError(f"layer {li}: the manager's rows must ascend strictly for the in-place "
+                                         "compaction")
+            return self.apply_plans_(plans, given_indices=given_indices, return_indices=return_indices, **kwargs)
+
+        return compress_with_manager(compact, self.lengths, (self.batch, self.heads, self.dtype, self.device),
+                                     h2o_manager, start_size, heavy_hitter_size, recent_size, skip_layers,
+                                     attention_scores, attention_queries)
 
     def evict_for_space_(self, num_coming: int, start_size: int = 4, recent_size: int = 508,
                          skip_layers: Sequence[int] = (), return_indices: bool = False):
