@@ -317,4 +317,145 @@ __global__ void __launch_bounds__(NT, MINB) kvc_slab_compress_kernel(const __gri
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// kvc_batch_reorder_kernel: the in-place batch gather of beam search (kvc_batch_reorder in kvc.h).  A work item is one
+// byte chunk of one unit of one region, and the CTA that takes it owns those bytes for EVERY batch entry: it loads the
+// distinct sources the index names (entries with idx[b] != b) into shared memory, synchronises, then stores the
+// entries with idx[b] != b.  No CTA reads bytes another CTA writes, so duplicates, cycles and forks are safe in place
+// with no scratch buffer and no host-side planning; an identity index writes nothing.
+constexpr int kReorderMaxRegions = KVC_MAX_REORDER_REGIONS;
+constexpr int kReorderThreads = 256;
+constexpr int kReorderCtasPerSM = 3;  // the register budget of __launch_bounds__ below
+constexpr int kReorderMaxBatch = 1024;
+
+struct ReorderRegionDev {
+    char* base;
+    int64_t sb, su;         // BYTE strides: batch entry, unit
+    int64_t unit_bytes;
+    int64_t item0;          // first work item of the region
+    int32_t units, nchunk;  // nchunk: chunks per unit
+    int32_t g, e;           // word of the 16/8/4/2-byte aligned body, element size of the edge
+};
+static_assert(sizeof(ReorderRegionDev) == 56, "ReorderRegionDev is passed by value in kernel params");
+
+struct ReorderBatchDev {
+    const void* index;
+    int64_t n_items;
+    int32_t B, index_bits;
+    int32_t chunk, n_regions;  // chunk: bytes of a unit per work item (a power of two >= 16)
+    ReorderRegionDev r[kReorderMaxRegions];
+};
+static_assert(sizeof(ReorderBatchDev) < 32 * 1024, "kernel parameters are limited to 32 KB");
+
+// Row i of n_rows: nb bytes from s0 + sidx[i] * ss to d0 + didx[i] * ds (a NULL table stands for i).  The body moves
+// in V-sized words, four in flight per thread (the loads of a batch are issued before its stores); the edge past the
+// last whole word moves in e-byte elements.  tpr threads (a power of two) share a row, so no thread divides.
+template <typename V>
+__device__ __forceinline__ void reorder_rows(int n_rows, int nb, int e, const char* s0, const int16_t* sidx, int64_t ss,
+                                             char* d0, const int16_t* didx, int64_t ds) {
+    constexpr int W = sizeof(V);
+    const int nv = nb / W;
+    int tpr = 1;
+    while (tpr < nv && tpr < kReorderThreads) tpr <<= 1;
+    const int lane = threadIdx.x & (tpr - 1);
+    for (int i = threadIdx.x / tpr; i < n_rows; i += kReorderThreads / tpr) {
+        const V* s = reinterpret_cast<const V*>(s0 + (sidx ? sidx[i] : i) * ss);
+        V* d = reinterpret_cast<V*>(d0 + (didx ? didx[i] : i) * ds);
+        for (int w0 = lane; w0 < nv; w0 += 4 * tpr) {
+            V x[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if (w0 + k * tpr < nv) x[k] = s[w0 + k * tpr];
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if (w0 + k * tpr < nv) d[w0 + k * tpr] = x[k];
+        }
+    }
+    const int ne = (nb - nv * W) / e;  // < W / e
+    for (int i = threadIdx.x; i < n_rows * ne; i += kReorderThreads) {
+        const int row = i / ne, off = nv * W + (i - row * ne) * e;
+        const char* s = s0 + (sidx ? sidx[row] : row) * ss + off;
+        char* d = d0 + (didx ? didx[row] : row) * ds + off;
+        if (e == 4)
+            *reinterpret_cast<uint32_t*>(d) = *reinterpret_cast<const uint32_t*>(s);
+        else
+            *reinterpret_cast<uint16_t*>(d) = *reinterpret_cast<const uint16_t*>(s);
+    }
+}
+
+__device__ __forceinline__ void reorder_rows_g(int g, int n_rows, int nb, int e, const char* s0, const int16_t* sidx,
+                                               int64_t ss, char* d0, const int16_t* didx, int64_t ds) {
+    switch (g) {
+        case 16: reorder_rows<int4>(n_rows, nb, e, s0, sidx, ss, d0, didx, ds); break;
+        case 8: reorder_rows<uint2>(n_rows, nb, e, s0, sidx, ss, d0, didx, ds); break;
+        case 4: reorder_rows<uint32_t>(n_rows, nb, e, s0, sidx, ss, d0, didx, ds); break;
+        default: reorder_rows<uint16_t>(n_rows, nb, e, s0, sidx, ss, d0, didx, ds); break;
+    }
+}
+
+// Dynamic shared memory: B staging slots of `chunk` bytes, then four int16 tables of B entries.
+// (A template, as every kernel here: instantiated only in the object that launches it.)
+template <int NT = kReorderThreads>
+__global__ void __launch_bounds__(NT, kReorderCtasPerSM) kvc_batch_reorder_kernel(const __grid_constant__ ReorderBatchDev bd) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ int n_ld, n_mv;
+    const int B = bd.B, chunk = bd.chunk, tid = threadIdx.x;
+    char* stage = reinterpret_cast<char*>(smem);
+    int16_t* slot_of = reinterpret_cast<int16_t*>(smem + (size_t)B * chunk);  // source entry -> staging slot
+    int16_t* ld_src = slot_of + B;                                             // slot -> source entry
+    int16_t* mv_dst = ld_src + B;                                              // k-th moving entry
+    int16_t* mv_slot = mv_dst + B;                                             // its source's slot
+    auto src_of = [&](int b) -> int {  // idx[b] clamped into [0, B)
+        int64_t s = bd.index_bits == 64 ? reinterpret_cast<const int64_t*>(bd.index)[b]
+                                        : (int64_t)reinterpret_cast<const int32_t*>(bd.index)[b];
+        return (int)(s < 0 ? 0 : (s >= B ? B - 1 : s));
+    };
+    if (tid == 0) n_ld = n_mv = 0;
+    for (int b = tid; b < B; b += kReorderThreads) slot_of[b] = -1;
+    __syncthreads();
+    for (int b = tid; b < B; b += kReorderThreads) {
+        const int s = src_of(b);
+        if (s != b) slot_of[s] = -2;  // a source some entry needs
+    }
+    __syncthreads();
+    for (int s = tid; s < B; s += kReorderThreads)
+        if (slot_of[s] == -2) {
+            const int k = atomicAdd(&n_ld, 1);
+            slot_of[s] = (int16_t)k;
+            ld_src[k] = (int16_t)s;
+        }
+    __syncthreads();
+    for (int b = tid; b < B; b += kReorderThreads) {
+        const int s = src_of(b);
+        if (s != b) {
+            const int k = atomicAdd(&n_mv, 1);
+            mv_dst[k] = (int16_t)b;
+            mv_slot[k] = slot_of[s];
+        }
+    }
+    __syncthreads();
+    const int nld = n_ld, nmv = n_mv;
+    if (nmv == 0) return;  // identity: nothing is written (CTA-uniform)
+
+    for (int64_t it = blockIdx.x; it < bd.n_items; it += gridDim.x) {
+        int lo = 0, hi = bd.n_regions - 1;  // last region with item0 <= it
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (bd.r[mid].item0 <= it) lo = mid;
+            else hi = mid - 1;
+        }
+        const ReorderRegionDev& R = bd.r[lo];
+        const int64_t rem = it - R.item0;
+        const int64_t u = rem / R.nchunk;
+        const int64_t c0 = (rem - u * R.nchunk) * chunk;
+        const int nb = (int)min((int64_t)chunk, R.unit_bytes - c0);
+        char* col = R.base + u * R.su + c0;  // batch entry 0's bytes of this item
+        const int64_t sb = R.sb;
+        __syncthreads();  // the previous item's stores have read the staging slots
+        reorder_rows_g(R.g, nld, nb, R.e, col, ld_src, sb, stage, nullptr, chunk);
+        __syncthreads();  // every source of this item is on chip before any destination is written
+        reorder_rows_g(R.g, nmv, nb, R.e, stage, mv_slot, chunk, col, mv_dst, sb);
+    }
+}
+
 }  // namespace kvc

@@ -990,6 +990,72 @@ int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_
     });
 }
 
+int kvc_batch_reorder(int32_t device, int32_t batch, const void* index, int32_t index_bits, int32_t n_regions,
+                      const kvc_batch_region* regions, void* stream) {
+    if (batch < 1 || batch > kReorderMaxBatch || !index || (index_bits != 32 && index_bits != 64) || n_regions < 0 ||
+        (n_regions > 0 && !regions))
+        return KVC_ERR_INVALID_ARG;
+    int n_active = 0;
+    for (int i = 0; i < n_regions; ++i) {
+        const kvc_batch_region& r = regions[i];
+        if (!r.base || r.stride_b < 0 || r.stride_u < 0 || r.unit_bytes < 0 || r.units < 0) return KVC_ERR_INVALID_ARG;
+        if (r.units == 0 || r.unit_bytes == 0) continue;
+        // every (entry, unit) of the region owns its bytes: entry-major ([B, U, ...]) or unit-major ([U, B, ...])
+        const __int128 ub = r.unit_bytes, su = r.stride_u, sb = r.stride_b;
+        const bool entry_major = (r.units == 1 || su >= ub) && (batch == 1 || sb >= su * (r.units - 1) + ub);
+        const bool unit_major = (batch == 1 || sb >= ub) && (r.units == 1 || su >= sb * (batch - 1) + ub);
+        if (!entry_major && !unit_major) return KVC_ERR_INVALID_ARG;
+        if (r.elem_bytes != 2 && r.elem_bytes != 4) return KVC_ERR_UNSUPPORTED;
+        if (((uintptr_t)r.base | (uint64_t)r.stride_b | (uint64_t)r.stride_u | (uint64_t)r.unit_bytes) % r.elem_bytes)
+            return KVC_ERR_UNSUPPORTED;
+        ++n_active;
+    }
+    if (n_active == 0) return KVC_OK;
+    // staging: `batch` slots of `chunk` bytes plus four int16 tables; chunk is the largest power of two (16 B .. 16 KB)
+    // that keeps them within 48 KB (no opt-in), so that several CTAs stay resident per SM at any batch
+    int chunk = 16 * 1024;
+    while (chunk > 16 && (int64_t)(chunk + 8) * batch > 48 * 1024) chunk >>= 1;
+    const size_t smem = (size_t)batch * chunk + (size_t)batch * 8;
+    const int per_sm = std::max(1, std::min(kReorderCtasPerSM, (int)(kSmemPerSM / (smem + 1024 + 16))));
+    DeviceGuard guard(device);
+    NvtxRange nvtx_range("kvc_batch_reorder");
+    if (guard.status != KVC_OK) return guard.status;
+    int st = KVC_OK;
+    ReorderBatchDev bd;
+    memset(&bd, 0, sizeof(bd));
+    bd.index = index;
+    bd.B = batch;
+    bd.index_bits = index_bits;
+    bd.chunk = chunk;
+    auto launch = [&]() -> int {
+        if (bd.n_regions == 0) return KVC_OK;
+        const int64_t blocks = std::min<int64_t>(bd.n_items, (int64_t)kSMs * per_sm);  // CTAs stride over the rest
+        kvc_batch_reorder_kernel<><<<(unsigned)blocks, kReorderThreads, smem, (cudaStream_t)stream>>>(bd);
+        const int s = launched("kvc_batch_reorder_kernel launch");
+        bd.n_regions = 0;
+        bd.n_items = 0;
+        return s;
+    };
+    for (int i = 0; i < n_regions; ++i) {
+        const kvc_batch_region& r = regions[i];
+        if (r.units == 0 || r.unit_bytes == 0) continue;
+        if (bd.n_regions == kReorderMaxRegions && (st = launch()) != KVC_OK) return st;
+        ReorderRegionDev& d = bd.r[bd.n_regions++];
+        d.base = (char*)r.base;
+        d.sb = r.stride_b;
+        d.su = r.stride_u;
+        d.unit_bytes = r.unit_bytes;
+        d.item0 = bd.n_items;
+        d.units = r.units;
+        d.nchunk = (int32_t)((r.unit_bytes + chunk - 1) / chunk);
+        const uint64_t a = (uintptr_t)r.base | (uint64_t)r.stride_b | (uint64_t)r.stride_u;
+        d.g = (a % 16 == 0) ? 16 : (a % 8 == 0) ? 8 : (a % 4 == 0) ? 4 : 2;
+        d.e = r.elem_bytes;
+        bd.n_items += (int64_t)r.units * d.nchunk;
+    }
+    return launch();
+}
+
 #endif  // KVC_HAS_SLAB
 
 #if KVC_HAS_VOTE

@@ -13,6 +13,7 @@ the current stream; all compute happens in the library's own sm_100a kernels.
 from __future__ import annotations
 
 import ctypes
+import operator
 import os
 import struct
 from typing import List, Optional, Sequence, Tuple
@@ -136,6 +137,9 @@ def load_library():
     lib.kvc_slab_compress_carry.argtypes = [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_char_p,
                                             ctypes.c_void_p, ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p,
                                             ctypes.c_int64, ctypes.c_void_p]
+    lib.kvc_batch_reorder.restype = ctypes.c_int
+    lib.kvc_batch_reorder.argtypes = [ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32,
+                                      ctypes.c_char_p, ctypes.c_void_p]
     if lib.kvc_abi_version() != KVC_ABI_VERSION:
         raise RuntimeError(f"{_LIB_NAME}: ABI version {lib.kvc_abi_version()} != {KVC_ABI_VERSION} — rebuild the library")
     _lib = lib
@@ -798,3 +802,81 @@ def h2o_accumulate_qk_tc(layers: Sequence[tuple], decay: float, group: int, work
     only, head_dim 64, 80 or 128, q and K with 16-byte aligned base and strides (``ValueError`` otherwise).  Two launches
     for every 32 layers, plus one for the score rows."""
     h2o_accumulate_qk(layers, decay, group, workspace, tensor_cores=True)
+
+
+_REGION = struct.Struct("P3q2i")  # kvc_batch_region: base | stride_b stride_u unit_bytes | units elem_bytes
+assert _REGION.size == 40
+
+
+def pack_regions(regions: Sequence[tuple]) -> bytes:
+    """The ``kvc_batch_region`` records of ``(base, stride_b, stride_u, unit_bytes, units, elem_bytes)`` tuples (bytes
+    and addresses): batch entry b, unit u of a region starts at ``base + b * stride_b + u * stride_u``."""
+    return b"".join(_REGION.pack(*r) for r in regions)
+
+
+_UNIT_BYTES = struct.Struct("q")
+_UNIT_BYTES_AT = 24  # offset of unit_bytes in a kvc_batch_region record
+
+
+class RegionRecords:
+    """``kvc_batch_region`` records over buffers whose addresses and strides do not change: packed once, with only
+    ``unit_bytes`` (the valid rows) written per call.  The owner builds one per buffer and builds a new one whenever it
+    reallocates, so the records always describe the live buffer."""
+
+    __slots__ = ("_buf", "_n")
+
+    def __init__(self, regions: Sequence[tuple]):
+        self._buf = bytearray(pack_regions(regions))
+        self._n = len(regions)
+
+    def packed(self, unit_bytes: Sequence[int]) -> bytes:
+        """The records with ``unit_bytes[i]`` for region i (0: the region moves nothing)."""
+        if len(unit_bytes) != self._n:
+            raise ValueError(f"{len(unit_bytes)} sizes for {self._n} regions")
+        buf, pack = self._buf, _UNIT_BYTES.pack_into
+        for i, n in enumerate(unit_bytes):
+            pack(buf, i * _REGION.size + _UNIT_BYTES_AT, n)
+        return bytes(buf)
+
+
+def reorder_index(index, batch: int, device: torch.device) -> torch.Tensor:
+    """The beam index of a reorder as the device tensor ``kvc_batch_reorder`` reads.  A 1-D int32 / int64 tensor of
+    length ``batch`` on ``device`` is used as it is (entries are clamped into ``[0, batch)`` on the device, never
+    dereferenced out of range); a CPU tensor or a sequence is range-checked here, then copied over."""
+    if isinstance(index, torch.Tensor):
+        if index.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f"the reorder index must be int32 or int64, got {index.dtype}")
+        if index.dim() != 1 or index.numel() != batch:
+            raise ValueError(f"the reorder index must be 1-D of length batch={batch}, got {tuple(index.shape)}")
+        if index.is_cuda:
+            if index.device != device:
+                raise ValueError(f"the reorder index is on {index.device}, the cache on {device}")
+            return index if index.stride(0) == 1 else index.contiguous()
+        if index.device.type != "cpu":
+            raise ValueError(f"the reorder index is on {index.device}, the cache on {device}")
+        values = index.tolist()
+    else:
+        try:
+            values = [operator.index(v) for v in index]
+        except TypeError:
+            raise ValueError(f"the reorder index must be integers, got {index!r}") from None
+        if len(values) != batch:
+            raise ValueError(f"the reorder index must have batch={batch} entries, got {len(values)}")
+    bad = [v for v in values if not 0 <= v < batch]
+    if bad:
+        raise ValueError(f"reorder index entries {bad[:4]} are outside [0, {batch})")
+    return torch.tensor(values, dtype=torch.int64).to(device)
+
+
+def batch_reorder(regions, index: torch.Tensor, batch: int) -> None:
+    """Reorder every region along the batch in place, ONE ``kvc_batch_reorder`` launch: entry b of each region takes
+    the bytes entry ``index[b]`` held before the call (``t.index_select(0, index)`` restricted to the regions' bytes).
+    regions: region tuples or packed records (:func:`pack_regions`, :meth:`RegionRecords.packed`); index: what
+    :func:`reorder_index` returns.  Nothing is allocated or synchronised."""
+    recs = regions if isinstance(regions, bytes) else pack_regions(regions)
+    if not recs:
+        return
+    status = load_library().kvc_batch_reorder(index.device.index, int(batch), index.data_ptr(),
+                                              64 if index.dtype == torch.int64 else 32, len(recs) // _REGION.size,
+                                              recs, ctypes.c_void_p(_stream_ptr(index.device)))
+    _check(status, "kvc_batch_reorder")

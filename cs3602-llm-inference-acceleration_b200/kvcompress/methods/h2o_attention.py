@@ -265,6 +265,7 @@ class H2OScoreSlab:
         self._gen = 0                               # bumped whenever the buffers are reallocated
         self._plan_cache: Dict[tuple, tuple] = {}
         self._ws: Optional[torch.Tensor] = None     # workspace of update_from_queries (uint8)
+        self._reorder_recs: Optional[tuple] = None  # (_gen, RegionRecords) of the accumulators, built by a reorder
 
     @property
     def accumulated_attention(self) -> Mapping:
@@ -536,6 +537,39 @@ class H2OScoreSlab:
         if carry is not None:
             return ps, given or None, scores or None, carry
         return ps, given or None, scores or None
+
+    def _reorder_records(self, batch: int, device: torch.device) -> bytes:
+        """``kvc_batch_region`` records of the valid accumulator entries ``[0, _lens[l])`` of every layer, for a batch
+        reorder (none before the first update).  Pointers and strides are packed once per accumulator buffer (``_gen``
+        changes whenever it is reallocated); each call writes the entries from ``_lens``.  Score rows are not moved:
+        they are marked stale and rebuilt from the moved accumulators by the next update or compression."""
+        self._scored = {}
+        acc = self._acc
+        if acc is None or not self._lens:
+            return b""
+        if acc.size(1) != batch or acc.device != torch.device(device):
+            raise ValueError(f"H2OScoreSlab: accumulators of batch {acc.size(1)} on {acc.device}, reordered with a cache "
+                             f"of batch {batch} on {device}")
+        e = acc.element_size()
+        if self._reorder_recs is None or self._reorder_recs[0] != self._gen:
+            self._reorder_recs = (self._gen, _engine.RegionRecords(
+                [(acc[l].data_ptr(), acc.stride(1) * e, acc.stride(2) * e, 0, acc.size(2), e)
+                 for l in range(self.num_layers)]))
+        return self._reorder_recs[1].packed([self._lens.get(l, 0) * e for l in range(self.num_layers)])
+
+    def reorder_(self, index) -> "H2OScoreSlab":
+        """Beam search's reorder of the accumulators: batch entry b of every layer's valid entries becomes what entry
+        ``index[b]`` held (``index_select(0, index)``), ONE ``kvc_batch_reorder`` launch — for the function path, where
+        transformers reorders a ``DynamicCache`` and the scores must follow.  ``index`` as in
+        :meth:`KVSlabCache.reorder_`, which takes this manager as a follower to move it in the slab's launch.  A
+        manager with no accumulators yet moves nothing."""
+        if self._acc is None or not self._lens:
+            self._scored = {}
+            return self
+        batch, device = self._acc.size(1), self._acc.device
+        recs = self._reorder_records(batch, device)
+        _engine.batch_reorder(recs, _engine.reorder_index(index, batch, device), batch)
+        return self
 
     def carried(self, plans, carry: dict) -> None:
         """Bookkeeping after a compaction that carried ``carry`` (from :meth:`compress_plans`) with ``plans``: each

@@ -55,6 +55,7 @@ class SnapKVQueryWindow:
                                 device=self.device)
         self.queries: List[torch.Tensor] = list(self._buf.unbind(0))
         self.filled: List[int] = [0] * self.num_layers
+        self._reorder_recs: Optional[_engine.RegionRecords] = None   # built by the first reorder
 
     @classmethod
     def for_model(cls, model, batch: int, window: int) -> "SnapKVQueryWindow":
@@ -93,6 +94,28 @@ class SnapKVQueryWindow:
         for l, q in enumerate(queries):
             if q is not None:
                 self.filled[l] = min(self.window, self.filled[l] + q.size(2))
+        return self
+
+    def _reorder_records(self, batch: int, device: torch.device) -> bytes:
+        """``kvc_batch_region`` records of the filled rows of every layer, for a batch reorder.  The window buffer is
+        allocated once, so its pointers and strides are packed once; each call writes the rows from ``filled``."""
+        buf = self._buf
+        if batch != self.batch or torch.device(device) != buf.device:
+            raise ValueError(f"SnapKVQueryWindow of batch {self.batch} on {buf.device}, reordered with a cache of "
+                             f"batch {batch} on {device}")
+        e = buf.element_size()
+        if self._reorder_recs is None:
+            self._reorder_recs = _engine.RegionRecords(
+                [(buf[l].data_ptr(), buf.stride(1) * e, buf.stride(2) * e, 0, self.num_heads, e)
+                 for l in range(self.num_layers)])
+        return self._reorder_recs.packed([n * self.head_dim * e for n in self.filled])
+
+    def reorder_(self, index) -> "SnapKVQueryWindow":
+        """Beam search's reorder of the window: batch entry b of the filled rows of every layer becomes what entry
+        ``index[b]`` held (``index_select(0, index)``), ONE ``kvc_batch_reorder`` launch.  ``index`` as in
+        :meth:`KVSlabCache.reorder_`, which takes this window as a follower to move it in the slab's launch."""
+        recs = self._reorder_records(self.batch, self._buf.device)
+        _engine.batch_reorder(recs, _engine.reorder_index(index, self.batch, self._buf.device), self.batch)
         return self
 
     def queries_for(self, observation_window: int, layers: Sequence[int]) -> List[torch.Tensor]:

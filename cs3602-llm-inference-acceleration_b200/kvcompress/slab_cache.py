@@ -126,6 +126,7 @@ class KVSlabCache:
                                                  ctypes.cast(lib.kvc_slab_append, ctypes.c_void_p).value).update
         self._ws = None
         self._launch_cache: Dict[int, tuple] = {}
+        self._reorder_recs: Optional[_engine.RegionRecords] = None   # built by the first reorder_
 
     # ------------------------------------------------------------------ construction / views
     @classmethod
@@ -180,12 +181,15 @@ class KVSlabCache:
         if self.pinned and not torch.cuda.is_current_stream_capturing():
             torch.cuda.current_stream(self.device).synchronize()
 
-    def as_hf_cache(self):
+    def as_hf_cache(self, followers: Sequence = ()):
         """This slab as a ``transformers.Cache``: the model's attention layers call ``update`` (in-place append)
-        and read lengths / mask sizes from the slab, so it can be passed as ``past_key_values``."""
+        and read lengths / mask sizes from the slab, so it can be passed as ``past_key_values``.  Beam search's
+        ``reorder_cache(beam_idx)`` is one :meth:`reorder_` of the slab and of ``followers`` (an ``H2OScoreSlab``, a
+        ``SnapKVQueryWindow``: per-row state that must follow the beams), one launch."""
         from transformers.cache_utils import Cache, CacheLayerMixin
 
         slab = self
+        followers = tuple(followers)
 
         class _SlabLayer(CacheLayerMixin):
             is_sliding = False
@@ -218,9 +222,38 @@ class KVSlabCache:
             def reset(self) -> None:
                 slab.lengths[self.layer_idx] = 0
 
-        cache = Cache(layers=[_SlabLayer(l) for l in range(self.num_layers)])
+        class _SlabHFCache(Cache):
+            def reorder_cache(self, beam_idx: torch.LongTensor) -> None:
+                slab.reorder_(beam_idx, *followers)
+
+        cache = _SlabHFCache(layers=[_SlabLayer(l) for l in range(self.num_layers)])
         cache.slab = self
         return cache
+
+    # ------------------------------------------------------------------ beam search
+    def _reorder_records(self) -> bytes:
+        """``kvc_batch_region`` records of the valid rows of K, V and the norms of every layer.  The slabs never move,
+        so pointers and strides are packed once; each call writes the per-layer ``unit_bytes`` from the lengths."""
+        e, D = self.k.element_size(), self.head_dim
+        if self._reorder_recs is None:
+            self._reorder_recs = _engine.RegionRecords(
+                [(t[l].data_ptr(), t.stride(1) * e, t.stride(2) * e, 0, self.heads, e)
+                 for l in range(self.num_layers) for t in (self.k, self.v, self.n)])
+        return self._reorder_recs.packed([n * row for n in self.lengths for row in (D * e, D * e, e)])
+
+    def reorder_(self, index, *followers) -> "KVSlabCache":
+        """Beam search's reorder in place: batch entry b of every layer's valid K, V and norm rows becomes what entry
+        ``index[b]`` held (``index_select(0, index)`` on each layer), and so does the per-row state of ``followers``
+        (:meth:`H2OScoreSlab.reorder_`, :meth:`SnapKVQueryWindow.reorder_`) — ONE ``kvc_batch_reorder`` launch, no
+        allocation, no synchronisation; lengths, pointers and captured ``capture_step`` graphs stay valid.
+        ``index``: a 1-D int32 / int64 tensor of length ``batch`` on the slab's device (trusted: entries are clamped
+        into ``[0, batch)`` on the device), or a CPU tensor / sequence, range-checked (``ValueError``) and copied over."""
+        if self.pinned:
+            raise ValueError("reorder_ runs on device-resident slabs; a pinned (host) slab cannot be reordered")
+        parts = [f._reorder_records(self.batch, self.device) for f in followers]
+        index = _engine.reorder_index(index, self.batch, self.device)
+        _engine.batch_reorder(b"".join([self._reorder_records()] + parts), index, self.batch)
+        return self
 
     # ------------------------------------------------------------------ append
     def _check_new(self, keys: torch.Tensor, values: torch.Tensor, layer_idx: int) -> None:

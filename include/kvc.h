@@ -47,7 +47,8 @@ extern "C" {
 #endif
 
 /* Additions that leave every existing struct layout, enum value and entry point as it was (a new score kind, the
- * kvc_h2o_layer / kvc_h2o_qk_layer / kvc_carry_layer / kvc_qwin_layer structs and their entry points) keep the version: a caller built against an older header sees the
+ * kvc_h2o_layer / kvc_h2o_qk_layer / kvc_carry_layer / kvc_qwin_layer / kvc_batch_region structs and their entry points)
+ * keep the version: a caller built against an older header sees the
  * same ABI, and a caller that uses the additions fails to link or gets KVC_ERR_INVALID_ARG from an older library. */
 #define KVC_ABI_VERSION 5
 
@@ -375,6 +376,31 @@ int kvc_slab_compress_carry(const kvc_shape* shape, int32_t n_layers, const kvc_
 int kvc_compress_layers_carry(const kvc_shape* shape, int32_t n_layers, const kvc_layer_plan* plans,
                               const kvc_layer_io* io, const kvc_carry_layer* carry, void* workspace,
                               int64_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Beam search: reorder a cache along the batch, in place (transformers' Cache.reorder_cache, i.e.
+ * t.index_select(0, beam_idx) on every K / V tensor, and the same for any per-row state that must follow the beams).
+ * For every region r, batch entry b < batch and unit u < r.units, the bytes [0, unit_bytes) of (r, b, u), at
+ *   base + b * stride_b + u * stride_u,
+ * become the bytes (r, idx[b], u) held before the call; idx[b] = index[b] clamped into [0, batch) (read on the device,
+ * int32 or int64, never dereferenced out of range).  Bytes outside [0, unit_bytes) of each unit are not touched, and an
+ * entry with idx[b] == b is not written (an identity index writes nothing).  Any index is safe in place: duplicates,
+ * cycles, forks ([0, 0, ...]).  Regions must not overlap one another or the index.  ONE launch for every region
+ * (KVC_MAX_REORDER_REGIONS per launch); no allocation, no synchronisation.  Refused before any CUDA call:
+ * KVC_ERR_INVALID_ARG for NULL pointers, batch outside [1, 1024], index_bits not 32 or 64, negative sizes or strides,
+ * and a region whose (entry, unit) byte ranges overlap; KVC_ERR_UNSUPPORTED for elem_bytes other than 2 or 4 and for
+ * base, strides or unit_bytes that are not multiples of elem_bytes. */
+#define KVC_MAX_REORDER_REGIONS 512
+typedef struct kvc_batch_region {
+    void* base;          /* batch entry 0, unit 0 */
+    int64_t stride_b;    /* bytes between batch entries */
+    int64_t stride_u;    /* bytes between units of one entry */
+    int64_t unit_bytes;  /* bytes moved per unit (the valid rows) */
+    int32_t units;       /* units per batch entry (e.g. heads) */
+    int32_t elem_bytes;  /* 2 or 4: the alignment of base, strides and unit_bytes */
+} kvc_batch_region;
+int kvc_batch_reorder(int32_t device, int32_t batch, const void* index, int32_t index_bits, int32_t n_regions,
+                      const kvc_batch_region* regions, void* stream);
 
 #ifdef __cplusplus
 }
